@@ -107,7 +107,7 @@ def cpu_port_run(n, p, K, steps, warmup, seed=0, budget_rows=2048):
 
 def cpu_reference_run(n, p, K, steps, warmup, seed=0, budget_s=150.0):
     """The UNMODIFIED reference (`oriana.models.ZIGaP.step()`, zigap.py:97-158: numba triple loop + numpy) installed
-    under baseline/_ref by `__graft_entry__.build()`, on a bounded row slab of the same workload, through its own
+    under oracle/_ref by `__graft_entry__.build()`, on a bounded row slab of the same workload, through its own
     public API.  The slab is sized so that warmup + steps fit the time budget (the per-entry cost is flat in the
     number of rows, BASELINE.md section 2).  Returns None when the install did not travel."""
     import warnings
@@ -137,7 +137,7 @@ def cpu_reference_run(n, p, K, steps, warmup, seed=0, budget_s=150.0):
     finally:
         refshim.release_reference()
     sample = ('%d-row slab of the workload (%d x %d, K=%d), %d steps of the unmodified reference ZIGaP.step() '
-              '(baseline/_ref; numba Z-loop on ONE thread by construction = ~80 %% of the step, the two np.dot on %d BLAS '
+              '(oracle/_ref; numba Z-loop on ONE thread by construction = ~80 %% of the step, the two np.dot on %d BLAS '
               'threads), %.2f s/step, state finite: %s' % (rows, rows, p, K, steps, os.cpu_count() or 1, dt, ok))
     return rows * p / dt, 1, sample, dt
 
@@ -228,6 +228,29 @@ def secondary_device_run(cfg, world, rank, dev, steps=5, warmup=3):
     return out
 
 
+DUMP_CELLS = 65536
+
+
+def dump_outputs(path, model, trace, rows, r0):
+    """What the timed `model.step()` leaves its caller after the last timed step, as <path>/<name>.npy: the model's
+    `state_dict()` and its ELBO trace.  The cell-side factors (a1, a2: cells x K) are a fixed sample of DUMP_CELLS of
+    this rank's cells, the same in every run of a configuration (their global indices in cells.npy), so that two builds
+    can be compared output for output within 64 MB.  The factors are float32 on the device and written as float32."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    cells = np.arange(rows) if rows <= DUMP_CELLS else np.sort(np.random.default_rng(0).choice(rows, DUMP_CELLS, replace=False))
+    out = {'cells': (r0 + cells).astype(np.float64), 'elbo_trace': np.asarray(trace, dtype=np.float64)}
+    for k, v in model.state_dict().items():
+        if k == 'iterations':
+            continue
+        v = np.asarray(v)
+        out[k] = (v[cells] if k in ('a1', 'a2') else v).astype(np.float32 if k in ('a1', 'a2', 'b1', 'b2') else np.float64)
+    total = sum(v.nbytes for v in out.values())
+    assert total <= 64 << 20, 'outputs of %d bytes exceed 64 MB' % total
+    for k, v in out.items():
+        np.save(os.path.join(path, k + '.npy'), v)
+
+
 def operator_seam_rates(lib):
     """The reference's plug-in point (`ZIGaP.compute_Z_q_expectations`, zigap.py:79-95) through its C-ABI replacement with
     HOST numpy arrays in and out, at config 2 and at a row slab of config 3: entries / s of the whole call (copies in)."""
@@ -267,7 +290,12 @@ def main():
     ap.add_argument('--e2e-x', default='auto', choices=['auto', 'sparse', 'u8esc', 'u16', 'f32'],
                     help='how the host holds X for the e2e leg: bitmap + non-zero bytes (sparse), saturating uint8 + escapes '
                          '(u8esc), uint16, float32; auto (default) = sparse when that is the smaller of the two lossless byte forms')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the model state they computed as DIR/<name>.npy (rank 0; a fixed '
+                         'sample of the cell-side factors, 64 MB at most)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the device run (--impl ours)')
     n, p, K = CONFIGS[args.config]
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
@@ -287,7 +315,7 @@ def main():
         if ref is not None:
             val, cores, sample, dt = ref
             kind = 'reference'
-        else:   # the install did not travel (baseline/_ref missing): the port is what is left
+        else:   # no reference install (oracle/_ref missing): the port is what is left
             val, cores, sample, dt = cpu_port_run(n, p, K, steps, W)
             kind = 'port'
         print(json.dumps({
@@ -365,6 +393,8 @@ def main():
     model.enable_kernel_timing(False)
     trace = model.elbo_trace
     elbo_ok = bool(np.isfinite(trace).all() and np.all(np.diff(trace[1:]) >= -1e-6 * np.abs(trace[1:-1])))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, trace, rows, r0)
 
     # ---- the same steps without the ELBO terms (SURVEY.md 8d: reported beside the contract number, not instead)
     state0 = model.state_dict(); state0['X'] = X[:, :p]

@@ -12,8 +12,8 @@ as the checker (or the timed CPU baseline) -- never as the product path.  The pr
 Pinning status
 --------------
 * CAVI step (Z-kernel, Gamma/Bernoulli updates, M-step): PINNED against the unmodified
-  reference run in the build container (`oracle/make_golden.py` imports
-  `/root/reference` under the `np.float/np.int` alias shim, copies the state out of a
+  reference (`oracle/make_golden.py` imports a checkout of it, `oracle/refshim.py`
+  CHECKOUT, under the `np.float/np.int` alias shim, copies the state out of a
   constructed reference model, steps it and stores the trajectories under
   `tests/golden/`).  `tests/test_oracle.py` replays those fixtures through this port.
 * Special functions (sigmoid/logit/digamma/inverse digamma, Gamma mean/meanlog,

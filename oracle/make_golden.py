@@ -1,6 +1,6 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (build container only).
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (a checkout of it, or its install under oracle/_ref).
 
-    python -m oracle.make_golden
+    [ORIANA_REFERENCE_CHECKOUT=<checkout>] python -m oracle.make_golden [seam | port | generator | nmf | ...]
 
 For each case: seeded synthetic counts (oracle.cavi_numpy.synth_counts), `np.random.seed(1)`,
 construct the reference model with `use_factors=False` (zigap.py:55-77, base.py:15-52), copy the
@@ -217,7 +217,87 @@ def write_nmf_fixture():
     refshim.release_reference()
 
 
+SEAM_CASES = [('seam_zigap', 'ZIGaP', (300, 220, 5)), ('seam_gap', 'GaP', (257, 190, 7)),
+              ('seam_zigap_tc', 'ZIGaP', (2100, 1100, 12))]      # the last: a slab the device runs on the tcgen05 kernels
+SEAM_ROWS, SEAM_D = 512, 8192          # at most this many rows of a1, a2 / b1, b2 and entries of D_hat are stored
+
+
+def seam_problem(name):
+    """Counts, initial state (the port's seeded `use_factors=False` bootstrap, oracle.cavi_numpy.init_state), number of
+    steps and the row / entry strides of the stored sample of one case of SEAM_CASES."""
+    model, (n, p, K) = {c[0]: c[1:] for c in SEAM_CASES}[name]
+    X = cn.synth_counts(n, p, K, seed=11)
+    s0 = cn.init_state(X, K, np.random.default_rng(3), model.lower())
+    strides = dict(a=-(-n // SEAM_ROWS), b=-(-p // SEAM_ROWS), D=-(-n * p // SEAM_D))
+    return model, K, X, s0, (5 if n * p < 1_000_000 else 2), strides
+
+
+def seam_digest(s0):
+    import hashlib
+    h = hashlib.sha256()
+    for k in sorted(s0):
+        h.update(k.encode()); h.update(np.ascontiguousarray(s0[k]).tobytes())
+    return h.hexdigest()
+
+
+def write_seam_fixtures():
+    """The reference stepped on its own numba Z kernel (zigap.py:79-95, gap.py:67-80): the twin that
+    tests/test_reference_seam_gpu.py steps the B200 operator against.  The test regenerates the counts and the initial
+    state from their seeds (checked by digest); the reference's state after the last step is stored on fixed strides:
+    every a-th cell, every b-th gene and every D-th entry of D_hat, row-major."""
+    import warnings
+    refshim.import_reference()
+    import oriana.models as ref_models
+    from oriana.singlecell import CountMatrix
+    for name, _, _ in SEAM_CASES:
+        model, K, X, s0, steps, st = seam_problem(name)
+        with warnings.catch_warnings():
+            warnings.simplefilter('ignore')
+            m = getattr(ref_models, model)(CountMatrix(X.copy()), k=K, use_factors=False)
+            for k, v in s0.items():
+                if k != 'X':
+                    getattr(m, k)[:] = v
+            m.update_expectations()
+            assert np.array_equal(refshim.snapshot(m)['a1'], s0['a1'])
+            for _ in range(steps):
+                m.step()
+        r = refshim.snapshot(m)
+        out = {'model': model, 'K': K, 'steps': steps, 'digest': seam_digest(s0)}
+        out.update({k: v for k, v in r.items() if v.ndim == 1})
+        out.update({k: r[k][::st[k[0]]].astype(np.float32) for k in ('a1', 'a2', 'b1', 'b2')})
+        if model == 'ZIGaP':
+            out['D_hat'] = np.asarray(m.D_hat, dtype=np.float32).ravel()[::st['D']]
+        np.savez_compressed(os.path.join(OUT, name + '.npz'), **out)
+        print(name, 'written')
+    refshim.release_reference()
+
+
+def write_port_fixture():
+    """ZIGaP 60 x 70, K = 3 from `np.random.seed(4)`: post-construction state and the state after 3 reference steps."""
+    refshim.import_reference()
+    from oriana.models import ZIGaP
+    from oriana.singlecell import CountMatrix
+    X = cn.synth_counts(60, 70, 3, seed=11)
+    np.random.seed(4)
+    m = ZIGaP(CountMatrix(X), k=3, use_factors=False)
+    out = {'model': 'ZIGaP', 'K': 3, 'steps': np.asarray([3])}
+    s0 = refshim.snapshot(m)
+    out['X'] = s0.pop('X').astype(np.int32)
+    out.update({'s0_' + k: v for k, v in s0.items()})
+    for _ in range(3):
+        m.step()
+    st = refshim.snapshot(m); st.pop('X')
+    out.update({'s3_' + k: v for k, v in st.items()})
+    np.savez_compressed(os.path.join(OUT, 'zigap_port.npz'), **out)
+    refshim.release_reference()
+    print('zigap_port written')
+
+
 def main():
+    if sys.argv[1:] == ['seam']:
+        return write_seam_fixtures()
+    if sys.argv[1:] == ['port']:
+        return write_port_fixture()
     if sys.argv[1:] == ['generator']:
         return write_generator_fixture()
     if sys.argv[1:] == ['nmf']:
@@ -313,6 +393,8 @@ def main():
     write_sparse_generator_fixture()
     write_sparse_nmf_fixture()
     write_large_k_fixtures()
+    write_seam_fixtures()
+    write_port_fixture()
 
 
 if __name__ == '__main__':

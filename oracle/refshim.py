@@ -1,14 +1,14 @@
 """Import the UNMODIFIED reference (TEST / BASELINE INFRASTRUCTURE, never on the product path).
 
 Two places hold it:
-  * `/root/reference` -- the read-only checkout, present in the build container only; `oracle/make_golden.py` records
-    the fixtures under `tests/golden/` from it;
-  * `baseline/_ref/`  -- the reference INSTALLED from that checkout by `install()` below (the base contract's recipe:
-    `pip install --no-index --no-build-isolation --no-deps --target baseline/_ref <copy of /root/reference>`; run by
-    `__graft_entry__.build()` whenever the checkout is visible).  The directory is git-ignored (not product source) but
-    travels to the GPU box with the snapshot, so `bench.py --impl reference`, `bench.py`'s `cpu_baseline` leg and
-    `tests/test_reference_seam_gpu.py` can run the reference's own `ZIGaP.step()` there.  Nothing on the GPU box reads
-    `/root/reference`.
+  * a read-only checkout of AntoinePassemiers/Oriana at CHECKOUT below ($ORIANA_REFERENCE_CHECKOUT overrides its
+    default); `oracle/make_golden.py` records the fixtures under `tests/golden/` from it;
+  * `oracle/_ref/` -- the reference INSTALLED from that checkout by `install()` below
+    (`pip install --no-index --no-build-isolation --no-deps --target oracle/_ref <copy of the checkout>`; run by
+    `__graft_entry__.build()` whenever the checkout is visible).  The directory is git-ignored (not product source); a
+    copy of the tree that carries it lets `bench.py --impl reference` and `bench.py`'s `cpu_baseline` leg run the
+    reference's own `ZIGaP.step()` on a machine without the checkout.  The test suite does not need either: it compares
+    against the fixtures.
 
 The reference pins numpy 1.13 and uses `np.float` / `np.int` (`oriana/parameters.py:11`), removed in numpy >= 1.24; the
 two-line alias below is the only change needed (SURVEY.md section 8c) -- the installed files are byte-identical to the
@@ -18,8 +18,12 @@ import os, shutil, subprocess, sys, tempfile
 import numpy as np
 
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CHECKOUT = '/root/reference'
-INSTALLED = os.path.join(_REPO, 'baseline', '_ref')
+CHECKOUT = os.environ.get('ORIANA_REFERENCE_CHECKOUT', '/root/reference')
+INSTALLED = os.path.join(_REPO, 'oracle', '_ref')
+
+
+def _checkout_present():
+    return bool(CHECKOUT) and os.path.isdir(os.path.join(CHECKOUT, 'oriana', 'models'))
 
 
 def _root():
@@ -28,7 +32,7 @@ def _root():
         return env
     if os.path.isdir(os.path.join(INSTALLED, 'oriana', 'models')):
         return INSTALLED                      # the install (byte-identical files) wins: same path here and on the GPU box
-    if os.path.isdir(os.path.join(CHECKOUT, 'oriana')):
+    if _checkout_present():
         return CHECKOUT
     return INSTALLED
 
@@ -41,9 +45,9 @@ def available():
 
 
 def install(force=False):
-    """Install the reference from the read-only checkout into baseline/_ref (no-op when the checkout is absent, e.g. on
-    the GPU box, or when the install is already there).  pip builds a wheel in the source tree, hence the /tmp copy."""
-    if not os.path.isdir(os.path.join(CHECKOUT, 'oriana')):
+    """Install the reference from the read-only checkout into oracle/_ref (no-op when the checkout is absent or when the
+    install is already there).  pip builds a wheel in the source tree, hence the temporary copy."""
+    if not _checkout_present():
         return os.path.isdir(os.path.join(INSTALLED, 'oriana'))
     if os.path.isdir(os.path.join(INSTALLED, 'oriana', 'models')) and not force:
         return True
@@ -57,7 +61,7 @@ def install(force=False):
         shutil.rmtree(INSTALLED, ignore_errors=True)
         os.makedirs(os.path.dirname(INSTALLED), exist_ok=True)
         r = subprocess.run([sys.executable, '-m', 'pip', 'install', '--no-index', '--no-build-isolation', '--no-deps',
-                            '--find-links', '/opt/wheelhouse', '--target', INSTALLED, src], capture_output=True, text=True)
+                            '--target', INSTALLED, src], capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError('pip install of the reference failed:\n' + r.stdout + r.stderr)
     return True
@@ -65,7 +69,7 @@ def install(force=False):
 
 def import_reference():
     if not available():
-        raise ImportError('reference not present at %s (neither the checkout nor baseline/_ref)' % REFERENCE_ROOT)
+        raise ImportError('reference not present at %s (neither the checkout nor oracle/_ref)' % REFERENCE_ROOT)
     np.float = float  # noqa: alias shim
     np.int = int
     sys.dont_write_bytecode = True  # the reference tree is read-only

@@ -290,9 +290,39 @@ def test_bench_initial_state_does_not_depend_on_the_sharding():
     assert bench.elbo_vs_n1('no-such-config', 1, 1, 1, -5.0) == 0.0 and bench.elbo_vs_n1('no-such-config', 1, 1, 2, -5.0) is None
 
 
+def test_bench_dump_outputs_writes_a_fixed_sample_of_the_state(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: state_dict() and the ELBO trace as float32 / float64 .npy files, the cell-side factors
+    sampled on the same cells in every run, and the cell indices beside them."""
+    import importlib.util
+    import os
+    spec = importlib.util.spec_from_file_location('bench_mod', os.path.join(ROOT, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, 'DUMP_CELLS', 64)
+    rng = np.random.default_rng(0)
+    n, p, K, r0 = 300, 40, 3, 1000
+    state = dict(a1=rng.random((n, K)), a2=rng.random((n, K)), b1=rng.random((p, K)), b2=rng.random((p, K)),
+                 alpha1=rng.random(K), pi_d=rng.random(p), iterations=7)
+
+    class Model:
+        def state_dict(self):
+            return {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in state.items()}
+    for d in ('one', 'two'):
+        bench.dump_outputs(str(tmp_path / d), Model(), np.arange(8.), n, r0)
+    names = sorted(os.listdir(tmp_path / 'one'))
+    assert names == ['a1.npy', 'a2.npy', 'alpha1.npy', 'b1.npy', 'b2.npy', 'cells.npy', 'elbo_trace.npy', 'pi_d.npy']
+    out = {f[:-4]: np.load(tmp_path / 'one' / f) for f in names}
+    for f in names:
+        assert np.array_equal(out[f[:-4]], np.load(tmp_path / 'two' / f))
+    cells = out['cells'].astype(np.int64) - r0
+    assert out['cells'].dtype == np.float64 and len(np.unique(cells)) == 64 and cells.min() >= 0 and cells.max() < n
+    assert out['a1'].dtype == np.float32 and np.array_equal(out['a1'], state['a1'][cells].astype(np.float32))
+    assert np.array_equal(out['b2'], state['b2'].astype(np.float32)) and out['pi_d'].dtype == np.float64
+
+
 def test_reference_install_is_importable_and_steps():
-    """The reference arm of bench.py and tests/test_reference_seam_gpu.py run the UNMODIFIED reference from baseline/_ref
-    (installed by __graft_entry__.build(), oracle/refshim.py): it imports under the alias shim and steps."""
+    """The reference arm of bench.py runs the UNMODIFIED reference from oracle/_ref (installed by
+    __graft_entry__.build(), oracle/refshim.py): it imports under the alias shim and steps."""
     import warnings
     from oracle import refshim, cavi_numpy as cn
     if not refshim.available():
@@ -303,7 +333,7 @@ def test_reference_install_is_importable_and_steps():
         from oriana.models import ZIGaP
         from oriana.singlecell import CountMatrix
         import oriana
-        assert 'baseline' in oriana.__file__ or 'reference' in oriana.__file__
+        assert os.path.realpath(oriana.__file__).startswith(os.path.realpath(refshim.REFERENCE_ROOT))
         with warnings.catch_warnings():
             warnings.simplefilter('ignore')
             np.random.seed(0)

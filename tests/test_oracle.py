@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN_CASES, golden_state, load_golden, relerr, relerr_quantile
-from oracle import cavi_numpy as cn, zloop, refshim
+from oracle import cavi_numpy as cn, zloop
 
 PARAMS = ('a1', 'a2', 'b1', 'b2', 'alpha1', 'alpha2', 'beta1', 'beta2')
 
@@ -70,24 +70,17 @@ def test_special_functions_against_reference_kats():
     np.testing.assert_almost_equal(cn.digamma(cn.inverse_digamma(x)), x)
 
 
-@pytest.mark.skipif(not refshim.available(), reason='reference checkout only exists in the build container')
 def test_port_matches_live_reference():
-    """Container only: run the real reference next to the port on a fresh problem (not a fixture)."""
-    refshim.import_reference()
-    try:
-        from oriana.models import ZIGaP
-        from oriana.singlecell import CountMatrix
-        X = cn.synth_counts(60, 70, 3, seed=11)
-        np.random.seed(4)
-        m = ZIGaP(CountMatrix(X), k=3, use_factors=False)
-        s = refshim.snapshot(m)
-        for _ in range(3):
-            m.step(); cn.step(s, quirk=True)
-        r = refshim.snapshot(m)
-        for k in PARAMS + ('pi_d',):
-            assert relerr(s[k], r[k]) < 2e-5, k
-    finally:
-        refshim.release_reference()     # leave the repo's alias package importable for later tests
+    """The port next to the reference's own run on a problem of its own (ZIGaP 60 x 70, K = 3, recorded by
+    oracle/make_golden.py port): 3 steps from the reference's post-construction state."""
+    g = load_golden('zigap_port')
+    s = golden_state(g, 0)
+    assert np.array_equal(s['X'], cn.synth_counts(60, 70, 3, seed=11))
+    for _ in range(3):
+        cn.step(s, quirk=True)
+    r = golden_state(g, 3)
+    for k in PARAMS + ('pi_d',):
+        assert relerr(s[k], r[k]) < 2e-5, k
 
 
 @pytest.mark.parametrize('name', ['zigap_nmf', 'gap_nmf'])

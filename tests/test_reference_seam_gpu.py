@@ -1,23 +1,23 @@
-"""GPU: the operator seam exercised INSIDE the reference's own `step()`.
+"""GPU: the operator seam exercised inside the reference's CAVI step.
 
-The unmodified reference (installed under baseline/_ref by `__graft_entry__.build()`, see oracle/refshim.py) is
-imported, and `ZIGaP.compute_Z_q_expectations` / `GaP.compute_Z_q_expectations` (zigap.py:79-95, gap.py:67-80) are
-replaced by the ctypes stubs of INTEGRATION.md section 1, i.e. by `ori_*_compute_Z_q_expectations_host` of
-liboriana_b200.so.  The reference's `update_variational_parameters` (zigap.py:97-141) then runs unchanged on host numpy
-arrays with the O(n p K) loop on the B200, and is stepped against its un-patched twin (the numba kernel) from the same
-constructed state.
+`ZIGaP.compute_Z_q_expectations` / `GaP.compute_Z_q_expectations` (zigap.py:79-95, gap.py:67-80) are replaced by the
+ctypes stubs of INTEGRATION.md section 1, i.e. by `ori_*_compute_Z_q_expectations_host` of liboriana_b200.so, called
+with host numpy arrays the way the reference calls its numba kernel.  The rest of the step is the oracle's restatement
+of the reference's `update_variational_parameters` (zigap.py:97-141, oracle/cavi_numpy.py, pinned against the
+reference by tests/test_oracle.py), so the O(n p K) loop runs on the B200 and everything else on the host.  It is
+stepped against the unmodified reference stepped on its own numba kernel from the same state (tests/golden/seam_*.npz,
+oracle/make_golden.py: the counts and the initial state are regenerated from their seeds and checked by digest).
 
 Tolerance: the reference accumulates the latent-count sums sequentially in float32; the device sums them in tiles.
 Over 5 steps the parameters agree to 2e-4 relative (floor 1e-6 max), D_hat to 2e-5 absolute on the CUDA-core kernels
 (small problems); a slab of >= 2^21 entries runs the tcgen05 kernels with TF32 operands: 2e-3 / 2e-4 after 2 steps.
 """
 import ctypes
-import warnings
 
 import numpy as np
 import pytest
 
-from conftest import relerr
+from conftest import load_golden, relerr
 
 pytestmark = pytest.mark.gpu
 
@@ -67,43 +67,38 @@ def _stubs(lib):
 
 @pytest.mark.parametrize('model_name,shape', [('ZIGaP', (300, 220, 5)), ('GaP', (257, 190, 7)),
                                               ('ZIGaP', (2100, 1100, 12))])     # the last: tensor-path sized slab
-def test_reference_step_with_the_b200_operator(cuda_lib, model_name, shape):
-    from oracle import refshim, cavi_numpy as cn
-    if not refshim.available():
-        pytest.skip('the reference install (baseline/_ref) did not travel: run __graft_entry__.build() in the container')
-    n, p, K = shape
-    X = cn.synth_counts(n, p, K, seed=11)
-    refshim.import_reference()
-    try:
-        import oriana.models as ref_models
-        from oriana.singlecell import CountMatrix
-        cls = getattr(ref_models, model_name)
-        original = cls.__dict__['compute_Z_q_expectations']
-        with warnings.catch_warnings():
-            warnings.simplefilter('ignore')
-            np.random.seed(3)
-            twin = cls(CountMatrix(X.copy()), k=K, use_factors=False)      # un-patched: numba kernel
-            np.random.seed(3)
-            ours = cls(CountMatrix(X.copy()), k=K, use_factors=False)
-            for k in ('a1', 'a2', 'b1', 'b2'):
-                assert np.array_equal(getattr(twin, k)[:], getattr(ours, k)[:])
-            zigap_z, gap_z, calls = _stubs(cuda_lib)
-            steps = 5 if n * p < 1_000_000 else 2
-            for _ in range(steps):
-                twin.step()
-            try:
-                cls.compute_Z_q_expectations = staticmethod(zigap_z if model_name == 'ZIGaP' else gap_z)
-                for _ in range(steps):
-                    ours.step()
-            finally:
-                cls.compute_Z_q_expectations = original
-        assert calls['zigap' if model_name == 'ZIGaP' else 'gap'] == steps
-        names = ('a1', 'a2', 'b1', 'b2', 'alpha1', 'alpha2', 'beta1', 'beta2') + (('pi_d',) if model_name == 'ZIGaP' else ())
-        tensor = n * p >= (1 << 21)          # slabs of this size run the tcgen05 kernels: TF32 operands (measured 3.5e-4)
-        for k in names:
-            e = relerr(getattr(ours, k)[:], getattr(twin, k)[:])
-            assert e < (2e-3 if tensor else 2e-4), (model_name, k, e)
-        if model_name == 'ZIGaP':
-            assert np.max(np.abs(ours.D_hat - twin.D_hat)) < (2e-4 if tensor else 2e-5)
-    finally:
-        refshim.release_reference()
+def test_reference_step_with_the_b200_operator(cuda_lib, monkeypatch, model_name, shape):
+    from oracle import cavi_numpy as cn, make_golden as mg
+    name = {(300, 220, 5): 'seam_zigap', (257, 190, 7): 'seam_gap', (2100, 1100, 12): 'seam_zigap_tc'}[shape]
+    model, K, X, s, steps, st = mg.seam_problem(name)
+    assert model == model_name and K == shape[2]
+    g = load_golden(name)
+    assert mg.seam_digest(s) == str(g['digest']) and steps == int(g['steps'])
+    zigap_z, gap_z, calls = _stubs(cuda_lib)
+
+    def device_z(log_U_hat, log_V_hat, X, D_hat=None, quirk=True, dtype=np.float32):
+        # the reference's call: outputs allocated by the caller, X[:] as a column-major float32 copy (zigap.py:102-111)
+        assert quirk and dtype == np.float32
+        n, K = log_U_hat.shape
+        p = log_V_hat.shape[0]
+        Zi, Zj = np.empty((n, K), np.float32), np.empty((p, K), np.float32)
+        X32 = np.asfortranarray(X, dtype=np.float32)
+        if D_hat is None:
+            gap_z(Zi, Zj, log_U_hat, log_V_hat, X32)
+        else:
+            zigap_z(Zi, Zj, np.empty((p, K), np.float32), log_U_hat, log_V_hat, D_hat, X32)
+        return Zi, Zj
+
+    monkeypatch.setattr(cn, 'z_expectations', device_z)
+    for _ in range(steps):
+        cn.step(s, quirk=True)
+    assert calls['zigap' if model_name == 'ZIGaP' else 'gap'] == steps
+    names = ('a1', 'a2', 'b1', 'b2', 'alpha1', 'alpha2', 'beta1', 'beta2') + (('pi_d',) if model_name == 'ZIGaP' else ())
+    tensor = X.size >= (1 << 21)         # slabs of this size run the tcgen05 kernels: TF32 operands (measured 3.5e-4)
+    for k in names:
+        got = s[k][::st[k[0]]] if s[k].ndim == 2 else s[k]
+        e = relerr(got, g[k])
+        assert e < (2e-3 if tensor else 2e-4), (model_name, k, e)
+    if model_name == 'ZIGaP':
+        D = s['p_d'].astype(np.float32).ravel()[::st['D']]
+        assert np.max(np.abs(D - g['D_hat'])) < (2e-4 if tensor else 2e-5)
