@@ -22,122 +22,44 @@
 // hence the transposed copies (prepared by k_tc_prep_*) and K-major descriptors everywhere
 // (scripts/tc_probe.cu checks every descriptor form used here against the CPU).
 //
-// CTA pairs (PAIR, the default): two CTAs of a cluster sweep the same chunk with neighbouring own tiles; every MMA
-// is a cta_group::2 instruction of M = 256 issued by the pair's leader, each CTA stages only half of every
-// streamed operand tile and TMA credits both halves to the leader's barrier; completion is multicast back.
+// CTA pairs: two CTAs of a cluster sweep the same chunk with neighbouring own tiles; every MMA is a cta_group::2
+// instruction of M = 256 issued by the pair's leader, each CTA stages only half of every streamed operand tile and
+// TMA credits both halves to the leader's barrier; completion is multicast back.
 //
 // Warp roles (320 threads):
 //   warp 0       TMA producer (whole warp walks the rings, one elected lane issues)
 //   warp 1       MMA issuer + TMEM owner (warp-uniform control flow, one elected lane issues)
 //   warps 2..9   element-wise warps; warp w owns TMEM lanes 32*(w%4).. and half of the tile's columns
-#include <cstdlib>
 #include <cstring>
-#include <type_traits>
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
 namespace ori {
 using namespace tc;
 
-// knock-out switches of the element-wise stage: timing experiments only (WRONG results), never set in the product build
-#ifndef ORI_KO_DMIN
-#define ORI_KO_DMIN 0
-#endif
-#ifndef ORI_KO_ULIM
-#define ORI_KO_ULIM 0
-#endif
-#ifndef ORI_KO_BIAS
-#define ORI_KO_BIAS 0
-#endif
-#ifndef ORI_KO_CS
-#define ORI_KO_CS 0
-#endif
-#ifndef ORI_KO_LG2
-#define ORI_KO_LG2 0
-#endif
-#ifndef ORI_KO_ENT2
-#define ORI_KO_ENT2 0
-#endif
-#ifndef ORI_KO_LDUV
-#define ORI_KO_LDUV 0      // skip the tcgen05.ld of the uv tile
-#endif
-#ifndef ORI_KO_STD
-#define ORI_KO_STD 0       // skip the tcgen05.st of the D_hat tile
-#endif
-#ifndef ORI_KO_TMA
-#define ORI_KO_TMA 0       // the producer issues one K box, one T box and no logit(pi) loads per tile (is it the floor?)
-#endif
-#ifndef ORI_KO_MATH
-#define ORI_KO_MATH 0      // no element-wise math at all: den / uv go back as they came
-#endif
-#ifndef ORI_TC_SPLIT
-#define ORI_TC_SPLIT 0     // 1 (with ORI_TC_NEW=16): the 16 element-wise warps form two groups of 8; group g takes the tiles of
-                           //    parity g (= TMEM stage g), 32 columns per warp, single register buffer.  While one group waits
-                           //    for its next S (behind its own P), the other group's tile keeps the sub-partition busy.
-#endif
-#ifndef ORI_TC_PROF
-#define ORI_TC_PROF 0      // 1: phase timers (clock()) in the element-wise warps and the MMA issuer of CTA 0 / 1, printed at the end
-                           //    of every launch (scripts/gpu_time_models.py quick; never in the product build)
-#endif
-#if ORI_TC_PROF
-#define PF_CLK(v) const uint32_t v = (uint32_t)clock()
-#define PF_ADD(acc, t1, t0) acc += (t1) - (t0)
-#else
-#define PF_CLK(v)
-#define PF_ADD(acc, t1, t0)
-#endif
-#ifndef ORI_TC_BF16X
-#define ORI_TC_BF16X 1     // 1: the two cross terms hi.lo + lo.hi of every 3xTF32 contraction run as ONE bf16 chain over
-                           //    [hi | lo] . [lo | hi] (error 2^-9 of a 2^-12 term): 4 instead of 6 MMA chains per tile
-#endif
-
 constexpr int TC_OWN = 128;
-#ifndef ORI_TC_NEW
-#define ORI_TC_NEW 8
-#endif
-constexpr int NEW = ORI_TC_NEW;       // element-wise warps: 8 (168 registers each) or 16 (96 registers, one column group per tile)
-constexpr int SLICES = NEW / 4;       // element-wise warps per TMEM lane quarter
-constexpr int ASUBS = SLICES / 2;     // warps sharing one own-side array / one accumulator
-#ifndef ORI_TC_ISSUERS
-#define ORI_TC_ISSUERS 1   // MMA-issuing warps.  2 = the den -> acc1 chain and the uv -> acc2 chain of a ZIGaP tile are issued by
-                           // two warps (disjoint TMEM columns, no ordering needed between them).  Measured SLOWER (250k x 20k,
-                           // K = 32: rows 5.24 vs 4.91 ms, no-math floor 4.13 vs 3.80 ms): kept as an experiment switch.
-#endif
-constexpr int NISS = ORI_TC_ISSUERS;
-constexpr int ISS2_WARP = 2 + NEW;    // the second issuer sits after the element-wise warps (quarter = warp & 3 stays valid)
-constexpr int TC_THREADS = 64 + 32 * NEW + (NISS == 2 ? 32 : 0);
-constexpr bool SPLIT = ORI_TC_SPLIT != 0;
-static_assert(!SPLIT || NEW == 16, "ORI_TC_SPLIT needs ORI_TC_NEW=16");
-constexpr int NEWT = SPLIT ? NEW / 2 : NEW;   // element-wise warps that work on one tile
+constexpr int NEW = 8;                // element-wise warps, two per TMEM lane quarter
+constexpr int TC_THREADS = 64 + 32 * NEW;
+constexpr int NCTA = 2;               // CTAs of a cluster (pair)
 
-// Plan of one kernel variant.  KP: padded latent dimension (32 or 64).  PAIR: the CTA-pair variant (cta_group::2,
-// M = 256 over two SMs): each CTA stages only half of every streamed operand tile (the pair's MMA reads both
-// halves), which halves the TMA fill and the tensor-core operand reads per SM and leaves room for deeper rings.
-#ifndef ORI_TC_DEEP
-#define ORI_TC_DEEP 0      // 1: KP = 32 runs 32-wide sweep tiles on a 4-deep TMEM pipeline (S three tiles ahead of the
-                           //    element-wise warps, which prefetch the next tile and defer their hand-off by one tile: no
-                           //    hand-off latency is exposed).  Measured SLOWER (250k x 20k, K = 32: rows 6.54 vs 4.89 ms, genes
-                           //    8.48 vs 6.86 ms; without any element-wise math 5.64 vs 3.80 ms): a tcgen05.mma of N <= 64 costs
-                           //    ~45 cycles of issue whatever its N, and 32-wide tiles need 48 instead of 32 of them per 64
-                           //    sweep entries.  0 (default): 64-wide tiles, 2 TMEM stages, two groups per warp and tile.
-#endif
-
+// Plan of one kernel variant.  KP: padded latent dimension (32 or 64).  The CTA pair (cta_group::2, M = 256 over two
+// SMs) stages only half of every streamed operand tile per CTA (the pair's MMA reads both halves), which halves the TMA
+// fill and the tensor-core operand reads per SM and leaves room for deeper rings.
+// The cross terms hi.lo + lo.hi of every 3xTF32 contraction run as ONE bf16 chain over [hi | lo] . [lo | hi] (error
+// 2^-9 of a 2^-12 term): 4 instead of 6 MMA chains per tile.
+//
 // PRECISE (KP = 32): the accumulating contractions R . S1 and D . S2 are split-precision too -- R, D and the factor operands
 // as tf32 hi plus a bf16 [hi | lo] . [lo | hi] chain for the two cross terms, like den / uv -- so every sum is fp32-grade
 // (~2^-21) instead of TF32-grade (~2^-12 per term).  The tile keeps R16 / D16 (the packed bf16 pairs) beside R / D in TMEM,
 // which halves the sweep width (32) to stay inside 512 columns.
-template <int KP, bool PAIR, bool PRECISE = false, bool DEVI = false>
+template <int KP, bool PRECISE = false, bool DEVI = false>
 struct Cfg {
     static_assert(KP == 32 || KP == 64, "tensor path: KP is 32 or 64");
     static_assert(!PRECISE || KP == 32, "the fp32-grade plan exists for KP = 32");
-    static constexpr int NCTA = PAIR ? 2 : 1;
-    static constexpr bool DEEP = (ORI_TC_DEEP != 0) && KP == 32 && !PRECISE;
-    static constexpr int SW = (DEEP || PRECISE) ? 32 : 2048 / KP;   // sweep entries per tile
-    static constexpr int NS = DEEP ? 4 : 2;               // TMEM stages of [den/R | uv/D]
+    static constexpr int SW = PRECISE ? 32 : 2048 / KP;   // sweep entries per tile
+    static constexpr int NS = 2;                          // TMEM stages of [den/R | uv/D]
     static constexpr int KB = KP / 32;                    // 128-byte K blocks of a K-major row
-    static constexpr int KST = DEEP ? 4 : (PAIR ? 3 : 2); // ring depths
-    static constexpr int TST = DEEP ? 4 : (PAIR ? 3 : 2);
-    static constexpr int XST = DEEP ? (PAIR ? 8 : 6) : (PAIR ? 4 : 3);
+    static constexpr int KST = 3, TST = 3, XST = 4;       // ring depths
     static constexpr int NTA = PRECISE ? 4 : 2;           // transposed operand arrays per stage: e, E [, bf16 pairs of e, of E]
     // K-major operand array of one tile: [KB blocks][SW / NCTA sweep rows][32 floats], 128-byte swizzled
     static constexpr uint32_t K_BLK = (SW / NCTA) * 128;
@@ -164,7 +86,7 @@ struct Cfg {
     static constexpr uint32_t TM_A = TM_ACC + 2 * KP;
     static constexpr uint32_t TM_COLS = 512;
     static_assert(TM_A + 4 * KP <= TM_COLS, "TMEM plan");
-    // mbarriers.  With PAIR, KFULL / TFULL / PREADY / ACC_FREE / A_READY are used in the leader CTA only
+    // mbarriers.  KFULL / TFULL / PREADY / ACC_FREE / A_READY are used in the leader CTA only
     // (the peer's TMA bytes and warp arrivals are credited there); the others are per CTA.
     static constexpr int B_KFULL = 0, B_KEMPTY = B_KFULL + KST, B_TFULL = B_KEMPTY + KST, B_TEMPTY = B_TFULL + TST,
                          B_XFULL = B_TEMPTY + TST, B_XEMPTY = B_XFULL + XST, B_SREADY = B_XEMPTY + XST,
@@ -179,7 +101,7 @@ struct TcMaps { CUtensorMap swK, swT, X; };
 struct TcArgs {
     long long own_total, sw_total;   // valid extents (cells / genes)
     long long sw_pad;                // padded sweep extent (multiple of 128): q-th operand array starts at row q*pad
-    int n_own_tiles, n_own_units, n_chunks, tiles_per_chunk, n_sw_tiles, n_items;   // unit = own tile (pair of own tiles with PAIR)
+    int n_own_tiles, n_own_units, n_chunks, tiles_per_chunk, n_sw_tiles, n_items;   // unit = pair of own tiles
     const float* own_e;              // [own_total x KP] exp(E log .) of the own side (raw factor array)
     const float* own_E;              // [own_total x KP] E[.] of the own side
     const float* lp2w;               // [genes_pad] logit(pi) * log2(e); -inf: D_hat = (X>0)
@@ -257,9 +179,9 @@ __device__ __forceinline__ void kahan_add(float& s, float& c, float v) {
 constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
 
-// Walks the tiles of the work items of this CTA (pair): item = chunk * n_own_units + own_unit (chunk-major, so
-// that the CTAs running at the same time sweep the same chunk and share its operands in L2).  With PAIR the two
-// CTAs of a cluster walk the same items; CTA `rank` owns own tile 2 * own_unit + rank.
+// Walks the tiles of the work items of this CTA pair: item = chunk * n_own_units + own_unit (chunk-major, so
+// that the CTAs running at the same time sweep the same chunk and share its operands in L2).  The two CTAs of a
+// cluster walk the same items; CTA `rank` owns own tile 2 * own_unit + rank.
 struct TileIter {
     int item, stride, t, t_begin, t_end, own0, ncta, rank;
     __device__ __forceinline__ void load(const TcArgs& a) {
@@ -288,20 +210,13 @@ struct TileIter {
 // loop cost the plain kernels 7 % (row pass) / 3 % (gene pass) when the hooks were runtime-switched.
 // DET: the ORI_F_DETERMINISTIC epilogue (TcArgs::tickets / item_part), a separate instantiation for the same reason (runtime-
 // switched it cost the plain kernels 2.6 % / 3.4 %).
-template <bool GENES, bool DROPOUT, bool ELBO, bool PAIR, int KP, bool PRECISE, bool DEVI = false, bool UFL = false, bool DET = false>
-#ifndef ORI_TC_MAXNREG
-#define ORI_TC_MAXNREG 96
-#endif
-#if ORI_TC_NEW == 16
-__global__ void __maxnreg__(ORI_TC_MAXNREG)
-#else
+template <bool GENES, bool DROPOUT, bool ELBO, int KP, bool PRECISE, bool DEVI = false, bool UFL = false, bool DET = false>
 __global__ void __launch_bounds__(TC_THREADS, 1)
-#endif
 k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
 {
-    using C = Cfg<KP, PAIR, PRECISE, DEVI>;
+    using C = Cfg<KP, PRECISE, DEVI>;
     static_assert(!DEVI || (!GENES && DROPOUT && !ELBO && !PRECISE), "deviance pass: row orientation, two contractions");
-    constexpr int NCTA = C::NCTA, SW = C::SW, NS = C::NS;
+    constexpr int SW = C::SW, NS = C::NS;
     constexpr uint32_t TM_UV = C::TM_UV;
     constexpr int KST = C::KST, TST = C::TST, XST = C::XST;
     constexpr uint32_t K_STAGE = C::K_STAGE, T_STAGE = C::T_STAGE, X_STAGE = C::X_STAGE, LP_STAGE = C::LP_STAGE;
@@ -310,11 +225,11 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
     constexpr int B_KFULL = C::B_KFULL, B_KEMPTY = C::B_KEMPTY, B_TFULL = C::B_TFULL, B_TEMPTY = C::B_TEMPTY,
                   B_XFULL = C::B_XFULL, B_XEMPTY = C::B_XEMPTY, B_SREADY = C::B_SREADY, B_PREADY = C::B_PREADY,
                   B_ACC_READY = C::B_ACC_READY, B_ACC_FREE = C::B_ACC_FREE, B_A_READY = C::B_A_READY, NBARS = C::NBARS;
-    constexpr int CW = SW / (SPLIT ? SLICES / 2 : SLICES);   // tile columns per element-wise warp: 32 or 16
+    constexpr int CW = SW / 2;                // tile columns per element-wise warp: 32 or 16
     constexpr int G = CW / 16;                // groups of 16 columns per tile for one warp
     constexpr int NQ = DROPOUT ? 4 : 2;       // K-major operand arrays in use
     constexpr int NT = DROPOUT ? 2 : 1;       // transposed operand arrays in use
-    const int rank = PAIR ? (int)cluster_ctarank() : 0;      // CTA of the pair; rank 0 leads (issues every MMA)
+    const int rank = (int)cluster_ctarank();  // CTA of the pair; rank 0 leads (issues every MMA)
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -323,20 +238,19 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
-        constexpr int NI = (NISS == 2 && DROPOUT) ? 2 : 1;      // issuers at work: each commits once per stage
-        for (int s = 0; s < KST; ++s) { mbar_init(&bars[B_KFULL + s], 1); mbar_init(&bars[B_KEMPTY + s], NI); }
-        for (int s = 0; s < TST; ++s) { mbar_init(&bars[B_TFULL + s], 1); mbar_init(&bars[B_TEMPTY + s], NI); }
-        for (int s = 0; s < XST; ++s) { mbar_init(&bars[B_XFULL + s], 1); mbar_init(&bars[B_XEMPTY + s], NEWT); }
-        for (int s = 0; s < NS; ++s) { mbar_init(&bars[B_SREADY + s], NI); mbar_init(&bars[B_PREADY + s], NEWT * NCTA); }
-        mbar_init(&bars[B_ACC_READY], NI);
+        for (int s = 0; s < KST; ++s) { mbar_init(&bars[B_KFULL + s], 1); mbar_init(&bars[B_KEMPTY + s], 1); }
+        for (int s = 0; s < TST; ++s) { mbar_init(&bars[B_TFULL + s], 1); mbar_init(&bars[B_TEMPTY + s], 1); }
+        for (int s = 0; s < XST; ++s) { mbar_init(&bars[B_XFULL + s], 1); mbar_init(&bars[B_XEMPTY + s], NEW); }
+        for (int s = 0; s < NS; ++s) { mbar_init(&bars[B_SREADY + s], 1); mbar_init(&bars[B_PREADY + s], NEW * NCTA); }
+        mbar_init(&bars[B_ACC_READY], 1);
         mbar_init(&bars[B_ACC_FREE], NEW * NCTA);
         mbar_init(&bars[B_A_READY], NEW * NCTA);
         fence_barrier_init();
     }
-    if (warp == 1) { if (PAIR) tmem_alloc_pair(tmem_slot, TM_COLS); else tmem_alloc(tmem_slot, TM_COLS); }
+    if (warp == 1) tmem_alloc_pair(tmem_slot, TM_COLS);
     tc_fence_before();
     __syncthreads();
-    if (PAIR) cluster_sync_all();          // both CTAs' barriers are initialised before any remote arrive / TMA credit
+    cluster_sync_all();                    // both CTAs' barriers are initialised before any remote arrive / TMA credit
     tc_fence_after();
     const uint32_t tmem = *tmem_slot;
 
@@ -359,20 +273,18 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                 uint8_t* st = smem + OFF_T + s * T_STAGE;
                 uint64_t* bar = &bars[B_TFULL + s];
                 const int sw0 = it_.t * SW;
-                constexpr int NTL = ORI_KO_TMA ? 1 : NT;
                 constexpr int NTP = PRECISE ? 2 : 1;                            // + the bf16 [lo | hi] pairs of each array
-                if (rank == 0) mbar_expect_tx(bar, NTP * NTL * C::T_ARR * NCTA);      // the whole pair's bytes land on the leader's barrier
+                if (rank == 0) mbar_expect_tx(bar, NTP * NT * C::T_ARR * NCTA);       // the whole pair's bytes land on the leader's barrier
 #pragma unroll
                 for (int h = 0; h < NTP; ++h)
 #pragma unroll
-                    for (int q0 = 0; q0 < NTL; ++q0)
+                    for (int q0 = 0; q0 < NT; ++q0)
 #pragma unroll
                         for (int c = 0; c < SW / 32; ++c) {
                             const int q = 2 * h + q0;                               // slot in the stage = array in global memory
                             uint8_t* dst = st + q * C::T_ARR + c * C::T_CHUNK;
                             const int row = q * KP + (KP / NCTA) * rank;            // this CTA's latent rows of array q
-                            if (PAIR) tma_load_2d_pair(dst, &maps.swT, bar, sw0 + 32 * c, row, L2_EVICT_LAST);
-                            else tma_load_2d_hint(dst, &maps.swT, bar, sw0 + 32 * c, row, L2_EVICT_LAST);
+                            tma_load_2d_pair(dst, &maps.swT, bar, sw0 + 32 * c, row, L2_EVICT_LAST);
                         }
             }
             __syncwarp();
@@ -386,16 +298,14 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     uint8_t* st = smem + OFF_K + s * K_STAGE;
                     uint64_t* bar = &bars[B_KFULL + s];
                     const int sw0 = ik.t * SW;
-                    constexpr int NQL = ORI_KO_TMA ? 1 : NQ;
-                    if (rank == 0) mbar_expect_tx(bar, NQL * C::K_ARR * NCTA);
+                    if (rank == 0) mbar_expect_tx(bar, NQ * C::K_ARR * NCTA);
 #pragma unroll
-                    for (int q = 0; q < NQL; ++q)
+                    for (int q = 0; q < NQ; ++q)
 #pragma unroll
                         for (int kb = 0; kb < C::KB; ++kb) {
                             uint8_t* dst = st + q * C::K_ARR + kb * C::K_BLK;
                             const int row = (int)(q * a.sw_pad + sw0 + (SW / NCTA) * rank);   // this CTA's sweep rows
-                            if (PAIR) tma_load_2d_pair(dst, &maps.swK, bar, 32 * kb, row, L2_EVICT_LAST);
-                            else tma_load_2d_hint(dst, &maps.swK, bar, 32 * kb, row, L2_EVICT_LAST);
+                            tma_load_2d_pair(dst, &maps.swK, bar, 32 * kb, row, L2_EVICT_LAST);
                         }
                 }
                 __syncwarp();
@@ -407,13 +317,13 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     uint8_t* st = smem + OFF_X + s * X_STAGE;
                     uint64_t* bar = &bars[B_XFULL + s];
                     const int sw0 = ik.t * SW;
-                    mbar_expect_tx(bar, X_STAGE + ((!GENES && DROPOUT && !ORI_KO_TMA) ? LP_STAGE : 0));
+                    mbar_expect_tx(bar, X_STAGE + ((!GENES && DROPOUT) ? LP_STAGE : 0));
                     if (DEVI) bulk_load(smem + OFF_LP + s * LP_STAGE, a.devlp + (long long)ik.t * (8 * SW), LP_STAGE, bar);
                     if (!GENES) {          // [128 cells][32 genes] boxes
 #pragma unroll
                         for (int c = 0; c < SW / 32; ++c)
                             tma_load_2d_hint(st + c * (TC_OWN * 128), &maps.X, bar, sw0 + 32 * c, ik.own0, L2_EVICT_FIRST);
-                        if (DROPOUT && !ORI_KO_TMA && !DEVI) {
+                        if (DROPOUT && !DEVI) {
                             bulk_load(smem + OFF_LP + s * LP_STAGE, a.lp2w + sw0, SW * 4, bar);
                             bulk_load(smem + OFF_LP + s * LP_STAGE + SW * 4, a.flw + sw0, SW * 4, bar);
                             bulk_load(smem + OFF_LP + s * LP_STAGE + SW * 8, a.cw + sw0, SW * 4, bar);
@@ -430,45 +340,33 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             ++nk; ik.next(a);
         }
         if (nk > 0) load_T();
-    } else if (warp == 1 || (NISS == 2 && warp == ISS2_WARP)) {
-        // ============================================ MMA issuer(s) ============================================
-        // Two issuers (ZIGaP): warp 1 issues the den chains and the R . S1 accumulation, the second issuer the uv chains
-        // and the D . S2 accumulation -- disjoint TMEM columns, so the two streams need no ordering between them.
+    } else if (warp == 1 || false) {      // `|| false` (and the mma / commit lambdas below) only fix the block layout
+                                          // nvcc picks: written plainly, some instances compile to a different schedule
+        // ============================================ MMA issuer ============================================
         // Warp-uniform control flow, one elected lane issues: descriptors and TMEM addresses stay in uniform
         // registers (a divergent single-lane loop makes the compiler wrap every tcgen05.mma in a
         // register->uniform-register broadcast loop, which throttles the issue rate).
-        // With PAIR only the leader CTA issues: cta_group::2 MMAs of M = 256 span both CTAs' TMEM and read each
-        // CTA's half of the B tile; completion is multicast to the barriers of both CTAs.
-        const bool two = (NISS == 2) && DROPOUT;
-        const int iss = (warp == 1) ? 0 : 1;
-        const bool do_den = !two || iss == 0, do_uv = DROPOUT && (!two || iss == 1);
-        if ((!PAIR || rank == 0) && (iss == 0 || two)) {
+        // Only the leader CTA issues: cta_group::2 MMAs of M = 256 span both CTAs' TMEM and read each CTA's half
+        // of the B tile; completion is multicast to the barriers of both CTAs.
+        if (rank == 0) {
             constexpr uint32_t idescS = make_idesc_tf32(TC_OWN * NCTA, SW, false, false);
             constexpr uint32_t idescP = make_idesc_tf32(TC_OWN * NCTA, KP, false, false);
+            constexpr uint32_t idescS16 = make_idesc_bf16(TC_OWN * NCTA, SW);
             const uint32_t sbase = smem_u32(smem);
             const uint64_t kdesc0 = make_smem_desc(sbase + OFF_K, 16, 1024);
             const uint64_t tdesc0 = make_smem_desc(sbase + OFF_T, 16, 1024);
             auto mma = [&](uint32_t d, uint32_t at, uint64_t bd, uint32_t idesc, bool acc) {
-                if (PAIR) mma_tf32_ts_pair(d, at, bd, idesc, acc); else mma_tf32_ts(d, at, bd, idesc, acc);
+                mma_tf32_ts_pair(d, at, bd, idesc, acc);
             };
             auto mma16 = [&](uint32_t d, uint32_t at, uint64_t bd, uint32_t idesc, bool acc) {
-                if (PAIR) mma_bf16_ts_pair(d, at, bd, idesc, acc); else mma_bf16_ts(d, at, bd, idesc, acc);
+                mma_bf16_ts_pair(d, at, bd, idesc, acc);
             };
-            constexpr uint32_t idescS16 = make_idesc_bf16(TC_OWN * NCTA, SW);
-            (void)idescS16; (void)mma16;
-            auto commit = [&](uint64_t* bar) { if (PAIR) tc_commit_pair(bar); else tc_commit(bar); };
-#if ORI_TC_PROF
-            uint32_t pm_pready = 0, pm_tfull = 0, pm_issP = 0, pm_kfull = 0, pm_issS = 0;
-            const uint32_t pm_begin = (uint32_t)clock();
-#endif
+            auto commit = [&](uint64_t* bar) { tc_commit_pair(bar); };
             auto issue_P = [&](uint32_t it, bool first, bool last, int li) {
                 const uint32_t s = it % NS, ts = it % TST;
-                PF_CLK(pq0);
                 mbar_wait(&bars[B_PREADY + s], (it / NS) & 1, 20);
-                PF_CLK(pq1); PF_ADD(pm_pready, pq1, pq0);
                 mbar_wait(&bars[B_TFULL + ts], (it / TST) & 1, 24);
                 if (first) mbar_wait(&bars[B_ACC_FREE], (li & 1) ^ 1, 21);
-                PF_CLK(pq2); PF_ADD(pm_tfull, pq2, pq1);
                 tc_fence_after();
                 if (elect_one()) {
                     const uint64_t td = tdesc0 + (uint64_t)((ts * T_STAGE) >> 4);
@@ -478,10 +376,9 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     // their throughput)
 #pragma unroll
                     for (int ks = 0; ks < SW / 8; ++ks) {
-                        if (do_den)
-                            mma(tmem + TM_ACC, tmem + s * TM_STAGE + ks * 8,
-                                td + (uint64_t)(((ks >> 2) * C::T_CHUNK + (ks & 3) * 32) >> 4), idescP, !(first && ks == 0));
-                        if (do_uv)
+                        mma(tmem + TM_ACC, tmem + s * TM_STAGE + ks * 8,
+                            td + (uint64_t)(((ks >> 2) * C::T_CHUNK + (ks & 3) * 32) >> 4), idescP, !(first && ks == 0));
+                        if (DROPOUT)
                             mma(tmem + TM_ACC + KP, tmem + s * TM_STAGE + TM_UV + ks * 8,
                                 td + (uint64_t)((C::T_ARR + (ks >> 2) * C::T_CHUNK + (ks & 3) * 32) >> 4), idescP,
                                 !(first && ks == 0));
@@ -492,10 +389,9 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                         constexpr uint32_t idescP16 = make_idesc_bf16(TC_OWN * NCTA, KP);
 #pragma unroll
                         for (int ks = 0; ks < SW / 8; ++ks) {
-                            if (do_den)
-                                mma16(tmem + TM_ACC, tmem + s * TM_STAGE + SW + ks * 8,
-                                      td + (uint64_t)((2 * C::T_ARR + (ks >> 2) * C::T_CHUNK + (ks & 3) * 32) >> 4), idescP16, true);
-                            if (do_uv)
+                            mma16(tmem + TM_ACC, tmem + s * TM_STAGE + SW + ks * 8,
+                                  td + (uint64_t)((2 * C::T_ARR + (ks >> 2) * C::T_CHUNK + (ks & 3) * 32) >> 4), idescP16, true);
+                            if (DROPOUT)
                                 mma16(tmem + TM_ACC + KP, tmem + s * TM_STAGE + TM_UV + SW + ks * 8,
                                       td + (uint64_t)((3 * C::T_ARR + (ks >> 2) * C::T_CHUNK + (ks & 3) * 32) >> 4), idescP16, true);
                         }
@@ -504,7 +400,6 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     if (last) commit(&bars[B_ACC_READY]);
                 }
                 __syncwarp();
-                PF_CLK(pq3); PF_ADD(pm_issP, pq3, pq2);
             };
             // S runs NS - 1 tiles ahead of P: S(it) overwrites the TMEM stage P(it - NS) has read (the tensor pipe executes in
             // issue order), so each loop iteration issues S(it) and then P(it - (NS - 1)); `tp` trails `ti` for the latter
@@ -524,91 +419,65 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             while (ti.valid(a)) {
                 const uint32_t s = it % NS, ks_ = it % KST;
                 const bool first = ti.first(), last = ti.last();
-                PF_CLK(pr0);
                 mbar_wait(&bars[B_KFULL + ks_], (it / KST) & 1, 23);
                 if (first) mbar_wait(&bars[B_A_READY], li & 1, 22);
-                PF_CLK(pr1); PF_ADD(pm_kfull, pr1, pr0);
                 tc_fence_after();
                 if (elect_one()) {
                     const uint64_t kd = kdesc0 + (uint64_t)((ks_ * K_STAGE) >> 4);
-                    // den (and uv) of this tile: three tf32 products per contraction, A operand from TMEM;
-                    // contraction over the KP latent components, 8 per MMA: K block kk / 4, 32 bytes per step
-#define ORI_CHAIN(D_, QA, QB, FRESH)                                                                              \
+                    // den (and uv) of this tile: hi.hi in tf32, A operand from TMEM; contraction over the KP latent
+                    // components, 8 per MMA: K block kk / 4, 32 bytes per step
+#define ORI_CHAIN(D_, Q)                                                                                          \
                     _Pragma("unroll") for (int kk = 0; kk < KP / 8; ++kk)                                         \
-                        mma((D_), tmem + TM_A + (QA) * KP + kk * 8,                                               \
-                            kd + (uint64_t)(((QB) * C::K_ARR + (kk >> 2) * C::K_BLK + (kk & 3) * 32) >> 4), idescS, \
-                            !((FRESH) && kk == 0))
-#if ORI_TC_BF16X
+                        mma((D_), tmem + TM_A + (Q) * KP + kk * 8,                                                \
+                            kd + (uint64_t)(((Q) * C::K_ARR + (kk >> 2) * C::K_BLK + (kk & 3) * 32) >> 4), idescS, kk != 0)
                     // arrays 1 and 3 hold bf16 pairs: own side [hi | lo], sweep side [lo | hi] (2 KP elements, the
                     // same bytes and the same 8-column / 32-byte steps as a tf32 array)
 #define ORI_CHAIN16(D_, Q)                                                                                        \
                     _Pragma("unroll") for (int kk = 0; kk < KP / 8; ++kk)                                         \
                         mma16((D_), tmem + TM_A + (Q) * KP + kk * 8,                                              \
                               kd + (uint64_t)(((Q) * C::K_ARR + (kk >> 2) * C::K_BLK + (kk & 3) * 32) >> 4), idescS16, true)
-                    if (do_den) {
-                        ORI_CHAIN(tmem + s * TM_STAGE, 0, 0, true);
-                        ORI_CHAIN16(tmem + s * TM_STAGE, 1);
-                    }
-                    if (do_uv) {
-                        ORI_CHAIN(tmem + s * TM_STAGE + TM_UV, 2, 2, true);
+                    ORI_CHAIN(tmem + s * TM_STAGE, 0);
+                    ORI_CHAIN16(tmem + s * TM_STAGE, 1);
+                    if (DROPOUT) {
+                        ORI_CHAIN(tmem + s * TM_STAGE + TM_UV, 2);
                         ORI_CHAIN16(tmem + s * TM_STAGE + TM_UV, 3);
                     }
 #undef ORI_CHAIN16
-#else
-                    if (do_den) {
-                        ORI_CHAIN(tmem + s * TM_STAGE, 0, 0, true);
-                        ORI_CHAIN(tmem + s * TM_STAGE, 0, 1, false);
-                        ORI_CHAIN(tmem + s * TM_STAGE, 1, 0, false);
-                    }
-                    if (do_uv) {
-                        ORI_CHAIN(tmem + s * TM_STAGE + TM_UV, 2, 2, true);
-                        ORI_CHAIN(tmem + s * TM_STAGE + TM_UV, 2, 3, false);
-                        ORI_CHAIN(tmem + s * TM_STAGE + TM_UV, 3, 2, false);
-                    }
-#endif
 #undef ORI_CHAIN
                     commit(&bars[B_SREADY + s]);
                     commit(&bars[B_KEMPTY + ks_]);
                 }
                 __syncwarp();
-                PF_CLK(pr2); PF_ADD(pm_issS, pr2, pr1);
                 if (it >= (uint32_t)(NS - 1)) trail_P();
                 if (last) ++li;
                 ++it;
                 ti.next(a);
             }
             while (itp < it) trail_P();
-#if ORI_TC_PROF
-            if (blockIdx.x < 2 && lane == 0 && !DEVI)
-                printf("PROF mma genes=%d cta=%d tiles=%u total=%u kfull=%u issS=%u pready=%u tfull=%u issP=%u\n", (int)GENES, (int)blockIdx.x,
-                       it, (uint32_t)clock() - pm_begin, pm_kfull, pm_issS, pm_pready, pm_tfull, pm_issP);
-#endif
         }
     } else {
         // ======================================= element-wise stage + epilogue =================================
         const int ew = warp - 2;
         const int quarter = warp & 3;                 // TMEM lane quarter this warp may touch
-        const int slice = ew >> 2;                    // which half of the tile's columns / of the own-side arrays
+        // slice: which half of the tile's columns, and which own-side array and accumulator
+        // (0: exp(E log .) and accumulator 1; 1: E[.] and accumulator 2)
+        const int slice = ew >> 2;
         const int lrow = quarter * 32 + lane;         // own index inside the tile = TMEM lane
-        const int colbase = (SPLIT ? (slice & 1) : slice) * CW;
-        const int group = slice >> 1;                 // SPLIT: parity of the tiles this warp works on
+        const int colbase = slice * CW;
         const uint32_t tlane = tmem + ((uint32_t)(quarter * 32) << 16);
         const uint32_t sbase = smem_u32(smem);
         const bool any_floor = DROPOUT && (*a.any_floor != 0);
-        auto arrive_leader = [&](uint64_t* bar) { if (PAIR) mbar_arrive_cluster(bar, 0); else mbar_arrive(bar); };
 
         // own-side operands of one work item -> TMEM: slice 0 writes hi / lo of exp(E log .), slice 1 (dropout only)
-        // hi / lo of E[.], for this warp's 32 lanes, 32 latent components at a time
-        const int aside = slice / ASUBS;              // 0: exp(E log .) and accumulator 1; 1: E[.] and accumulator 2
-        const int asub = slice % ASUBS;
+        // hi / lo of E[.], for this warp's 32 lanes, 16 latent components at a time
         auto a_load_store = [&](int own0) {
-            if (aside * 2 < NQ) {
+            if (slice * 2 < NQ) {
                 const long long idx = (long long)own0 + lrow;
-                const float* src = (aside ? a.own_E : a.own_e) + idx * KP;
+                const float* src = (slice ? a.own_E : a.own_e) + idx * KP;
                 const bool ok = idx < a.own_total;
-                const bool scale = GENES && aside;                 // uv is kept in log2 units: V_hat side * log2(e)
+                const bool scale = GENES && slice;                 // uv is kept in log2 units: V_hat side * log2(e)
 #pragma unroll
-                for (int c16 = asub; c16 < KP / 16; c16 += ASUBS) {        // 16 latent components at a time
+                for (int c16 = 0; c16 < KP / 16; ++c16) {
                     float av[16];
 #pragma unroll
                     for (int c = 0; c < 4; ++c) {
@@ -623,8 +492,7 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                         whi[e] = __float_as_uint(hi);
                         wlo[e] = __float_as_uint(v - hi);
                     }
-                    tmem_st16(tlane + TM_A + (2 * aside) * KP + 16 * c16, whi);
-#if ORI_TC_BF16X
+                    tmem_st16(tlane + TM_A + (2 * slice) * KP + 16 * c16, whi);
                     // cross-term operand [hi | lo] as bf16 pairs: these 16 components -> 8 + 8 columns
                     uint32_t phi[8], plo[8];
 #pragma unroll
@@ -632,17 +500,14 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                         phi[e] = pack_bf16x2(__uint_as_float(whi[2 * e]), __uint_as_float(whi[2 * e + 1]));
                         plo[e] = pack_bf16x2(__uint_as_float(wlo[2 * e]), __uint_as_float(wlo[2 * e + 1]));
                     }
-                    tmem_st8(tlane + TM_A + (2 * aside + 1) * KP + 8 * c16, phi);
-                    tmem_st8(tlane + TM_A + (2 * aside + 1) * KP + KP / 2 + 8 * c16, plo);
-#else
-                    tmem_st16(tlane + TM_A + (2 * aside + 1) * KP + 16 * c16, wlo);
-#endif
+                    tmem_st8(tlane + TM_A + (2 * slice + 1) * KP + 8 * c16, phi);
+                    tmem_st8(tlane + TM_A + (2 * slice + 1) * KP + KP / 2 + 8 * c16, plo);
                 }
             }
             tmem_wait_st();
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_leader(&bars[B_A_READY]);
+            if (lane == 0) mbar_arrive_cluster(&bars[B_A_READY], 0);
         };
 
         // gene pass: X is staged [cell][gene]; lane (gene) reads one float per cell, 128-byte swizzle undone here
@@ -654,10 +519,6 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
         ti.init(a, NCTA, rank);
         uint32_t it = 0;                              // tiles of this CTA so far: TMEM stage it & 1, X stage it % XST
         int li = 0;
-#if ORI_TC_PROF
-        uint32_t pf_wait = 0, pf_ld = 0, pf_math = 0, pf_st = 0, pf_ho = 0, pf_epi = 0;
-        const uint32_t pf_begin = (uint32_t)clock();
-#endif
         if (ti.valid(a)) a_load_store(ti.own0);
         while (ti.valid(a)) {
             const long long own_idx = (long long)ti.own0 + lrow;
@@ -710,9 +571,7 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             };
             auto ld_group = [&](const Tile& c, int g, int b) {
                 tmem_ld16(c.tden + colbase + g * 16, dr[b]);
-#if !ORI_KO_LDUV
                 if (DROPOUT) tmem_ld16(c.tden + TM_UV + colbase + g * 16, ur[b]);
-#endif
             };
             // PRECISE: v -> tf32 hi (written where the MMA reads R / D) and the bf16 pairs of (hi, lo) of two neighbouring
             // entries (written beside them): words 0..7 of a group = hi pairs, pk[8..15] = lo pairs
@@ -797,63 +656,35 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     }
                 }
                 float dmin = 1.f;
-#if ORI_KO_MATH
-                g_cs += x[b][0] + ((DROPOUT && !GENES) ? cc[0] : 0.f);
-                return dmin;
-#endif
 #pragma unroll
                 for (int e = 0; e < 16; ++e) {
                     const float den = __uint_as_float(dr[b][e]);
                     const float xe = x[b][e];
-#if !ORI_KO_DMIN
                     dmin = fminf(dmin, den);                  // den <= 0 (zigap.py:90): the group is redone below
-#endif
                     float tt = den, uvp = 0.f;
                     if (DROPOUT) {
-#if ORI_KO_LDUV
-                        uvp = den * 1e-30f;
-#else
                         uvp = __uint_as_float(ur[b][e]);                          // U_hat.V_hat * log2(e)
-#endif
-#if !ORI_KO_ULIM
                         if (GENES && ELBO) uvp = fminf(uvp, ulim);                // keeps 2^uv, tz and e2 finite
-#endif
                         const float tz = fmaf(ex2_approx(uvp), GENES ? cj : cc[e], 1.f);   // 1 + exp(uv - logit pi)
                         tt = sel_nz_a(xe, den, tz);
                     }
                     const float r = rcp_approx(tt);
-#if ORI_KO_BIAS
-                    dr[b][e] = __float_as_uint(xe * r);
-#else
                     dr[b][e] = PRECISE ? __float_as_uint(xe * r) : tf32_bias(xe * r);   // R = X / den; 0 where X == 0
-#endif
                     float D = 1.f;
                     if (DROPOUT) {
                         D = sel_nz_b(xe, 1.f, r);                                 // zigap.py:131-136
-#if ORI_KO_BIAS
-                        ur[b][e] = __float_as_uint(D);
-#else
                         ur[b][e] = PRECISE ? __float_as_uint(D) : tf32_bias(D);
-#endif
                     }
                     if (GENES) {
-#if !ORI_KO_CS
                         if (DROPOUT) g_cs += D;
-#endif
                         if (ELBO) {
-#if ORI_KO_LG2
-                            const float l2 = tt;
-#else
                             const float l2 = lg2_approx(tt);
-#endif
                             g_xl = fmaf(xe, l2, g_xl);
                             if (DROPOUT) {
                                 g_ent = fmaf(is_zero_f(xe), l2, g_ent);           // log2(1 + 2^e2) on zeros
-#if !ORI_KO_ENT2
                                 const float e2 = uvp - lp2f;                      // <= 127 (uvp was clamped)
                                 const float w = 1.f - D;                          // 0 on non-zeros
                                 g_ent = fmaf(-w, e2, g_ent);
-#endif
                             }
                         }
                     }
@@ -874,16 +705,14 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     }
                 }
                 tmem_st16(c.tden + c0, dr[b]);
-#if !ORI_KO_STD
                 if (DROPOUT) tmem_st16(c.tden + TM_UV + c0, ur[b]);
-#endif
             };
             // R / D_hat of the tile are in TMEM (after tcgen05.wait::st): P may run; the X stage may be refilled
             auto hand_off = [&](const Tile& c) {
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) {
-                    arrive_leader(&bars[B_PREADY + c.s]);
+                    mbar_arrive_cluster(&bars[B_PREADY + c.s], 0);
                     mbar_arrive(&bars[B_XEMPTY + c.xs]);
                 }
             };
@@ -992,41 +821,25 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     }
                     hand_off(c);
                 }
-            } else if constexpr (!C::DEEP) {
-                // ---- round-1 plan: every warp owns G groups of the tile; the next group's loads fly during the current one;
+            } else {
+                // ---- every warp owns G groups of the tile; the next group's loads fly during the current one;
                 //      the tile is handed to the MMA warp as soon as its last group is stored
                 for (int t = ti.t_begin; t < t_end; ++t, ++it) {
                     const bool last = (t == t_end - 1);
-                    if (SPLIT && (int)(it & 1) != group) {
-                        // the other group's tile.  The item's last tile still carries this warp's share of the next item's
-                        // own-side operands: wait until its S (hence every S of the item) has completed
-                        if (last && has_next) {
-                            mbar_wait(&bars[B_SREADY + it % NS], (it / NS) & 1, 33);
-                            tc_fence_after();
-                            a_load_store(next_own0);
-                        }
-                        continue;
-                    }
                     const Tile c = tile_of(it, t);
-                    PF_CLK(pc0);
                     wait_tile(it);
-                    PF_CLK(pc1); PF_ADD(pf_wait, pc1, pc0);
                     if (last && has_next) a_load_store(next_own0);   // every S of this item has completed: A can be replaced
                     if (!c.slow) ld_group(c, 0, 0);
                     load_x(c, 0, 0);
                     float t_xl = 0.f, t_ent = 0.f;
 #pragma unroll
                     for (int g = 0; g < G; ++g) {
-                        const int b = SPLIT ? 0 : (g & 1);       // SPLIT: one register buffer, no prefetch inside the tile
+                        const int b = g & 1;
                         bool redo = c.slow;
-                        if (!SPLIT && g + 1 < G) load_x(c, g + 1, b ^ 1);
-                        if (SPLIT && g > 0) { if (!c.slow) ld_group(c, g, 0); load_x(c, g, 0); }
+                        if (g + 1 < G) load_x(c, g + 1, b ^ 1);
                         if (!c.slow) {
                             tmem_wait_ld();
-#if ORI_TC_PROF
-                            if (g == 0) { PF_CLK(pc2); PF_ADD(pf_ld, pc2, pc1); PF_ADD(pf_math, 0u, pc2); }
-#endif
-                            if (!SPLIT && g + 1 < G) ld_group(c, g + 1, b ^ 1);
+                            if (g + 1 < G) ld_group(c, g + 1, b ^ 1);
                             float g_cs = 0.f, g_xl = 0.f, g_ent = 0.f;
                             const float dmin = fast_group(c, g, b, g_cs, g_xl, g_ent);
                             redo = __any_sync(0xffffffffu, dmin <= den_lim) != 0;
@@ -1036,58 +849,9 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                         st_group(c, g, b);
                     }
                     if (GENES && ELBO) { kahan_add(xl_s, xl_c, t_xl); if (DROPOUT) kahan_add(ent_s, ent_c, t_ent); }
-                    PF_CLK(pc3); PF_ADD(pf_math, pc3, 0u);
                     tmem_wait_st();
-                    PF_CLK(pc4); PF_ADD(pf_st, pc4, pc3);
                     hand_off(c);
-                    PF_CLK(pc5); PF_ADD(pf_ho, pc5, pc4);
                 }
-            } else {
-                // ---- deep plan (one 16-column group per warp and tile, S three tiles ahead): while tile t is computed the
-                //      loads of tile t+1 (barrier wait, tcgen05.ld, X) are in flight in the other register buffer, and tile
-                //      t-1 is handed to the MMA warp only now -- its tcgen05.st has had a whole tile to complete -- so no
-                //      latency of the hand-off chain is exposed.  Buffer parity is a compile-time constant: the loop body is
-                //      instantiated for even and odd tiles of the item.
-                static_assert(G == 1, "deep plan: one group per warp and tile");
-                Tile pend = tile_of(0, 0);
-                bool have_pend = false;
-                auto tile_step = [&](auto PAR_, int t) {
-                    constexpr int b = decltype(PAR_)::value;
-                    const bool last = (t == t_end - 1);
-                    const Tile c = tile_of(it, t);
-                    if (t == ti.t_begin) {                       // nothing was prefetched across the item boundary
-                        wait_tile(it);
-                        ld_group(c, 0, b);
-                        load_x(c, 0, b);
-                    }
-                    if (last && has_next) a_load_store(next_own0);   // every S of this item has completed: A can be replaced
-                    bool redo = c.slow;
-                    float t_xl = 0.f, t_ent = 0.f;
-                    tmem_wait_ld();
-                    if (!last) {
-                        const Tile nc = tile_of(it + 1, t + 1);
-                        wait_tile(it + 1);                       // S(t+1) was issued NS - 1 tiles ago
-                        ld_group(nc, 0, b ^ 1);
-                        load_x(nc, 0, b ^ 1);
-                    }
-                    if (!c.slow) {
-                        float g_cs = 0.f, g_xl = 0.f, g_ent = 0.f;
-                        const float dmin = fast_group(c, 0, b, g_cs, g_xl, g_ent);
-                        redo = __any_sync(0xffffffffu, dmin <= den_lim) != 0;
-                        if (GENES && !redo) { cs += g_cs; t_xl += g_xl; t_ent += g_ent; }
-                    }
-                    if (redo) slow_group(c, 0, b, t_xl, t_ent);
-                    if (GENES && ELBO) { kahan_add(xl_s, xl_c, t_xl); if (DROPOUT) kahan_add(ent_s, ent_c, t_ent); }
-                    if (have_pend) { tmem_wait_st(); hand_off(pend); }
-                    st_group(c, 0, b);
-                    pend = c; have_pend = true;
-                    ++it;
-                };
-                for (int t = ti.t_begin; t < t_end; t += 2) {
-                    tile_step(std::integral_constant<int, 0>{}, t);
-                    if (t + 1 < t_end) tile_step(std::integral_constant<int, 1>{}, t + 1);
-                }
-                if (have_pend) { tmem_wait_st(); hand_off(pend); }
             }
             if constexpr (DEVI) {
                 unsigned long long r0 = (unsigned long long)dv0, r1 = (unsigned long long)dv1, r2 = (unsigned long long)dv2;
@@ -1107,7 +871,6 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                 continue;
             }
             double acc_xl = (double)xl_s - (double)xl_c, acc_ent = (double)ent_s - (double)ent_c;
-            PF_CLK(pe0);
             // ---- epilogue of the work item: accumulators -> global (atomics: the sweep of one own tile is split);
             //      slice 0 drains acc1, slice 1 acc2
             mbar_wait(&bars[B_ACC_READY], li & 1, 32);
@@ -1122,12 +885,12 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                 __syncwarp();
                 __threadfence();
             }
-            if (aside == 0 || DROPOUT) {
-                float* out = (aside == 0 ? a.acc1 : a.acc2) + own_idx * KP;
+            if (slice == 0 || DROPOUT) {
+                float* out = (slice == 0 ? a.acc1 : a.acc2) + own_idx * KP;
 #pragma unroll
-                for (int g = asub; g < KP / 16; g += ASUBS) {
+                for (int g = 0; g < KP / 16; ++g) {
                     uint32_t v[16];
-                    tmem_ld16(tlane + TM_ACC + aside * KP + g * 16, v);
+                    tmem_ld16(tlane + TM_ACC + slice * KP + g * 16, v);
                     tmem_wait_ld();
                     if (own_ok) {
 #pragma unroll
@@ -1137,12 +900,9 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_leader(&bars[B_ACC_FREE]);
+            if (lane == 0) mbar_arrive_cluster(&bars[B_ACC_FREE], 0);
             if (GENES) {
-                if (DROPOUT && own_ok) {
-                    static_assert(!DET || SLICES == 2, "deterministic epilogue: two column slices");
-                    atomicAdd(((DET && slice) ? a.colsum2 : a.colsum) + own_idx, (double)cs);
-                }
+                if (DROPOUT && own_ok) atomicAdd(((DET && slice) ? a.colsum2 : a.colsum) + own_idx, (double)cs);
                 if (ELBO) {
                     if (!own_ok) { acc_xl = 0.0; acc_ent = 0.0; }
 #pragma unroll
@@ -1170,23 +930,18 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             ++li;
             ti.item += ti.stride;
             ti.load(a);
-            PF_CLK(pe1); PF_ADD(pf_epi, pe1, pe0);
         }
-#if ORI_TC_PROF
-        if (blockIdx.x < 2 && lane == 0 && !DEVI)
-            printf("PROF ew genes=%d cta=%d warp=%d tiles=%u total=%u wait=%u ld=%u math=%u st=%u handoff=%u epi=%u\n", (int)GENES,
-                   (int)blockIdx.x, ew, it, (uint32_t)clock() - pf_begin, pf_wait, pf_ld, pf_math, pf_st, pf_ho, pf_epi);
-#endif
     }
     tc_fence_before();
     __syncthreads();
-    if (PAIR) cluster_sync_all();          // the leader's MMAs read the peer's shared memory and TMEM until the very end
-    if (warp == 1) { if (PAIR) tmem_dealloc_pair(tmem, TM_COLS); else tmem_dealloc(tmem, TM_COLS); }
+    cluster_sync_all();                    // the leader's MMAs read the peer's shared memory and TMEM until the very end
+    if (warp == 1) tmem_dealloc_pair(tmem, TM_COLS);
 }
 
 // ---- operand preparation -------------------------------------------------------------------------------------
-// K-major operand arrays: out[q][pad][KP], q = 0: hi(e) 1: lo(e) 2: hi(E) 3: lo(E); hi = tf32 round-to-nearest
-// (the tensor core truncates fp32 operands to tf32: scripts/tc_probe.cu T4), lo = x - hi.  Pad rows are zero.
+// K-major operand arrays: out[q][pad][KP], q = 0: hi(e) 1: bf16 pairs of lo(e) | hi(e) 2: hi(E) 3: the same pairs of E;
+// hi = tf32 round-to-nearest (the tensor core truncates fp32 operands to tf32: scripts/tc_probe.cu T4), lo = x - hi.
+// Pad rows are zero.
 __global__ void __launch_bounds__(256)
 k_tc_prep_K(const float* __restrict__ e, const float* __restrict__ E, float Escale, float* __restrict__ out, long long n,
             long long pad, int KP)
@@ -1197,7 +952,6 @@ k_tc_prep_K(const float* __restrict__ e, const float* __restrict__ E, float Esca
     const float v = ok ? e[idx] : 0.f;
     const float hv = to_tf32_rna(v);
     out[idx] = hv;
-#if ORI_TC_BF16X
     // arrays 1 and 3: row i = 2 KP bf16 [lo(0..KP-1) | hi(0..KP-1)], i.e. KP 32-bit words; this thread writes word w
     const long long i = idx / KP;
     const int w = (int)(idx - i * KP), half = KP / 2;
@@ -1213,15 +967,6 @@ k_tc_prep_K(const float* __restrict__ e, const float* __restrict__ E, float Esca
         out[2 * pad * KP + idx] = to_tf32_rna(x);
         reinterpret_cast<uint32_t*>(out)[3 * pad * KP + idx] = word(E, Escale);
     }
-#else
-    out[pad * KP + idx] = v - hv;
-    if (E) {
-        const float w = ok ? E[idx] * Escale : 0.f;
-        const float hw = to_tf32_rna(w);
-        out[2 * pad * KP + idx] = hw;
-        out[3 * pad * KP + idx] = w - hw;
-    }
-#endif
 }
 // transposed operand: out[k][i] = tf32(src[i][k]),  src [n x KP], out [KP x pad]; grid (pad / 32, KP / 32).
 // out16 (PRECISE, else NULL): the bf16 pairs [lo | hi] of the same values, 32 words per block of 32 sweep entries:
@@ -1459,13 +1204,6 @@ int launch_tc_prep_rows_logsum(const ori_problem_t* P, int g, cudaStream_t st) {
     return check_launch("k_tc_prep(rows, logsum)");
 }
 
-static int env_int(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-// CTA-pair kernels (cta_group::2) by default; ORI_TC_PAIR=0 selects the single-CTA variant (kept for A/B runs, KP 32)
-static bool use_pair() { static int v = env_int("ORI_TC_PAIR", 1); return v != 0; }
-
 // Split the sweep into chunks of a FIXED length: the accumulators of a work item live in TMEM, and the tensor core's fp32
 // accumulation truncates -- a chain of S accumulating MMAs comes out about S * 3e-8 low (measured: sum_ij D_ij (U V^T)_ij
 // at 100k x 20k differed by 8e-6 between a 2504-step and an 830-step chaining of the same state, and with it the ELBO by
@@ -1496,34 +1234,44 @@ static void tc_partition(TcArgs& a, bool genes, int units, int sw, bool precise,
     a.n_items = a.n_own_units * a.n_chunks;
 }
 
-template <bool GENES, bool D, bool E, bool PAIR, int KP, bool PRECISE, bool UFL = false, bool DET = false>
+template <bool GENES, bool D, bool E, int KP, bool PRECISE, bool DEVI, bool UFL, bool DET>
 static int launch_tc_variant(const TcMaps& maps, const TcArgs& a, int grid, cudaStream_t st) {
-    auto kern = k_tc_pass<GENES, D, E, PAIR, KP, PRECISE, false, UFL, DET>;
+    auto kern = k_tc_pass<GENES, D, E, KP, PRECISE, DEVI, UFL, DET>;
+    constexpr uint32_t smem = Cfg<KP, PRECISE, DEVI>::SMEM_BYTES;
     static bool attr_done = false;
     if (!attr_done) {
-        cudaError_t e_ = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<KP, PAIR, PRECISE>::SMEM_BYTES);
+        cudaError_t e_ = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e_));
         attr_done = true;
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = Cfg<KP, PAIR, PRECISE>::SMEM_BYTES; cfg.stream = st;
+    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = PAIR ? 2 : 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    attr[0].val.clusterDim.x = NCTA; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     cudaError_t e_ = cudaLaunchKernelEx(&cfg, kern, maps, a);
     if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaLaunchKernelEx(k_tc_pass): %s", cudaGetErrorString(e_));
     return ORI_OK;
 }
 
+// the instance of a pass for its (dropout, ELBO) flags
+template <bool GENES, int KP, bool PRECISE, bool UFL, bool DET>
+static int launch_tc_flags(bool drop, bool elbo, const TcMaps& maps, const TcArgs& a, int grid, cudaStream_t st) {
+    if (drop && elbo) return launch_tc_variant<GENES, true, true, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
+    if (drop) return launch_tc_variant<GENES, true, false, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
+    if (elbo) return launch_tc_variant<GENES, false, true, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
+    return launch_tc_variant<GENES, false, false, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
+}
+
 // logsum: the dropout-free sweep of the sparse model's third gene-side sum into red32 block 2
-template <bool GENES, bool PAIR, int KP, bool PRECISE>
+template <bool GENES, int KP, bool PRECISE>
 static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st, bool logsum = false) {
-    using C = Cfg<KP, PAIR, PRECISE>;
+    using C = Cfg<KP, PRECISE>;
     const TcWs w = tc_carve(P);
     const bool sparse = P->flags & ORI_F_SPARSE;
     const bool drop = (P->flags & ORI_F_DROPOUT) && !logsum, elbo = (P->flags & ORI_F_ELBO) && !logsum;
-    constexpr int NCTA = C::NCTA, SW = C::SW;
+    constexpr int SW = C::SW;
     TcMaps maps;
     TcArgs a;
     bool ok;
@@ -1561,6 +1309,7 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
     a.tickets = nullptr; a.item_part = nullptr; a.colsum2 = nullptr;
     const bool det = (P->flags & ORI_F_DETERMINISTIC) && P->det_ws;
     if (det) {
+        if (ufl) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC and the underflow thresholds cannot be combined on the tensor path");
         if (a.n_items > det_max_items(P->n_rows, P->p)) return set_error(ORI_EINVAL, "det_ws too small for %d items", a.n_items);
         a.colsum2 = P->det_ws + (long long)DET_FU_BLOCKS * DET_FU_SLOTS;
         a.item_part = a.colsum2 + pad128(P->p);
@@ -1572,37 +1321,14 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
         cudaError_t e_ = cudaMemsetAsync(a.tickets, 0, sizeof(int) * (size_t)(a.n_own_tiles + 2), st);
         if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaMemsetAsync(tickets): %s", cudaGetErrorString(e_));
         if (!(GENES && elbo)) a.item_part = nullptr;
-        else {      // slots of the second CTA stay unwritten with the single-CTA kernels
+        else {      // the kernel writes every (CTA, warp) slot of an item; zeroed all the same, so no stale value is ever summed
             e_ = cudaMemsetAsync(a.item_part, 0, sizeof(double) * (size_t)a.n_items * DET_ITEM_SLOTS, st);
             if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaMemsetAsync(item_part): %s", cudaGetErrorString(e_));
         }
     }
-    int rc;
-    if (det) {
-        if (ufl) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC and the underflow thresholds cannot be combined on the tensor path");
-        if constexpr (PAIR && NEW == 8) {
-            if (drop && elbo) rc = launch_tc_variant<GENES, true, true, PAIR, KP, PRECISE, false, true>(maps, a, grid, st);
-            else if (drop) rc = launch_tc_variant<GENES, true, false, PAIR, KP, PRECISE, false, true>(maps, a, grid, st);
-            else if (elbo) rc = launch_tc_variant<GENES, false, true, PAIR, KP, PRECISE, false, true>(maps, a, grid, st);
-            else rc = launch_tc_variant<GENES, false, false, PAIR, KP, PRECISE, false, true>(maps, a, grid, st);
-        } else {
-            return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC needs the CTA-pair kernels (ORI_TC_PAIR=1)");
-        }
-    } else
-    if (ufl) {
-        if constexpr (PAIR) {
-            if (drop && elbo) rc = launch_tc_variant<GENES, true, true, PAIR, KP, PRECISE, true>(maps, a, grid, st);
-            else if (drop) rc = launch_tc_variant<GENES, true, false, PAIR, KP, PRECISE, true>(maps, a, grid, st);
-            else if (elbo) rc = launch_tc_variant<GENES, false, true, PAIR, KP, PRECISE, true>(maps, a, grid, st);
-            else rc = launch_tc_variant<GENES, false, false, PAIR, KP, PRECISE, true>(maps, a, grid, st);
-        } else {
-            return set_error(ORI_EUNSUPPORTED, "underflow emulation on the tensor path needs the CTA-pair kernels (ORI_TC_PAIR=1)");
-        }
-    } else
-    if (drop && elbo) rc = launch_tc_variant<GENES, true, true, PAIR, KP, PRECISE>(maps, a, grid, st);
-    else if (drop) rc = launch_tc_variant<GENES, true, false, PAIR, KP, PRECISE>(maps, a, grid, st);
-    else if (elbo) rc = launch_tc_variant<GENES, false, true, PAIR, KP, PRECISE>(maps, a, grid, st);
-    else rc = launch_tc_variant<GENES, false, false, PAIR, KP, PRECISE>(maps, a, grid, st);
+    const int rc = det ? launch_tc_flags<GENES, KP, PRECISE, false, true>(drop, elbo, maps, a, grid, st)
+                 : ufl ? launch_tc_flags<GENES, KP, PRECISE, true, false>(drop, elbo, maps, a, grid, st)
+                       : launch_tc_flags<GENES, KP, PRECISE, false, false>(drop, elbo, maps, a, grid, st);
     if (rc != ORI_OK) return rc;
     int extra = 0;
     if (det && GENES && drop) { k_det_add<<<cdiv(P->p, 256), 256, 0, st>>>(P->red64, a.colsum2, P->p); ++extra; }
@@ -1617,20 +1343,10 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
 
 template <bool GENES>
 static int launch_tc_pass(const ori_problem_t* P, int gen_old, cudaStream_t st, bool logsum = false) {
-    if (P->flags & ORI_F_PRECISE) {      // fp32-grade contractions: KP = 32 plan with 32-wide sweep tiles (tc_eligible checks KP)
-#if ORI_TC_NEW == 8
-        return launch_tc_pass_p<GENES, true, 32, true>(P, gen_old, st, logsum);
-#else
-        return set_error(ORI_EUNSUPPORTED, "this build (ORI_TC_NEW != 8) has no fp32-grade plan");
-#endif
-    }
-#if ORI_TC_NEW == 8
-    if (P->KP == 64) return launch_tc_pass_p<GENES, true, 64, false>(P, gen_old, st, logsum);
-#else
-    if (P->KP == 64) return set_error(ORI_EUNSUPPORTED, "this build (ORI_TC_NEW != 8) has no KP = 64 plan");
-#endif
-    return use_pair() ? launch_tc_pass_p<GENES, true, 32, false>(P, gen_old, st, logsum)
-                      : launch_tc_pass_p<GENES, false, 32, false>(P, gen_old, st, logsum);
+    // fp32-grade contractions: KP = 32 plan with 32-wide sweep tiles (tc_eligible checks KP)
+    if (P->flags & ORI_F_PRECISE) return launch_tc_pass_p<GENES, 32, true>(P, gen_old, st, logsum);
+    if (P->KP == 64) return launch_tc_pass_p<GENES, 64, false>(P, gen_old, st, logsum);
+    return launch_tc_pass_p<GENES, 32, false>(P, gen_old, st, logsum);
 }
 
 // The three truncated log-likelihood sums behind reconstruction_deviance / explained_deviance (base.py:58-82) on the
@@ -1638,8 +1354,8 @@ static int launch_tc_pass(const ori_problem_t* P, int gen_old, cudaStream_t st, 
 template <int KP>
 static int launch_deviance_tc_kp(const ori_problem_t* P, int g, const double* pi, const double* cmean, long long* out_int,
                                  cudaStream_t st) {
-    using C = Cfg<KP, true, false, true>;
-    constexpr int NCTA = C::NCTA, SW = C::SW;
+    using C = Cfg<KP, false, true>;
+    constexpr int SW = C::SW;
     const TcWs w = tc_carve(P);
     const bool sparse = P->flags & ORI_F_SPARSE;
     // gene-side K-major operands: [hi | lo] of the effective V_hat (rate) and of the V_hat that generates D_hat (log2 units)
@@ -1675,32 +1391,15 @@ static int launch_deviance_tc_kp(const ori_problem_t* P, int g, const double* pi
     a.n_chunks = cdiv(a.n_sw_tiles, a.tiles_per_chunk);
     a.n_items = a.n_own_units * a.n_chunks;
     const int grid = NCTA * (a.n_items < units ? a.n_items : units);
-    auto kern = k_tc_pass<false, true, false, true, KP, false, true>;
-    static bool attr_done = false;
-    if (!attr_done) {
-        cudaError_t e_ = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
-        if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e_));
-        attr_done = true;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = C::SMEM_BYTES; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    cudaError_t e_ = cudaLaunchKernelEx(&cfg, kern, maps, a);
-    if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaLaunchKernelEx(k_tc_pass deviance): %s", cudaGetErrorString(e_));
+    const int rc = launch_tc_variant<false, true, false, KP, false, true, false, false>(maps, a, grid, st);
+    if (rc != ORI_OK) return rc;
     return check_launch("k_tc_pass(deviance)");
 }
 
 // integer sums only (the float64 sums stay on the CUDA-core kernel); `pi`, `cmean` as for launch_deviance
 int launch_deviance_tc(const ori_problem_t* P, int g, const double* pi, const double* cmean, long long* out_int, cudaStream_t st) {
-#if ORI_TC_NEW == 8
     if (P->KP == 64) return launch_deviance_tc_kp<64>(P, g, pi, cmean, out_int, st);
     return launch_deviance_tc_kp<32>(P, g, pi, cmean, out_int, st);
-#else
-    return set_error(ORI_EUNSUPPORTED, "this build (ORI_TC_NEW != 8) has no deviance pass on the tensor path");
-#endif
 }
 
 int launch_pass_rows_tc(const ori_problem_t* P, int gen_old, cudaStream_t st) { return launch_tc_pass<false>(P, gen_old, st); }

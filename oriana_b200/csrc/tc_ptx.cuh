@@ -19,7 +19,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
 }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
@@ -37,27 +36,14 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
         : "memory");
     return ok != 0;
 }
-__device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {   // pure poll, never suspends
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
 // Bounded wait: a protocol bug must surface as a launch failure, never as a hung GPU.
 #ifndef ORI_MBAR_TIMEOUT_CYCLES
 #define ORI_MBAR_TIMEOUT_CYCLES 6000000000ll
 #endif
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity);
-// cluster = true: the barrier also receives arrivals from the peer CTA (acquire at cluster scope)
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int tag = 0, bool cluster = false) {
-    if (cluster ? mbar_try_wait_cluster(bar, parity) : mbar_try_wait(bar, parity)) return;
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int tag = 0) {
+    if (mbar_try_wait(bar, parity)) return;
     const long long t0 = clock64();
-    while (!(cluster ? mbar_try_wait_cluster(bar, parity) : mbar_try_wait(bar, parity))) {
+    while (!mbar_try_wait(bar, parity)) {
         if (clock64() - t0 > ORI_MBAR_TIMEOUT_CYCLES) {
             printf("oriana_b200: mbarrier timeout tag=%d block=%d thread=%d parity=%u\n", tag, blockIdx.x, threadIdx.x, parity);
             __trap();
@@ -138,17 +124,6 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t rank
         "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
         "mbarrier.arrive.shared::cluster.b64 _, [ra];\n\t}"
         ::"r"(smem_u32(bar)), "r"(rank) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {   // acquire at cluster scope
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
 }
 
 // ---- TMEM ---------------------------------------------------------------------------------------------
@@ -252,14 +227,7 @@ __device__ __forceinline__ void mma_tf32_ts_pair(uint32_t d_tmem, uint32_t a_tme
         : "memory");
 }
 
-// bf16 operands: A from TMEM (two consecutive K elements per 32-bit cell, lower index in the low half), B from smem
-__device__ __forceinline__ void mma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, bool accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate)
-        : "memory");
-}
+// bf16 operands, CTA pair: A from TMEM (two consecutive K elements per 32-bit cell, lower index in the low half), B from smem
 __device__ __forceinline__ void mma_bf16_ts_pair(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, bool accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
