@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .models.base import pad_k
+from .problem import build_problem, gene_buffers, kernel_plan, logit_pi, row_pitch
 from .sharding import RowSharding
 
 
@@ -44,7 +44,41 @@ def bind_host_thread_to_gpu(device_index):
         return None
 
 
-class CompactCounts:
+class _EscapeList:
+    """The counts >= 255, which a byte cannot hold: X[row, col] = val, sorted by row (int32, int32, float32; pinned).
+    Each slab's escapes follow it to the device, where `ori_scatter_counts_f32` writes them into X."""
+
+    def _set_escapes(self, row, col, val):
+        assert row.dtype == torch.int32 and col.dtype == torch.int32 and val.dtype == torch.float32
+        assert row.numel() == col.numel() == val.numel()
+        self.row, self.col, self.val, self._row_np = row, col, val, row.numpy()
+        assert (np.diff(self._row_np) >= 0).all(), 'escape list must be sorted by row'
+
+    @staticmethod
+    def _gather_escapes(blk, r0, parts):
+        """Append the escapes of the row block `blk`, whose first row is row r0, to `parts`."""
+        idx = (blk >= 255).nonzero(as_tuple=False)
+        if idx.numel():
+            parts.append(((idx[:, 0] + r0).to(torch.int32).cpu(), idx[:, 1].to(torch.int32).cpu(),
+                          blk[idx[:, 0], idx[:, 1]].to(torch.float32).cpu()))
+
+    @staticmethod
+    def _join_escapes(parts, pin):
+        if not parts:                                  # no escapes: empty, unpinned
+            return [torch.empty((0,), dtype=dt) for dt in (torch.int32, torch.int32, torch.float32)]
+        return [t.pin_memory() if pin else t for t in (torch.cat(c) for c in zip(*parts))]
+
+    def escapes(self, r0, r1):
+        """[lo, hi) of the escapes of rows [r0, r1)."""
+        return int(np.searchsorted(self._row_np, r0)), int(np.searchsorted(self._row_np, r1))
+
+    def _with_escapes(self, X):
+        """The float32 host matrix X of the byte form with the escapes written in."""
+        X[self.row.long(), self.col.long()] = self.val
+        return X
+
+
+class CompactCounts(_EscapeList):
     """A count matrix held on the host as saturating uint8 plus an escape list for the (rare) counts >= 255:
     one byte per entry crosses PCIe per step instead of four.  Lossless: `dense()` gives the counts back.
 
@@ -54,50 +88,31 @@ class CompactCounts:
 
     def __init__(self, u8, row, col, val):
         assert u8.dtype == torch.uint8 and u8.dim() == 2 and not u8.is_cuda
-        assert row.dtype == torch.int32 and col.dtype == torch.int32 and val.dtype == torch.float32
-        assert row.numel() == col.numel() == val.numel()
-        self.u8, self.row, self.col, self.val = u8, row, col, val
-        self.shape = tuple(u8.shape)
-        # escapes of slab [r0, r1) = [bounds(r0), bounds(r1)) in the row-sorted list
-        self._row_np = row.numpy()
-        assert (np.diff(self._row_np) >= 0).all(), 'escape list must be sorted by row'
+        self.u8, self.shape = u8, tuple(u8.shape)
+        self._set_escapes(row, col, val)
 
     @classmethod
     def from_tensor(cls, X, chunk_rows=1 << 15, pin=True):
         """Encode a [n, p] count tensor (any real dtype, host or device; non-negative integers)."""
         n, p = X.shape
-        u8 = torch.empty((n, p), dtype=torch.uint8, pin_memory=pin and torch.cuda.is_available())
-        rows, cols, vals = [], [], []
+        pin = pin and torch.cuda.is_available()
+        u8 = torch.empty((n, p), dtype=torch.uint8, pin_memory=pin)
+        parts = []
         for r in range(0, n, chunk_rows):
             blk = X[r:r + chunk_rows]
-            big = blk >= 255
             u8[r:r + chunk_rows].copy_(torch.clamp(blk, max=255).to(torch.uint8))
-            idx = big.nonzero(as_tuple=False)
-            if idx.numel():
-                rows.append((idx[:, 0] + r).to(torch.int32).cpu()); cols.append(idx[:, 1].to(torch.int32).cpu())
-                vals.append(blk[big].to(torch.float32).cpu())
-
-        def cat(parts, dt):
-            t = torch.cat(parts) if parts else torch.empty((0,), dtype=dt)
-            return t.pin_memory() if (pin and torch.cuda.is_available() and t.numel()) else t
-        return cls(u8, cat(rows, torch.int32), cat(cols, torch.int32), cat(vals, torch.float32))
-
-    def escapes(self, r0, r1):
-        lo = int(np.searchsorted(self._row_np, r0, side='left')); hi = int(np.searchsorted(self._row_np, r1, side='left'))
-        return lo, hi
+            cls._gather_escapes(blk, r, parts)
+        return cls(u8, *cls._join_escapes(parts, pin))
 
     def dense(self):
-        X = self.u8.to(torch.float32)
-        if self.row.numel():
-            X[self.row.long(), self.col.long()] = self.val
-        return X
+        return self._with_escapes(self.u8.to(torch.float32))
 
     @property
     def nbytes(self):
         return self.u8.numel() + 12 * self.row.numel()
 
 
-class SparseCounts:
+class SparseCounts(_EscapeList):
     """A count matrix held on the host the way single-cell data is shaped -- mostly zeros (cmatrix.py:100-104,
     `as_sparse_matrix`): per cell one bit per gene, the non-zero counts in gene order as saturating bytes, and the escape
     list of `CompactCounts` for the counts >= 255.  p / 8 + nnz bytes per cell cross PCIe per step instead of p
@@ -114,13 +129,11 @@ class SparseCounts:
         n, p = shape
         assert bitmap.dtype == torch.int32 and tuple(bitmap.shape) == (n, (p + 31) // 32) and not bitmap.is_cuda
         assert nz.dtype == torch.uint8 and rowoff.dtype == torch.int64 and rowoff.numel() == n + 1
-        assert row.dtype == torch.int32 and col.dtype == torch.int32 and val.dtype == torch.float32
         self.shape = (int(n), int(p))
-        self.bitmap, self.nz, self.rowoff, self.row, self.col, self.val = bitmap, nz, rowoff, row, col, val
+        self.bitmap, self.nz, self.rowoff = bitmap, nz, rowoff
         self._off_np = rowoff.numpy()
         assert int(self._off_np[-1]) == nz.numel() and (np.diff(self._off_np) >= 0).all()
-        self._row_np = row.numpy()
-        assert (np.diff(self._row_np) >= 0).all(), 'escape list must be sorted by row'
+        self._set_escapes(row, col, val)
 
     @staticmethod
     def _pack_bits(mask):
@@ -149,28 +162,17 @@ class SparseCounts:
         total = int(rowoff[-1])
         bitmap = torch.empty((n, W), dtype=torch.int32, pin_memory=pin)
         nz = torch.empty((total,), dtype=torch.uint8, pin_memory=pin and total > 0)
-        rows, cols, vals = [], [], []
+        parts = []
         for r in range(0, n, chunk_rows):
             blk = X[r:r + chunk_rows]
             mask = blk != 0
             bitmap[r:r + chunk_rows].copy_(cls._pack_bits(mask))
             lo, hi = int(rowoff[r]), int(rowoff[min(n, r + chunk_rows)])
             nz[lo:hi].copy_(torch.clamp(blk[mask], max=255).to(torch.uint8))
-            idx = (blk >= 255).nonzero(as_tuple=False)
-            if idx.numel():
-                rows.append((idx[:, 0] + r).to(torch.int32).cpu()); cols.append(idx[:, 1].to(torch.int32).cpu())
-                vals.append(blk[idx[:, 0], idx[:, 1]].to(torch.float32).cpu())
-
-        def cat(parts, dt):
-            t = torch.cat(parts) if parts else torch.empty((0,), dtype=dt)
-            return t.pin_memory() if (pin and t.numel()) else t
+            cls._gather_escapes(blk, r, parts)
         if pin:
             rowoff = rowoff.pin_memory()
-        return cls((n, p), bitmap, nz, rowoff, cat(rows, torch.int32), cat(cols, torch.int32), cat(vals, torch.float32))
-
-    def escapes(self, r0, r1):
-        lo = int(np.searchsorted(self._row_np, r0, side='left')); hi = int(np.searchsorted(self._row_np, r1, side='left'))
-        return lo, hi
+        return cls((n, p), bitmap, nz, rowoff, *cls._join_escapes(parts, pin))
 
     def byte_range(self, r0, r1):
         return int(self._off_np[r0]), int(self._off_np[r1])
@@ -181,9 +183,7 @@ class SparseCounts:
         bits = np.unpackbits(self.bitmap.numpy().view(np.uint8).reshape(n, -1), axis=1, bitorder='little')[:, :p].astype(bool)
         X = np.zeros((n, p), dtype=np.float32)
         X[bits] = self.nz.numpy().astype(np.float32)
-        if self.row.numel():
-            X[self.row.numpy().astype(np.int64), self.col.numpy().astype(np.int64)] = self.val.numpy()
-        return torch.from_numpy(X)
+        return self._with_escapes(torch.from_numpy(X))
 
     @property
     def nbytes(self):
@@ -230,24 +230,19 @@ class HostStreamedCAVI:
             self._xbytes = X_host.element_size()
             self.n, self.p = int(X_host.shape[0]), int(X_host.shape[1])
         self.k = int(k)
-        ldx0 = (self.p + 3) // 4 * 4
-        S0 = slab_rows if slab_rows is not None else self._default_slab(self.n, ldx0)
-        S0 = int(min(max(1, S0), max(1, self.n)))
-        # slabs large enough to fill the machine take the tcgen05/TMA kernels (K <= 64), like the device model
-        self._tensor = self.k <= (32 if precise else 64) and S0 * self.p >= (1 << 21)
-        KP = self._KP = (32 if self.k <= 32 else 64) if self._tensor else pad_k(self.k)
         n, p, K, dev = self.n, self.p, self.k, self._dev
+        ldx = self._ldx = row_pitch(p)
+        if slab_rows is None:
+            slab_rows = self._default_slab(n, ldx)
+        self.slab = S = int(min(max(1, slab_rows), max(1, n)))
+        # slabs large enough to fill the machine take the tcgen05/TMA kernels, like the device model
+        self._tensor, self._KP, plan_flags = kernel_plan(K, S * p, precise=precise)
         self._shard = RowSharding(process_group, enabled=bool(sharded or process_group is not None))
         self.n_total = self._shard.total_rows(n, dev)
         self.dropout = bool(dropout)
         self._flags = (_lib.ORI_F_DROPOUT if dropout else 0) | (_lib.ORI_F_ELBO if elbo else 0) \
-            | (_lib.ORI_F_QUIRK if (compat_quirk and dropout) else 0) \
-            | (_lib.ORI_F_PRECISE if (precise and self._tensor and self.k <= 32) else 0) \
-            | (_lib.ORI_F_FIXED_CHAIN if self.n > S0 else 0)
-        ldx = self._ldx = (p + 3) // 4 * 4
-        if slab_rows is None:
-            slab_rows = self._default_slab(n, ldx)
-        self.slab = S = int(min(max(1, slab_rows), max(1, n)))
+            | (_lib.ORI_F_QUIRK if (compat_quirk and dropout) else 0) | plan_flags \
+            | (_lib.ORI_F_FIXED_CHAIN if n > S else 0)
         self.h2d_bytes = 0
         self.d2h_bytes = 0
 
@@ -268,21 +263,20 @@ class HostStreamedCAVI:
         self.iterations = 0
 
         f32 = dict(dtype=torch.float32, device=dev); f64 = dict(dtype=torch.float64, device=dev)
-        # device: gene side + reduction buffers (small), two sets of slab buffers
-        g = self._g = dict(
-            b1=torch.zeros((p, KP), **f32), b2=torch.zeros((p, KP), **f32), V_hat=torch.zeros((p, KP), **f32),
-            eV=torch.zeros((p, KP), **f32), red32=torch.zeros((2, p, KP), **f32),
-            lp=torch.zeros((p,), **f32), pfloor=torch.zeros((p,), **f32), hyper=torch.ones((4, K), **f64),
-            red64=torch.zeros((p + 2 * KP + _lib.R64_NSLOTS,), **f64), gsum=torch.zeros((2 * KP + 8,), **f64),
-            pi=torch.zeros((p,), **f64), scal=torch.zeros((_lib.SCAL_SLOTS,), **f64), trace=torch.zeros((4,), **f64),
-            xcol=torch.zeros((p,), **f32))
+        # device: gene side + reduction buffers (small), two sets of slab buffers.  lp, pfloor and pi_d exist with or
+        # without dropout (every step uploads lp and pfloor)
+        KP = self._KP
+        g = self._g = gene_buffers(p, K, KP, dev, dropout=True, sparse=False, trace_cap=4)
+        g['xcol'] = torch.zeros((p,), **f32)
         self._slabs = []
         for _ in range(2 if n > S else 1):
             s = dict(X=torch.zeros((S, ldx), **f32), red64=torch.zeros_like(g['red64']),
                      acc64=torch.zeros_like(g['red64']), xrow=torch.zeros((S,), **f32),
-                     cs64=torch.zeros((p,), **f64), csacc=torch.zeros((p,), **f64))
-            for name in ('a1', 'a2', 'U0', 'U1', 'e0', 'e1', 'Zi', 'a2s', 'eUw'):
+                     cs64=torch.zeros((p,), **f64), csacc=torch.zeros((p,), **f64),
+                     tc_ws=torch.empty((int(self._lib.ori_tc_workspace_floats(S, p, KP)) + 32,), **f32) if self._tensor else None)
+            for name in ('a1', 'a2', 'Zi', 'a2s', 'eUw'):
                 s[name] = torch.zeros((S, KP), **f32)
+            s['U_hat'], s['eU'] = [[torch.zeros((S, KP), **f32) for _ in range(2)] for _ in range(2)]
             if self._sparse is not None:
                 off = self._sparse._off_np
                 nzcap = max(int(off[min(n, r + S)] - off[r]) for r in range(0, n, S)) + 16
@@ -295,8 +289,6 @@ class HostStreamedCAVI:
                 cap = max(1024, int(4 * self._compact.row.numel() * S / max(1, n)) + 1024)
                 s['esc'] = [torch.zeros((cap,), dtype=torch.int32, device=dev), torch.zeros((cap,), dtype=torch.int32, device=dev),
                             torch.zeros((cap,), dtype=torch.float32, device=dev)]
-            if self._tensor:
-                s['tc_ws'] = torch.empty((int(self._lib.ori_tc_workspace_floats(S, p, KP)) + 32,), **f32)
             s['stage'] = torch.zeros((2, S, K), **f32)     # unpadded a1|a2 as they travel
             self._slabs.append(s)
         self._streams = [torch.cuda.Stream(device=dev) for _ in self._slabs]
@@ -308,48 +300,25 @@ class HostStreamedCAVI:
         # generated by pi_prev (zigap.py:131-132), not the indicator of a freshly constructed model (zigap.py:77)
         it0 = int(state.get('iterations', 0) or 0)
         if self.dropout and state.get('pi_prev') is not None:
-            pi = np.asarray(state['pi_prev'], dtype=np.float64).reshape(p)
-            pc = np.clip(pi, 1e-15, 1. - 1e-15)
-            with np.errstate(divide='ignore'):
-                lp = np.log(pc / (1. - pc))
-            lp = np.where(pi <= 0, -np.inf, np.where(pi >= 1, np.inf, lp))
-            self.lp.copy_(torch.as_tensor(lp.astype(np.float32)))
-            self.pfloor.copy_(torch.as_tensor(np.where(pi <= 0, 1e-10, 0.).astype(np.float32)))
-            self.pi_d.copy_(torch.as_tensor(pi))
-            self.iterations = it0
+            self.pi_d.copy_(torch.as_tensor(np.asarray(state['pi_prev'], dtype=np.float64).reshape(p)))
+            lp, pfloor = logit_pi(self.pi_d)
+            self.lp.copy_(lp); self.pfloor.copy_(pfloor)
         elif self.dropout and it0 > 0:
             raise ValueError('a mid-run state (iterations=%d) must carry "pi_prev", the Bernoulli prior that generated its '
                              'dropout posterior (SURVEY.md section 8c)' % it0)
-        else:
-            self.iterations = it0
+        self.iterations = it0
 
     # ------------------------------------------------------------------------------------------------
     def _problem(self, s, rows):
-        g = self._g
-        P = _lib.OriProblem()
-        P.n_rows, P.n_total, P.ldx = rows, self.n_total, self._ldx
-        P.p, P.K, P.KP, P.flags = self.p, self.k, self._KP, self._flags
-        P.iter, P.trace_cap = 0, 4
-        dummy = g['red32'].data_ptr()
-        if s is not None:
-            P.X = s['X'].data_ptr()
-            P.a1, P.a2 = s['a1'].data_ptr(), s['a2'].data_ptr()
-            P.U_hat[0], P.U_hat[1] = s['U0'].data_ptr(), s['U1'].data_ptr()
-            P.eU[0], P.eU[1] = s['e0'].data_ptr(), s['e1'].data_ptr()
-            P.Zi, P.a2s, P.eUw = s['Zi'].data_ptr(), s['a2s'].data_ptr(), s['eUw'].data_ptr()
-            if 'tc_ws' in s:
-                P.tc_ws, P.tc_ws_floats = s['tc_ws'].data_ptr(), s['tc_ws'].numel()
-            P.xrow = s['xrow'].data_ptr()
+        """The problem of one slab, or (s=None) of the gene side alone: ori_problem_check wants the row pointers even then,
+        so they point at a gene-side buffer."""
+        if s is None:
+            d = self._g['red32']
+            row = dict(a1=d, a2=d, Zi=d, a2s=d, eUw=d, U_hat=(d, d), eU=(d, d))
         else:
-            P.X = None
-            P.a1 = P.a2 = P.Zi = P.a2s = P.eUw = dummy
-            P.U_hat[0] = P.U_hat[1] = P.eU[0] = P.eU[1] = dummy
-        P.b1, P.b2, P.V_hat, P.eV = (g[q].data_ptr() for q in ('b1', 'b2', 'V_hat', 'eV'))
-        P.red32, P.lp, P.pfloor = g['red32'].data_ptr(), g['lp'].data_ptr(), g['pfloor'].data_ptr()
-        P.hyper, P.red64, P.gsum = g['hyper'].data_ptr(), g['red64'].data_ptr(), g['gsum'].data_ptr()
-        P.pi_d, P.scal, P.elbo_trace = g['pi'].data_ptr(), g['scal'].data_ptr(), g['trace'].data_ptr()
-        P.xcol = g['xcol'].data_ptr()
-        return P
+            row = {q: s[q] for q in ('X', 'a1', 'a2', 'U_hat', 'eU', 'Zi', 'a2s', 'eUw', 'xrow', 'tc_ws')}
+        return build_problem(n_rows=rows, n_total=self.n_total, ldx=self._ldx, p=self.p, K=self.k, KP=self._KP,
+                             flags=self._flags, trace_cap=4, **self._g, **row)
 
     def _call(self, name, P, *args, stream=None):
         st = ctypes.c_void_p((stream or torch.cuda.current_stream()).cuda_stream)
@@ -482,7 +451,7 @@ class HostStreamedCAVI:
         self.scal.copy_(g['scal'], non_blocking=True)
         self.d2h_bytes += 4 * K * 8 + _lib.SCAL_SLOTS * 8
         if self.dropout:
-            self.pi_d.copy_(g['pi'], non_blocking=True)
+            self.pi_d.copy_(g['pi_d'], non_blocking=True)
             self.lp.copy_(g['lp'], non_blocking=True); self.pfloor.copy_(g['pfloor'], non_blocking=True)
             self.d2h_bytes += self.p * 16
 

@@ -26,15 +26,9 @@ from .. import _lib
 from ..dims import Dimensions
 from ..nodes import Einsum
 from ..parameters import Parameter
+from ..problem import build_problem, gene_buffers, kernel_plan, row_pitch
 from ..sharding import RowSharding
 from ..singlecell.cmatrix import CountMatrix
-
-
-def pad_k(K):
-    for kp in (8, 16, 32, 64):
-        if K <= kp:
-            return kp
-    raise ValueError('k=%d: the CUDA kernels support latent dimensions up to 64' % K)
 
 
 class DeviceView(Parameter):
@@ -92,27 +86,15 @@ class FactorModel(metaclass=ABCMeta):
         self.n = int(cmatrix.shape[0])
         self.m = self.p = int(cmatrix.shape[1])
         self.dims = Dimensions({'n': self.n, 'm': self.m, 'p': self.p, 'k': self.k})
-        # kernel family: the tcgen05/TMA tensor path (K <= 64, tf32 contractions with fp32 accumulation) for
-        # problems large enough to fill the machine, the CUDA-core fp32 kernels otherwise (or when forced)
-        if tensor is None:
-            tensor = (not force_simt) and self.k <= 64 and self.n * self.p >= (1 << 21)
-        if tensor and (self.k > 64 or force_simt):
-            raise ValueError('the tensor path needs k <= 64 and force_simt=False')
-        # precise=True: fp32-grade arithmetic everywhere.  On the tensor path (k <= 32) R, D_hat and the factor operands of
-        # the accumulating contractions are split hi/lo like the denominator (ORI_F_PRECISE, about half the rate of the
-        # default TF32-operand kernels); for k > 32 the CUDA-core kernels are used.
         self.precise = bool(precise)
-        if self.precise and tensor and self.k > 32:
-            tensor = False
-        self._tensor = bool(tensor)
-        self._KP = (32 if self.k <= 32 else 64) if self._tensor else pad_k(self.k)
+        self._tensor, self._KP, plan_flags = kernel_plan(self.k, self.n * self.p, precise=self.precise, tensor=tensor,
+                                                         force_simt=force_simt, sparse=self._sparse)
         self._shard = RowSharding(process_group if (sharded or process_group is not None) else None,
                                   enabled=bool(sharded or process_group is not None))
         self.n_total = self._shard.total_rows(self.n, self._dev)
         self._flags = (_lib.ORI_F_DROPOUT if self._dropout else 0) | (_lib.ORI_F_ELBO if elbo else 0) \
-            | (_lib.ORI_F_QUIRK if (compat_quirk and self._dropout) else 0) \
-            | (_lib.ORI_F_NO_TENSOR if force_simt else 0) | (_lib.ORI_F_SPARSE if self._sparse else 0) \
-            | (_lib.ORI_F_DEVICE_ITER if graphs else 0) | (_lib.ORI_F_PRECISE if (self.precise and self._tensor) else 0)
+            | (_lib.ORI_F_QUIRK if (compat_quirk and self._dropout) else 0) | (_lib.ORI_F_SPARSE if self._sparse else 0) \
+            | (_lib.ORI_F_DEVICE_ITER if graphs else 0) | plan_flags
         # graphs=True: step() replays one captured CUDA graph per generation parity (every launch of the iteration and
         # the memsets) instead of ~15 separate launches; single rank only
         if graphs and (sharded or process_group is not None):
@@ -172,7 +154,7 @@ class FactorModel(metaclass=ABCMeta):
         dev, n, p, K, KP = self._dev, self.n, self.p, self.k, self._KP
         f32 = dict(dtype=torch.float32, device=dev)
         f64 = dict(dtype=torch.float64, device=dev)
-        ldx = (p + 3) // 4 * 4
+        ldx = row_pitch(p)
         src = cmatrix.as_tensor()
         if isinstance(src, torch.Tensor) and src.is_cuda and src.dtype == torch.float32 \
                 and src.shape[1] == p and src.stride(1) == 1 and src.stride(0) % 4 == 0 \
@@ -192,63 +174,33 @@ class FactorModel(metaclass=ABCMeta):
 
         def genef():
             return torch.zeros((p, KP), **f32)
-        self._a1, self._a2 = rowf(), rowf()
-        self._Uhat = [rowf(), rowf()]
-        self._eU = [rowf(), rowf()]
-        self._Zi = rowf()
+        self._a1, self._a2, self._Zi = rowf(), rowf(), rowf()
+        self._Uhat, self._eU = [rowf(), rowf()], [rowf(), rowf()]
         self._a2s = rowf() if self._dropout else None
-        self._eUw = rowf() if (self._flags & _lib.ORI_F_QUIRK) else None
-        self._b1, self._b2, self._Vhat, self._eV = genef(), genef(), genef(), genef()
-        self._red32 = torch.zeros((3 if self._sparse else 2, p, KP), **f32)
-        self._lp = torch.full((p,), float('-inf'), **f32) if self._dropout else None
-        self._pfloor = torch.zeros((p,), **f32) if self._dropout else None
-        self._hyper = torch.ones((4, K), **f64)
-        self._red64 = torch.zeros((p + 2 * KP + _lib.R64_NSLOTS,), **f64)
-        self._gsum = torch.zeros((2 * KP + 8,), **f64)
-        self._pi = torch.zeros((p,), **f64) if self._dropout else None
-        self._scal = torch.zeros((_lib.SCAL_SLOTS,), **f64)
-        self._trace = torch.zeros((self._trace_cap,), **f64)
+        g = gene_buffers(p, K, KP, dev, dropout=self._dropout, sparse=self._sparse, trace_cap=self._trace_cap)
+        self._b1, self._b2, self._Vhat, self._eV, self._red32 = g['b1'], g['b2'], g['V_hat'], g['eV'], g['red32']
+        self._lp, self._pfloor, self._pi, self._hyper = g['lp'], g['pfloor'], g['pi_d'], g['hyper']
+        self._red64, self._scal, self._trace = g['red64'], g['scal'], g['elbo_trace']
         # row sums of this rank's X and column sums of the whole X: the ELBO takes the per-row / per-gene scales of
         # the exp(E[log .]) operands back through them (include/oriana_b200.h, xrow / xcol)
-        self._xrow = self._xcol = None
+        self._xrow = xcol = None
         if self._flags & _lib.ORI_F_ELBO:
             self._xrow = torch.zeros((max(n, 1),), **f32)
             cs = torch.zeros((p,), **f64)
             _lib.check(self._lib.ori_row_sums_f32(self._X.data_ptr(), ldx, n, p, self._xrow.data_ptr(), _lib.stream_ptr()))
             _lib.check(self._lib.ori_column_sums_f64(self._X.data_ptr(), ldx, n, p, cs.data_ptr(), _lib.stream_ptr()))
-            self._xcol = self._shard.allreduce_sum(cs).to(torch.float32)
-        self._thrU = torch.zeros((2, max(n, 1)), **f32) if self.emulate_underflow else None
-        self._thrV = torch.zeros((p,), **f32) if self.emulate_underflow else None
-        self._tc_ws = None
-        if self._tensor:
-            self._tc_ws = torch.empty((int(self._lib.ori_tc_workspace_floats(n, p, KP)) + 32,), **f32)
-
-        P = _lib.OriProblem()
-        P.n_rows, P.n_total, P.ldx = n, self.n_total, ldx
-        P.p, P.K, P.KP, P.flags = p, K, KP, self._flags
-        P.iter, P.trace_cap = 0, self._trace_cap
-
-        def ptr(t):
-            return None if t is None else t.data_ptr()
-        P.X = ptr(self._X)
-        P.a1, P.a2 = ptr(self._a1), ptr(self._a2)
-        P.U_hat[0], P.U_hat[1] = ptr(self._Uhat[0]), ptr(self._Uhat[1])
-        P.eU[0], P.eU[1] = ptr(self._eU[0]), ptr(self._eU[1])
-        P.eUw, P.Zi, P.a2s = ptr(self._eUw), ptr(self._Zi), ptr(self._a2s)
-        P.b1, P.b2, P.V_hat, P.eV = ptr(self._b1), ptr(self._b2), ptr(self._Vhat), ptr(self._eV)
-        P.red32, P.lp, P.pfloor = ptr(self._red32), ptr(self._lp), ptr(self._pfloor)
-        P.hyper, P.red64, P.gsum = ptr(self._hyper), ptr(self._red64), ptr(self._gsum)
-        P.pi_d, P.scal, P.elbo_trace = ptr(self._pi), ptr(self._scal), ptr(self._trace)
-        if self._tc_ws is not None:
-            P.tc_ws, P.tc_ws_floats = self._tc_ws.data_ptr(), self._tc_ws.numel()
-        P.xrow, P.xcol = ptr(self._xrow), ptr(self._xcol)
-        P.thrU, P.thrV = ptr(self._thrU), ptr(self._thrV)
-        self._det_ws = None
-        if self.deterministic:
-            self._det_ws = torch.zeros((int(self._lib.ori_det_workspace_doubles(n, p, KP)) + 8,), **f64)
-            P.det_ws, P.det_ws_doubles = self._det_ws.data_ptr(), self._det_ws.numel()
-        self._bind_extra(P, rowf, genef, ptr)
-        self._P = P
+            xcol = self._shard.allreduce_sum(cs).to(torch.float32)
+        under = self.emulate_underflow
+        # every array the problem points at: this dict owns the memory of those the model has no name for
+        self._arrays = dict(
+            X=self._X, a1=self._a1, a2=self._a2, U_hat=self._Uhat, eU=self._eU, Zi=self._Zi, a2s=self._a2s,
+            eUw=rowf() if (self._flags & _lib.ORI_F_QUIRK) else None, xrow=self._xrow, xcol=xcol,
+            thrU=torch.zeros((2, max(n, 1)), **f32) if under else None, thrV=torch.zeros((p,), **f32) if under else None,
+            tc_ws=torch.empty((int(self._lib.ori_tc_workspace_floats(n, p, KP)) + 32,), **f32) if self._tensor else None,
+            det_ws=torch.zeros((int(self._lib.ori_det_workspace_doubles(n, p, KP)) + 8,), **f64) if self.deterministic else None,
+            **g, **self._extra_fields(rowf, genef))
+        P = self._P = build_problem(n_rows=n, n_total=self.n_total, ldx=ldx, p=p, K=K, KP=KP, flags=self._flags,
+                                   trace_cap=self._trace_cap, **self._arrays)
         _lib.check(self._lib.ori_problem_check(ctypes.byref(P)))
         self.uses_tensor_path = bool(self._lib.ori_uses_tensor_path(ctypes.byref(P)))
         if self._tensor and not self.uses_tensor_path and n > 0:
@@ -264,8 +216,9 @@ class FactorModel(metaclass=ABCMeta):
         self.beta1 = DeviceView(self, lambda: self._hyper[2])
         self.beta2 = DeviceView(self, lambda: self._hyper[3])
 
-    def _bind_extra(self, P, rowf, genef, ptr):
-        """Hook for model-specific device state (SparseZIGaP)."""
+    def _extra_fields(self, rowf, genef):
+        """Hook for model-specific device state (SparseZIGaP): further `ori_problem_t` fields by name."""
+        return {}
 
     def _call(self, name, *args):
         self._P.iter = self._iter

@@ -36,31 +36,20 @@ class SparseZIGaP(ZIGaP):
     def __init__(self, *args, tau=0.5, **kwargs):
         if kwargs.get('compat_quirk'):
             raise ValueError('compat_quirk is a ZIGaP switch (zigap.py:94); sparse_zigap.py:115 has the correct index')
-        k = kwargs.get('k', args[1] if len(args) > 1 else 2)
-        if k > 64:
-            raise ValueError('SparseZIGaP supports k <= 64')
-        if k > 32:                                                # the tensor plans of this model exist for k <= 32
-            if kwargs.get('tensor'):
-                raise ValueError('SparseZIGaP: the tensor path needs k <= 32 (32 < k <= 64 runs on the CUDA-core kernels)')
-            kwargs['tensor'] = False
         kwargs['elbo'] = False
         kwargs.setdefault('precise', True)                        # fp32-grade sums (see the module docstring)
         self._col_mean = None
         ZIGaP.__init__(self, *args, tau=tau, **kwargs)
 
     # -- device state ----------------------------------------------------------------------------------
-    def _bind_extra(self, P, rowf, genef, ptr):
-        self._ps, self._logV, self._eVd, self._eVz, self._Vh_old = genef(), genef(), genef(), genef(), genef()
-        self._eUl = [rowf(), rowf()]
+    def _extra_fields(self, rowf, genef):
+        self._ps, self._logV, self._Vh_old = genef(), genef(), genef()
         self._pis = torch.ones((self.p,), dtype=torch.float64, device=self._dev)
-        P.p_s, P.logV, P.eVd, P.eVz, P.Vh_old = (ptr(t) for t in (self._ps, self._logV, self._eVd, self._eVz,
-                                                                   self._Vh_old))
-        P.eUl[0], P.eUl[1] = ptr(self._eUl[0]), ptr(self._eUl[1])
-        P.pi_s = ptr(self._pis)
-        P.tau = float(self.tau)
         K_ = self.k
         self.p_s = DeviceView(self, lambda: self._ps[:, :K_])
         self.pi_s = DeviceView(self, lambda: self._pis, on_write=False)
+        return dict(p_s=self._ps, logV=self._logV, eVd=genef(), eVz=genef(), Vh_old=self._Vh_old, eUl=[rowf(), rowf()],
+                    pi_s=self._pis, tau=float(self.tau))
 
     # -- model graph (sparse_zigap.py:21-40) -------------------------------------------------------------
     def build_v_node(self):

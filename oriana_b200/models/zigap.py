@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 from ..nodes import Bernoulli, Gamma, Multiply, Poisson
+from ..problem import logit_pi
 from .base import DeviceView, FactorModel
 
 
@@ -87,12 +88,8 @@ class ZIGaP(FactorModel):
 
     def _set_generating_pi(self, pi_prev):
         pi = torch.as_tensor(np.asarray(pi_prev, dtype=np.float64), device=self._dev)
-        pc = torch.clamp(pi, 1e-15, 1. - 1e-15)
-        lp = torch.log(pc / (1. - pc))
-        lp = torch.where(pi <= 0, torch.full_like(lp, float('-inf')), lp)
-        lp = torch.where(pi >= 1, torch.full_like(lp, float('inf')), lp)
-        self._lp.copy_(lp.to(torch.float32))
-        self._pfloor.copy_(torch.where(pi <= 0, 1e-10, 0.).to(torch.float32))
+        lp, pfloor = logit_pi(pi)
+        self._lp.copy_(lp); self._pfloor.copy_(pfloor)
         self._pi_gen = pi.clone()
         # `_finalize()` snapshots `_pi` as the generating pi before it refreshes it: keep the two in step, so that a
         # state_dict() taken right after a load (no step in between) carries the same pi_prev it was loaded with

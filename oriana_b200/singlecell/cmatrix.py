@@ -151,10 +151,11 @@ class CountMatrix:
         """float32 [n, p] view of a [n, ldx] device buffer (ldx = p rounded up to 4: the kernels' row pitch), filled
         slab by slab; integer counts cross PCIe in their narrow type and are widened by `ori_widen_counts_f32`."""
         from .. import _lib
+        from ..problem import row_pitch
         lib = _lib.load()
         dev = torch.device(device)
         n, p = self.shape
-        ldx = (p + 3) // 4 * 4
+        ldx = row_pitch(p)
         out = torch.zeros((n, ldx), dtype=torch.float32, device=dev)
         if isinstance(self._data, torch.Tensor) and self._data.is_cuda:
             out[:, :p] = self._data.to(torch.float32)

@@ -8,13 +8,14 @@ section 2 #13), so the bench does not use it.
 import torch
 
 from .. import _lib
+from ..problem import row_pitch
 
 
 def synth_counts_device(n_rows, p, K, seed=0, zero_level=0.5, nb=True, row0=0, ldx=None, chunk_rows=None):
     """Returns a float32 CUDA tensor [n_rows, ldx] (ldx = p rounded up to 4; pad columns are zero)."""
     dev = _lib.require_cuda()
     lib = _lib.load()
-    ldx = ldx or (p + 3) // 4 * 4
+    ldx = ldx or row_pitch(p)
     X = torch.empty((n_rows, ldx), dtype=torch.float32, device=dev)
     chunk = chunk_rows or max(1, min(n_rows, (1 << 28) // max(1, ldx)))
     Vs = torch.empty((p, K), dtype=torch.float32, device=dev)
