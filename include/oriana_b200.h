@@ -4,7 +4,7 @@
  * (oriana/models/base.py:54-56) for the ZIGaP and GaP models (and, behind ORI_F_SPARSE, SparseZIGaP,
  * oriana/models/sparse_zigap.py:100-204, with the deviance metrics of base.py:58-82), i.e. the E-step
  * `update_variational_parameters` (oriana/models/zigap.py:97-141, gap.py:82-115) with its numba kernel
- * `compute_Z_q_expectations` (zigap.py:79-95, gap.py:67-80), the node expectations `Gamma.mean/meanlog`
+ * `compute_Z_q_expectations` (zigap.py:79-95, gap.py:67-80, sparse_zigap.py:100-116), the node expectations `Gamma.mean/meanlog`
  * (oriana/nodes/probabilistic/gamma.py:37-61), `Bernoulli.mean` (bernoulli.py:41-48), and the M-step
  * `update_prior_hyper_parameters` (zigap.py:143-158, gap.py:117-129) with `inverse_digamma`
  * (oriana/utils.py:39-51).
@@ -264,6 +264,22 @@ int ori_zigap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* DZ_hat_i, floa
 int ori_gap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* Z_hat_i, float* Z_hat_j,
                                          const float* log_U_hat, const float* log_V_hat,
                                          const float* X, int64_t n, int64_t p, int64_t K);
+/* `SparseZIGaP.compute_Z_q_expectations` (sparse_zigap.py:100-116), same argument order: C-contiguous float32 HOST
+ * arrays, log_U_hat [n x K], log_V_hat = E[log V'] [p x K], S_tilde = the mask (p_s > tau) and S_hat [p x K], D_hat and
+ * X [n x p].  DSZ_hat [n x K], DZ_hat [p x K] and DZ_exp_logsum_hat [p x K] are overwritten; all three outputs and
+ * D_hat are required (the reference's S-step reads the third, sparse_zigap.py:155).  K <= 64 (ORI_EUNSUPPORTED above).
+ * Row slabs of >= 2^21 entries with K <= 32 run the tcgen05 passes with fp32-grade contractions (ORI_F_PRECISE), all
+ * other slabs the CUDA-core kernels.  Synchronous. */
+int ori_sparse_zigap_compute_Z_q_expectations_host(float* DSZ_hat, float* DZ_hat, float* DZ_exp_logsum_hat,
+                                                   const float* log_U_hat, const float* log_V_hat,
+                                                   const float* S_tilde, const float* S_hat,
+                                                   const float* D_hat, const float* X,
+                                                   int64_t n, int64_t p, int64_t K);
+int ori_sparse_zigap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* DSZ_hat, float* DZ_hat, float* DZ_exp_logsum_hat,
+                                                  const float* log_U_hat, const float* log_V_hat,
+                                                  const float* S_tilde, const float* S_hat,
+                                                  const float* D_hat, const float* X,
+                                                  int64_t n, int64_t p, int64_t K);
 
 /* ---- synthetic counts on device (SURVEY.md section 8d; bench only) ------------------------------- */
 /* X[i, j] = Poisson(g_ij * sum_k U*[i,k] V*[j,k]) * Bernoulli(pi_j) with U*, V* ~ Gamma(2, 1/2),

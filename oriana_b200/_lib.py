@@ -76,6 +76,8 @@ _SIGNATURES = {
     'ori_ctx_stats': ([C.c_void_p] + [C.POINTER(C.c_uint64)] * 4, C.c_int),
     'ori_zigap_compute_Z_q_expectations_ctx': ([C.c_void_p] * 8 + [C.c_int64] * 3 + [C.c_int], C.c_int),
     'ori_gap_compute_Z_q_expectations_ctx': ([C.c_void_p] * 6 + [C.c_int64] * 3, C.c_int),
+    'ori_sparse_zigap_compute_Z_q_expectations_host': ([C.c_void_p] * 9 + [C.c_int64] * 3, C.c_int),
+    'ori_sparse_zigap_compute_Z_q_expectations_ctx': ([C.c_void_p] * 10 + [C.c_int64] * 3, C.c_int),
     'ori_widen_counts_f32': ([C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p], C.c_int),
     'ori_expand_bitmap_counts_f32': ([C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
                                       C.c_int32, C.c_void_p], C.c_int),

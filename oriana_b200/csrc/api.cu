@@ -87,6 +87,25 @@ __global__ void k_exp_pad(const float* __restrict__ logE, const float* __restric
     }
     out[idx] = v;
 }
+// sparse model's gene-side operands (sparse_zigap.py:109, :114): eVd = centred exp(lV) * S_tilde (denominator), eVz =
+// eVd * S_hat (row sums); thr from the UNMASKED lV -- the reference's mask multiplies after its float32 exp
+__global__ void k_exp_pad_sparse(const float* __restrict__ logE, const float* __restrict__ St, const float* __restrict__ Sh,
+                                 float* __restrict__ eVd, float* __restrict__ eVz, float* __restrict__ thr_out,
+                                 long long rows, int K, int KP) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= rows * KP) return;
+    const long long i = idx / KP; const int k = (int)(idx % KP);
+    float vd = 0.f, vz = 0.f;
+    if (k < K) {
+        float m = -INFINITY;
+        for (int q = 0; q < K; ++q) m = fmaxf(m, logE[i * K + q]);
+        if (k == 0) thr_out[i] = underflow_thr_f32(m);
+        vd = centred_exp_f32(logE[i * K + k], m) * St[i * K + k];
+        vz = vd * Sh[i * K + k];
+    }
+    eVd[idx] = vd;
+    eVz[idx] = vz;
+}
 __global__ void k_mul(const float* __restrict__ a, const float* __restrict__ b, float* __restrict__ out, long long n) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = a[i] * b[i];
@@ -413,7 +432,7 @@ struct ori_ctx {
     unsigned long long staged_bytes = 0;
     struct Buf { void* p = nullptr; size_t cap = 0; };
     enum { X0, X1, D0, D1, LUS0, LUS1, EU0, EU1, EUW0, EUW1, EUL0, EUL1, ZI0, ZI1, OI0, OI1, WS0, WS1, THRU0, THRU1,
-           LVRAW, EV, ZJ, ZJ3A, ZJ3B, OUTJ, D64, THRV, NBUF };
+           LVRAW, EV, ZJ, ZJ3A, ZJ3B, OUTJ, D64, THRV, EVZ, SRAW, NBUF };     // EVZ, SRAW: sparse calls only
     Buf buf[NBUF];
     unsigned long long allocs = 0, calls = 0, tensor_slabs = 0, simt_slabs = 0;
     int64_t slab_rows = 0;     // 0: ~256 MB of X per slab
@@ -496,15 +515,27 @@ struct ori_ctx {
     template <class T> T* as(int id) { return (T*)buf[id].p; }
 };
 
-static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_out, const float* logU, const float* logV,
-                          const float* D, const float* X, int64_t n, int64_t p, int64_t K, int quirk)
+static int z_operator_args(const float* Zi_out, const float* Zj_out, const float* logU, const float* logV, const float* D,
+                           const float* X, int64_t n, int64_t p, int64_t K, int quirk)
 {
-    if (!C) return set_error(ORI_EINVAL, "null context");
     if (n < 0 || p <= 0 || K <= 0) return set_error(ORI_EINVAL, "bad shape n=%lld p=%lld K=%lld", (long long)n, (long long)p, (long long)K);
     if (p > 0x7fffffff) return set_error(ORI_EINVAL, "p too large");
     if (!Zi_out || !Zj_out || !logU || !logV || !X) return set_error(ORI_EINVAL, "null array (the reference raises TypeError, zigap.py:79)");
     if (pad_k(K) < 0) return set_error(ORI_EUNSUPPORTED, "K=%lld > 64 is not supported", (long long)K);
     if (quirk && D && p < K) return set_error(ORI_EINVAL, "quirk mode needs p >= K");
+    return ORI_OK;
+}
+
+// St, Sh non-NULL: the sparse model's operator (sparse_zigap.py:100-116), with D and Z3_out required.  Its denominator
+// operand carries the mask S_tilde, the row sums contract with eVd * S_hat, the third gene sum is always formed, and the
+// kernel family follows the sparse model's plan (tensor path for K <= 32 only, in the fp32-grade mode).
+static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_out, const float* logU, const float* logV,
+                          const float* St, const float* Sh, const float* D, const float* X, int64_t n, int64_t p, int64_t K,
+                          int quirk)
+{
+    if (!C) return set_error(ORI_EINVAL, "null context");
+    ORI_TRY(z_operator_args(Zi_out, Zj_out, logU, logV, D, X, n, p, K, quirk));
+    const bool sparse = St != nullptr;
     if (n == 0) { memset(Zj_out, 0, sizeof(float) * p * K); if (Z3_out) memset(Z3_out, 0, sizeof(float) * p * K); return ORI_OK; }
     std::lock_guard<std::mutex> lock(C->mu);
     ++C->calls;
@@ -517,8 +548,10 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     if (slab > n) slab = n;
     const int nbuf = n > slab ? 2 : 1;
     // kernel family: slabs that fill the machine take the tcgen05 / TMA passes (GaP-shaped: D_hat is an explicit input
-    // here, folded into X), smaller ones the CUDA-core kernels -- the same rule as the device models
-    const bool tensor = slab * p >= (1ll << 21);
+    // here, folded into X), smaller ones the CUDA-core kernels -- the same rule as the device models.  The sparse model:
+    // K <= 32 only, with fp32-grade contractions (its S-step is a sigmoid of the difference of two large gene sums,
+    // sparse_zigap.py:155-157, which amplifies their absolute error exponentially: no TF32 operands)
+    const bool tensor = slab * p >= (1ll << 21) && !(sparse && K > 32);
     const int KP = tensor ? (K <= 32 ? 32 : 64) : pad_k(K);
     const size_t ws_floats = tensor ? (size_t)tc_workspace_floats(slab, (int)p, KP) + 32 : 0;
 
@@ -528,7 +561,7 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         if (D) ORI_TRY(C->need(B::D0 + b, sizeof(float) * slab * ldx));
         ORI_TRY(C->need(B::LUS0 + b, sizeof(float) * slab * K));
         ORI_TRY(C->need(B::EU0 + b, sizeof(float) * slab * KP));
-        ORI_TRY(C->need(B::EUW0 + b, sizeof(float) * slab * KP));
+        if (!sparse) ORI_TRY(C->need(B::EUW0 + b, sizeof(float) * slab * KP));
         if (Z3_out) ORI_TRY(C->need(B::EUL0 + b, sizeof(float) * slab * KP));
         ORI_TRY(C->need(B::ZI0 + b, sizeof(float) * slab * KP));
         ORI_TRY(C->need(B::OI0 + b, sizeof(float) * slab * K));
@@ -537,9 +570,16 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     }
     ORI_TRY(C->need(B::LVRAW, sizeof(float) * p * K));
     ORI_TRY(C->need(B::EV, sizeof(float) * p * KP));
-    ORI_TRY(C->need(B::ZJ, sizeof(float) * 2 * p * KP));
-    ORI_TRY(C->need(B::ZJ3A, sizeof(float) * 2 * p * KP));
-    ORI_TRY(C->need(B::ZJ3B, sizeof(float) * 2 * p * KP));
+    // gene sums [Zj | (unused) | Zl]: the third block for the sparse model's Zl
+    const size_t zj_bytes = sizeof(float) * (sparse ? 3 : 2) * p * KP;
+    ORI_TRY(C->need(B::ZJ, zj_bytes));
+    if (sparse) {
+        ORI_TRY(C->need(B::EVZ, sizeof(float) * p * KP));
+        ORI_TRY(C->need(B::SRAW, sizeof(float) * 2 * p * K));
+    } else {
+        ORI_TRY(C->need(B::ZJ3A, sizeof(float) * 2 * p * KP));
+        ORI_TRY(C->need(B::ZJ3B, sizeof(float) * 2 * p * KP));
+    }
     ORI_TRY(C->need(B::OUTJ, sizeof(float) * p * K));
     ORI_TRY(C->need(B::D64, sizeof(double) * (p + 2 * KP + R64_NSLOTS)));
     ORI_TRY(C->need(B::THRV, sizeof(float) * p));
@@ -552,11 +592,22 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     ORI_CUDA(cudaMemcpyAsync(dlogVraw, logV, sizeof(float) * p * K, cudaMemcpyHostToDevice, st));
     // the operator IS the reference's numba loop: its float32 exp underflow (den = 0 -> 1, zigap.py:86-90) is part of
     // the contract here, so the thresholds are always on
-    k_exp_pad<<<cdiv(p * KP, 256), 256, 0, st>>>(dlogVraw, nullptr, 0, 0, deV, p, (int)K, KP, C->as<float>(B::THRV));
+    float* deVz = sparse ? C->as<float>(B::EVZ) : nullptr;
+    if (sparse) {    // deV = eVd (denominator, masked by S_tilde), deVz = eVd * S_hat (row sums)
+        float* dS = C->as<float>(B::SRAW);
+        ORI_CUDA(cudaMemcpyAsync(dS, St, sizeof(float) * p * K, cudaMemcpyHostToDevice, st));
+        ORI_CUDA(cudaMemcpyAsync(dS + p * K, Sh, sizeof(float) * p * K, cudaMemcpyHostToDevice, st));
+        k_exp_pad_sparse<<<cdiv(p * KP, 256), 256, 0, st>>>(dlogVraw, dS, dS + p * K, deV, deVz, C->as<float>(B::THRV),
+                                                            p, (int)K, KP);
+    } else {
+        k_exp_pad<<<cdiv(p * KP, 256), 256, 0, st>>>(dlogVraw, nullptr, 0, 0, deV, p, (int)K, KP, C->as<float>(B::THRV));
+    }
     ORI_TRY(check_launch("k_exp_pad"));
-    ORI_CUDA(cudaMemsetAsync(dZj, 0, sizeof(float) * 2 * p * KP, st));
-    ORI_CUDA(cudaMemsetAsync(dZj3a, 0, sizeof(float) * 2 * p * KP, st));
-    ORI_CUDA(cudaMemsetAsync(dZj3b, 0, sizeof(float) * 2 * p * KP, st));
+    ORI_CUDA(cudaMemsetAsync(dZj, 0, zj_bytes, st));
+    if (!sparse) {
+        ORI_CUDA(cudaMemsetAsync(dZj3a, 0, sizeof(float) * 2 * p * KP, st));
+        ORI_CUDA(cudaMemsetAsync(dZj3b, 0, sizeof(float) * 2 * p * KP, st));
+    }
     // [0],[1]: last work on each stream; [2]: gene-side operands ready
     ORI_CUDA(cudaEventRecord(C->ev[2], st));
     ORI_CUDA(cudaStreamWaitEvent(st2, C->ev[2], 0));
@@ -565,14 +616,21 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     memset(&P, 0, sizeof(P));
     P.p = (int)p; P.K = (int)K; P.KP = KP; P.ldx = ldx;
     P.eV = deV; P.V_hat = deV;
+    P.eVd = deV; P.eVz = deVz;
     P.thrV = C->as<float>(B::THRV);
     P.red64 = C->as<double>(B::D64);
+    // the sparse problem has no dropout layer (D_hat is folded into X): ori_problem_check refuses it from outside callers
+    const uint32_t flags = sparse ? ORI_F_SPARSE | (tensor ? ORI_F_PRECISE : 0u) : 0u;
 
-    // gene sums of one slab (zigap.py:94): both streams add into the same accumulators with atomics
+    // gene sums of one slab (zigap.py:94): both streams add into the same accumulators with atomics.  Sparse: Zj and Zl
+    // (sparse_zigap.py:115-116), in one sweep on the CUDA-core kernels, in a second dropout-free sweep on the tensor path
     auto genes = [&](cudaStream_t s) -> int {
         if (!tc_eligible(&P)) return launch_pass_genes_simt(&P, 0, s);
         ORI_TRY(launch_tc_prep_rows(&P, 0, s));
-        return launch_pass_genes_tc(&P, 0, s);
+        ORI_TRY(launch_pass_genes_tc(&P, 0, s));
+        if (!(P.flags & ORI_F_SPARSE)) return ORI_OK;
+        ORI_TRY(launch_tc_prep_rows_logsum(&P, 0, s));
+        return launch_pass_genes_logsum_tc(&P, 0, s);
     };
     auto rows = [&](cudaStream_t s) -> int {
         if (!tc_eligible(&P)) return launch_pass_rows_simt(&P, 0, s);
@@ -609,8 +667,9 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         }
         ORI_TRY(check_launch("operator prologue"));
         ORI_CUDA(cudaMemsetAsync(dZi, 0, sizeof(float) * nr * KP, s));
-        P.n_rows = nr; P.n_total = n; P.flags = 0;
+        P.n_rows = nr; P.n_total = n; P.flags = flags;
         P.eU[0] = deU; P.U_hat[0] = deU; P.U_hat[1] = deU;
+        if (sparse) P.eUl[0] = deUl;
         P.Zi = dZi;
         P.thrU = C->as<float>(B::THRU0 + b);
         P.tc_ws = tensor ? C->as<float>(B::WS0 + b) : nullptr;
@@ -625,7 +684,7 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         if (D && quirk) { P.X = xq; P.flags = ORI_F_QUIRK; P.eUw = deUw; }
         P.red32 = dZj;
         ORI_TRY(genes(s));
-        if (Z3_out) {  // zigap.py:95 = eV * (R_D^T (eU*logU)) + logV * [eV * (R_D^T eU)]
+        if (Z3_out && !sparse) {  // zigap.py:95 = eV * (R_D^T (eU*logU)) + logV * [eV * (R_D^T eU)]
             P.X = x; P.flags = ORI_F_QUIRK; P.eUw = deUl; P.red32 = dZj3a;
             ORI_TRY(genes(s));
             if (D && quirk) { P.flags = 0; P.red32 = dZj3b; ORI_TRY(genes(s)); }
@@ -636,9 +695,10 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     ORI_CUDA(cudaStreamWaitEvent(st, C->ev[1 % nbuf], 0));
     k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(dZj, deV, nullptr, nullptr, dOutJ, p, (int)K, KP);
     ORI_CUDA(cudaMemcpyAsync(Zj_out, dOutJ, sizeof(float) * p * K, cudaMemcpyDeviceToHost, st));
-    if (Z3_out) {
+    if (Z3_out) {   // sparse_zigap.py:116 likewise: eVd * Zl + logV * DZ_hat
         const float* plain = (D && quirk) ? dZj3b : dZj;
-        k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(dZj3a, deV, plain, dlogVraw, dOutJ, p, (int)K, KP);
+        k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(sparse ? dZj + 2 * p * KP : dZj3a, deV, plain, dlogVraw, dOutJ, p,
+                                                        (int)K, KP);
         ORI_CUDA(cudaMemcpyAsync(Z3_out, dOutJ, sizeof(float) * p * K, cudaMemcpyDeviceToHost, st));
     }
     ORI_TRY(check_launch("operator epilogue"));
@@ -697,12 +757,12 @@ int ori_zigap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* DZ_hat_i, floa
                                            const float* D_hat, const float* X,
                                            int64_t n, int64_t p, int64_t K, int quirk) {
     if (!D_hat) return set_error(ORI_EINVAL, "D_hat is NULL");
-    return z_operator_ctx(ctx, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, D_hat, X, n, p, K, quirk);
+    return z_operator_ctx(ctx, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, nullptr, nullptr, D_hat, X, n, p, K, quirk);
 }
 
 int ori_gap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* Z_hat_i, float* Z_hat_j, const float* log_U_hat,
                                          const float* log_V_hat, const float* X, int64_t n, int64_t p, int64_t K) {
-    return z_operator_ctx(ctx, Z_hat_i, Z_hat_j, nullptr, log_U_hat, log_V_hat, nullptr, X, n, p, K, 0);
+    return z_operator_ctx(ctx, Z_hat_i, Z_hat_j, nullptr, log_U_hat, log_V_hat, nullptr, nullptr, nullptr, X, n, p, K, 0);
 }
 
 int ori_zigap_compute_Z_q_expectations_host(float* DZ_hat_i, float* DZ_hat_j, float* DZ_exp_logsum_hat,
@@ -713,7 +773,7 @@ int ori_zigap_compute_Z_q_expectations_host(float* DZ_hat_i, float* DZ_hat_j, fl
     int rc;
     ori_ctx* c = default_ctx(&rc);
     if (!c) return rc;
-    return z_operator_ctx(c, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, D_hat, X, n, p, K, quirk);
+    return z_operator_ctx(c, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, nullptr, nullptr, D_hat, X, n, p, K, quirk);
 }
 
 int ori_gap_compute_Z_q_expectations_host(float* Z_hat_i, float* Z_hat_j, const float* log_U_hat,
@@ -721,7 +781,37 @@ int ori_gap_compute_Z_q_expectations_host(float* Z_hat_i, float* Z_hat_j, const 
     int rc;
     ori_ctx* c = default_ctx(&rc);
     if (!c) return rc;
-    return z_operator_ctx(c, Z_hat_i, Z_hat_j, nullptr, log_U_hat, log_V_hat, nullptr, X, n, p, K, 0);
+    return z_operator_ctx(c, Z_hat_i, Z_hat_j, nullptr, log_U_hat, log_V_hat, nullptr, nullptr, nullptr, X, n, p, K, 0);
+}
+
+// sparse_zigap.py:100-116: D_hat, S_tilde, S_hat and the third output (read by the S-step, :155) are required; checked
+// with the shape before any device work
+static int sparse_args(const float* DSZ_hat, const float* DZ_hat, const float* DZ_exp_logsum_hat, const float* log_U_hat,
+                       const float* log_V_hat, const float* S_tilde, const float* S_hat, const float* D_hat, const float* X,
+                       int64_t n, int64_t p, int64_t K) {
+    if (!D_hat) return set_error(ORI_EINVAL, "D_hat is NULL");
+    if (!DZ_exp_logsum_hat) return set_error(ORI_EINVAL, "DZ_exp_logsum_hat is NULL (sparse_zigap.py:155 reads it)");
+    if (!S_tilde || !S_hat) return set_error(ORI_EINVAL, "S_tilde / S_hat is NULL");
+    return z_operator_args(DSZ_hat, DZ_hat, log_U_hat, log_V_hat, D_hat, X, n, p, K, 0);
+}
+
+int ori_sparse_zigap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* DSZ_hat, float* DZ_hat, float* DZ_exp_logsum_hat,
+                                                  const float* log_U_hat, const float* log_V_hat, const float* S_tilde,
+                                                  const float* S_hat, const float* D_hat, const float* X,
+                                                  int64_t n, int64_t p, int64_t K) {
+    ORI_TRY(sparse_args(DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat, S_tilde, S_hat, D_hat, X, n, p, K));
+    return z_operator_ctx(ctx, DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat, S_tilde, S_hat, D_hat, X, n, p, K, 0);
+}
+
+int ori_sparse_zigap_compute_Z_q_expectations_host(float* DSZ_hat, float* DZ_hat, float* DZ_exp_logsum_hat,
+                                                   const float* log_U_hat, const float* log_V_hat, const float* S_tilde,
+                                                   const float* S_hat, const float* D_hat, const float* X,
+                                                   int64_t n, int64_t p, int64_t K) {
+    ORI_TRY(sparse_args(DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat, S_tilde, S_hat, D_hat, X, n, p, K));
+    int rc;
+    ori_ctx* c = default_ctx(&rc);
+    if (!c) return rc;
+    return z_operator_ctx(c, DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat, S_tilde, S_hat, D_hat, X, n, p, K, 0);
 }
 
 }  // extern "C"

@@ -44,7 +44,8 @@ constexpr int PR_TG = 32;
 
 // SPARSE (sparse_zigap.py:100-116, :140-142, :166): the denominator operand eV carries the mask S_tilde, the row
 // sums contract with eVz = eV * S_hat, D_hat is rebuilt from Vh = the PREVIOUS effective V_hat and the rate sums
-// contract with Vc = the current one.  Otherwise eVz == eV and Vc == Vh (not read).
+// contract with Vc = the current one.  Otherwise eVz == eV and Vc == Vh (not read).  SPARSE without DROPOUT (the
+// operator seam, D_hat folded into X): Vh and Vc are not read.
 // TG: genes per tile (32; 16 for the sparse model at KP = 64, whose four gene-side operand tiles would not fit 48 KB)
 template <int KP, bool DROPOUT, bool ELBO, bool SPARSE, int TG = PR_TG>
 __global__ void __launch_bounds__(PR_TR)
@@ -65,7 +66,7 @@ k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
     __shared__ __align__(16) float sV[TG][KP];
     __shared__ __align__(16) float sVh[DROPOUT ? TG : 1][KP];
     __shared__ __align__(16) float sVz[SPARSE ? TG : 1][KP];
-    __shared__ __align__(16) float sVc[SPARSE ? TG : 1][KP];
+    __shared__ __align__(16) float sVc[SPARSE && DROPOUT ? TG : 1][KP];
     __shared__ float slp[TG], sfl[TG];
     __shared__ float scs[PR_TR / 32][TG];
     __shared__ double sred[PR_TR / 32];
@@ -108,7 +109,7 @@ k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
             if (DROPOUT) sVhf[idx] = ok ? Vh[(long long)j0 * KP + idx] : 0.f;
             if (SPARSE) {
                 sVzf[idx] = ok ? eVz[(long long)j0 * KP + idx] : 0.f;
-                sVcf[idx] = ok ? Vc[(long long)j0 * KP + idx] : 0.f;
+                if (DROPOUT) sVcf[idx] = ok ? Vc[(long long)j0 * KP + idx] : 0.f;
             }
         }
         if (DROPOUT && tid < TG) {
@@ -162,7 +163,7 @@ k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
             }
             if (ELBO && nz) t_xl = fmaf(x, logf(den), t_xl);
             const float4* z4 = SPARSE ? reinterpret_cast<const float4*>(&sVz[SPARSE ? g : 0][0]) : v4;
-            const float4* c4 = SPARSE ? reinterpret_cast<const float4*>(&sVc[SPARSE ? g : 0][0]) : h4;
+            const float4* c4 = SPARSE ? reinterpret_cast<const float4*>(&sVc[SPARSE && DROPOUT ? g : 0][0]) : h4;
 #pragma unroll
             for (int q = 0; q < KP / 4; ++q) {
                 const float4 v = z4[q];
@@ -1045,11 +1046,15 @@ static int pass_rows_kp(const ori_problem_t* P, int g, cudaStream_t st) {
         return nk ? check_launch("k_det_sum_cols", nk) : ORI_OK;
     };
     dim3 grid(bx, gy);
-    if (P->flags & ORI_F_SPARSE) {
-        k_pass_rows<KP, true, false, true, TGS><<<grid, PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->eU[g],
-            P->U_hat[g], P->eVd, P->Vh_old, P->eVz, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part,
-            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,
-            det_cs, det_part);
+    if (P->flags & ORI_F_SPARSE) {      // without ORI_F_DROPOUT: the operator seam (api.cu), D_hat folded into X
+#define ORI_LAUNCH_PRS(D)                                                                                       \
+        k_pass_rows<KP, D, false, true, TGS><<<grid, PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->eU[g],    \
+            P->U_hat[g], P->eVd, P->Vh_old, P->eVz, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part,     \
+            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,    \
+            det_cs, det_part)
+        if (drop) ORI_LAUNCH_PRS(true);
+        else ORI_LAUNCH_PRS(false);
+#undef ORI_LAUNCH_PRS
         if (check_launch("k_pass_rows(sparse)") != ORI_OK) return ORI_ECUDA;
         return det_sums();
     }
@@ -1107,12 +1112,16 @@ static int pass_genes_kp(const ori_problem_t* P, int g, cudaStream_t st) {
         k_det_sum_chunks_strided<<<cdiv(total, 256), 256, 0, st>>>(P->red32, det_z, gy, total, det_stride);
         return check_launch("k_det_sum_chunks");
     };
-    if (P->flags & ORI_F_SPARSE) {
-        k_pass_genes<KP, true, false, true><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc,
-            P->eU[g], nullptr, P->U_hat[g], P->U_hat[1 - g], P->eUl[g], P->eVd, P->Vh_old, P->lp, P->pfloor,
-            Zj, b2s, P->red32 + 2ll * P->p * P->KP,
-            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,
-            det_z, det_stride);
+    if (P->flags & ORI_F_SPARSE) {      // without ORI_F_DROPOUT: the operator seam (api.cu), D_hat folded into X
+#define ORI_LAUNCH_PGS(D)                                                                                       \
+        k_pass_genes<KP, D, false, true><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc,        \
+            P->eU[g], nullptr, P->U_hat[g], P->U_hat[1 - g], P->eUl[g], P->eVd, P->Vh_old, P->lp, P->pfloor,    \
+            Zj, b2s, P->red32 + 2ll * P->p * P->KP,                                                              \
+            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,    \
+            det_z, det_stride)
+        if (drop) ORI_LAUNCH_PGS(true);
+        else ORI_LAUNCH_PGS(false);
+#undef ORI_LAUNCH_PGS
         if (check_launch("k_pass_genes(sparse)") != ORI_OK) return ORI_ECUDA;
         return det_sums();
     }
