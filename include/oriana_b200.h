@@ -99,7 +99,8 @@ typedef struct ori_problem {
     float* b2;             /* zigap.py:124 */
     float* V_hat;
     float* eV;
-    float* red32;          /* [2 x p x KP]: Zj partial | b2s partial -- allreduce(sum) buffer #1 */
+    float* red32;          /* [2 x p x KP]: Zj partial | b2s partial -- allreduce(sum) buffer #1; [3 x p x KP]
+                              with eUl (ORI_F_SPARSE) */
 
     float* lp;             /* [p] logit(pi) generating the CURRENT D_hat; -inf: D_hat=(X>0) (zigap.py:77) */
     float* pfloor;         /* [p] 1e-10 where pi<=0 (zigap.py:133), else 0               */
@@ -129,7 +130,8 @@ typedef struct ori_problem {
     float* eVz;            /* eVd * S_hat: operand of the row sums (:114)                                  */
     float* Vh_old;         /* S_hat * V'_hat of the PREVIOUS iteration: generates the current D_hat
                               (:166 multiplies the new U_hat with the V_hat local of :140)                 */
-    float* eUl[2];         /* row side, per generation: eU * E[log U] (operand of :116)                    */
+    float* eUl[2];         /* row side, per generation: eU * E[log U] (operand of :116).  Set, it asks the gene
+                              pass for the third sum in red32 block 2; only with ORI_F_SPARSE (ori_problem_check) */
     double* pi_s;          /* [p] prior of S, row means of p_s (:196), float64                             */
     double tau;            /* threshold of S_tilde (:134)                                                  */
 

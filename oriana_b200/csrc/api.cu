@@ -196,6 +196,8 @@ int ori_problem_check(const ori_problem_t* P) {
             return set_error(ORI_EINVAL, "sparse buffers missing");
         if (((uintptr_t)P->eVd & 15) || ((uintptr_t)P->eVz & 15) || ((uintptr_t)P->Vh_old & 15))
             return set_error(ORI_EINVAL, "eVd, eVz, Vh_old must be 16-byte aligned");
+    } else if (P->eUl[0] || P->eUl[1]) {
+        return set_error(ORI_EINVAL, "eUl (the third gene sum) needs ORI_F_SPARSE");
     }
     if (((uintptr_t)P->X & 15) || ((uintptr_t)P->eV & 15) || ((uintptr_t)P->V_hat & 15))
         return set_error(ORI_EINVAL, "X, eV, V_hat must be 16-byte aligned");
@@ -228,15 +230,20 @@ static int pass_rows_any(const ori_problem_t* P, int gen_old, cudaStream_t st) {
     ORI_TRY(launch_tc_prep_genes(P, st));
     return launch_pass_rows_tc(P, gen_old, st);
 }
-static int pass_genes_any(const ori_problem_t* P, int gen_old, cudaStream_t st) {
-    if (P->flags & ORI_F_QUIRK) ORI_TRY(launch_quirk_weights(P, gen_old, st));
+// gene sums: Zj | b2s, and with eUl[gen_old] the third sum sum_i R_ij eU_ik E[log U_ik] into red32 block 2 (zigap.py:95,
+// sparse_zigap.py:116) -- in the same sweep on the CUDA-core kernels, in a second, dropout-free one on the tensor path
+static int gene_sums(const ori_problem_t* P, int gen_old, cudaStream_t st) {
     if (!tc_eligible(P)) return launch_pass_genes_simt(P, gen_old, st);
     ORI_TRY(launch_tc_prep_rows(P, gen_old, st));
     ORI_TRY(launch_pass_genes_tc(P, gen_old, st));
-    if (!(P->flags & ORI_F_SPARSE)) return ORI_OK;
-    // sparse model: second, dropout-free sweep for sum_i R_ij eU_ik E[log U_ik] (sparse_zigap.py:116)
+    if (!P->eUl[gen_old]) return ORI_OK;
     ORI_TRY(launch_tc_prep_rows_logsum(P, gen_old, st));
     return launch_pass_genes_logsum_tc(P, gen_old, st);
+}
+// the models' gene pass: under the quirk the Zj weight eU * D_hat[:, :K] (zigap.py:94) comes from their own state first
+static int pass_genes_any(const ori_problem_t* P, int gen_old, cudaStream_t st) {
+    if (P->flags & ORI_F_QUIRK) ORI_TRY(launch_quirk_weights(P, gen_old, st));
+    return gene_sums(P, gen_old, st);
 }
 
 int64_t ori_tc_workspace_floats(int64_t n_rows, int32_t p, int32_t KP) { return tc_workspace_floats(n_rows, p, KP); }
@@ -280,7 +287,7 @@ static int zero_accumulators(const ori_problem_t* P, cudaStream_t st, bool genes
         ORI_CUDA(cudaMemsetAsync(P->Zi, 0, rowf_bytes(P), st));
         if (P->flags & ORI_F_DROPOUT) ORI_CUDA(cudaMemsetAsync(P->a2s, 0, rowf_bytes(P), st));
     }
-    if (genes) ORI_CUDA(cudaMemsetAsync(P->red32, 0, sizeof(float) * ((P->flags & ORI_F_SPARSE) ? 3 : 2) * (size_t)P->p * P->KP, st));
+    if (genes) ORI_CUDA(cudaMemsetAsync(P->red32, 0, sizeof(float) * (P->eUl[0] ? 3 : 2) * (size_t)P->p * P->KP, st));
     ORI_CUDA(cudaMemsetAsync(P->red64, 0, red64_bytes(P), st));
     return ORI_OK;
 }
@@ -432,7 +439,7 @@ struct ori_ctx {
     unsigned long long staged_bytes = 0;
     struct Buf { void* p = nullptr; size_t cap = 0; };
     enum { X0, X1, D0, D1, LUS0, LUS1, EU0, EU1, EUW0, EUW1, EUL0, EUL1, ZI0, ZI1, OI0, OI1, WS0, WS1, THRU0, THRU1,
-           LVRAW, EV, ZJ, ZJ3A, ZJ3B, OUTJ, D64, THRV, EVZ, SRAW, NBUF };     // EVZ, SRAW: sparse calls only
+           LVRAW, EV, ZJ, ZJ3, OUTJ, D64, THRV, EVZ, SRAW, NBUF };     // EVZ, SRAW: sparse calls only
     Buf buf[NBUF];
     unsigned long long allocs = 0, calls = 0, tensor_slabs = 0, simt_slabs = 0;
     int64_t slab_rows = 0;     // 0: ~256 MB of X per slab
@@ -527,14 +534,13 @@ static int z_operator_args(const float* Zi_out, const float* Zj_out, const float
 }
 
 // St, Sh non-NULL: the sparse model's operator (sparse_zigap.py:100-116), with D and Z3_out required.  Its denominator
-// operand carries the mask S_tilde, the row sums contract with eVd * S_hat, the third gene sum is always formed, and the
-// kernel family follows the sparse model's plan (tensor path for K <= 32 only, in the fp32-grade mode).
+// operand carries the mask S_tilde, the row sums contract with eVd * S_hat, and the kernel family follows the sparse
+// model's plan (tensor path for K <= 32 only, in the fp32-grade mode).  The arguments are checked by the entry points.
 static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_out, const float* logU, const float* logV,
                           const float* St, const float* Sh, const float* D, const float* X, int64_t n, int64_t p, int64_t K,
                           int quirk)
 {
     if (!C) return set_error(ORI_EINVAL, "null context");
-    ORI_TRY(z_operator_args(Zi_out, Zj_out, logU, logV, D, X, n, p, K, quirk));
     const bool sparse = St != nullptr;
     if (n == 0) { memset(Zj_out, 0, sizeof(float) * p * K); if (Z3_out) memset(Z3_out, 0, sizeof(float) * p * K); return ORI_OK; }
     std::lock_guard<std::mutex> lock(C->mu);
@@ -554,6 +560,13 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     const bool tensor = slab * p >= (1ll << 21) && !(sparse && K > 32);
     const int KP = tensor ? (K <= 32 ? 32 : 64) : pad_k(K);
     const size_t ws_floats = tensor ? (size_t)tc_workspace_floats(slab, (int)p, KP) + 32 : 0;
+    // the third output takes the third gene sum, weighted by D_hat[i, j] (zigap.py:95, sparse_zigap.py:116).  Under the
+    // quirk Zj is weighted by D_hat[i, k] instead (zigap.py:94): the third sum then takes a sweep over X*D_hat of its own,
+    // into ZJ3 = [plain gene sums | (unused) | Zl]; otherwise it comes out of the Zj sweep, into ZJ's third block
+    const bool qw = D && quirk;
+    const bool sweep3 = Z3_out && qw;
+    const size_t gblk = sizeof(float) * p * KP;
+    const size_t zj_bytes = (Z3_out && !sweep3 ? 3 : 2) * gblk;
 
     typedef ori_ctx B;
     for (int b = 0; b < nbuf; ++b) {
@@ -561,7 +574,7 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         if (D) ORI_TRY(C->need(B::D0 + b, sizeof(float) * slab * ldx));
         ORI_TRY(C->need(B::LUS0 + b, sizeof(float) * slab * K));
         ORI_TRY(C->need(B::EU0 + b, sizeof(float) * slab * KP));
-        if (!sparse) ORI_TRY(C->need(B::EUW0 + b, sizeof(float) * slab * KP));
+        if (qw) ORI_TRY(C->need(B::EUW0 + b, sizeof(float) * slab * KP));
         if (Z3_out) ORI_TRY(C->need(B::EUL0 + b, sizeof(float) * slab * KP));
         ORI_TRY(C->need(B::ZI0 + b, sizeof(float) * slab * KP));
         ORI_TRY(C->need(B::OI0 + b, sizeof(float) * slab * K));
@@ -570,15 +583,11 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     }
     ORI_TRY(C->need(B::LVRAW, sizeof(float) * p * K));
     ORI_TRY(C->need(B::EV, sizeof(float) * p * KP));
-    // gene sums [Zj | (unused) | Zl]: the third block for the sparse model's Zl
-    const size_t zj_bytes = sizeof(float) * (sparse ? 3 : 2) * p * KP;
     ORI_TRY(C->need(B::ZJ, zj_bytes));
+    if (sweep3) ORI_TRY(C->need(B::ZJ3, 3 * gblk));
     if (sparse) {
         ORI_TRY(C->need(B::EVZ, sizeof(float) * p * KP));
         ORI_TRY(C->need(B::SRAW, sizeof(float) * 2 * p * K));
-    } else {
-        ORI_TRY(C->need(B::ZJ3A, sizeof(float) * 2 * p * KP));
-        ORI_TRY(C->need(B::ZJ3B, sizeof(float) * 2 * p * KP));
     }
     ORI_TRY(C->need(B::OUTJ, sizeof(float) * p * K));
     ORI_TRY(C->need(B::D64, sizeof(double) * (p + 2 * KP + R64_NSLOTS)));
@@ -586,7 +595,8 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
 
     float* dlogVraw = C->as<float>(B::LVRAW);
     float* deV = C->as<float>(B::EV);
-    float* dZj = C->as<float>(B::ZJ); float* dZj3a = C->as<float>(B::ZJ3A); float* dZj3b = C->as<float>(B::ZJ3B);
+    float* dZj = C->as<float>(B::ZJ);
+    float* dZ3 = sweep3 ? C->as<float>(B::ZJ3) : dZj;     // the buffer of the third sum
     float* dOutJ = C->as<float>(B::OUTJ);
 
     ORI_CUDA(cudaMemcpyAsync(dlogVraw, logV, sizeof(float) * p * K, cudaMemcpyHostToDevice, st));
@@ -604,10 +614,7 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     }
     ORI_TRY(check_launch("k_exp_pad"));
     ORI_CUDA(cudaMemsetAsync(dZj, 0, zj_bytes, st));
-    if (!sparse) {
-        ORI_CUDA(cudaMemsetAsync(dZj3a, 0, sizeof(float) * 2 * p * KP, st));
-        ORI_CUDA(cudaMemsetAsync(dZj3b, 0, sizeof(float) * 2 * p * KP, st));
-    }
+    if (sweep3) ORI_CUDA(cudaMemsetAsync(dZ3, 0, 3 * gblk, st));
     // [0],[1]: last work on each stream; [2]: gene-side operands ready
     ORI_CUDA(cudaEventRecord(C->ev[2], st));
     ORI_CUDA(cudaStreamWaitEvent(st2, C->ev[2], 0));
@@ -622,22 +629,6 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     // the sparse problem has no dropout layer (D_hat is folded into X): ori_problem_check refuses it from outside callers
     const uint32_t flags = sparse ? ORI_F_SPARSE | (tensor ? ORI_F_PRECISE : 0u) : 0u;
 
-    // gene sums of one slab (zigap.py:94): both streams add into the same accumulators with atomics.  Sparse: Zj and Zl
-    // (sparse_zigap.py:115-116), in one sweep on the CUDA-core kernels, in a second dropout-free sweep on the tensor path
-    auto genes = [&](cudaStream_t s) -> int {
-        if (!tc_eligible(&P)) return launch_pass_genes_simt(&P, 0, s);
-        ORI_TRY(launch_tc_prep_rows(&P, 0, s));
-        ORI_TRY(launch_pass_genes_tc(&P, 0, s));
-        if (!(P.flags & ORI_F_SPARSE)) return ORI_OK;
-        ORI_TRY(launch_tc_prep_rows_logsum(&P, 0, s));
-        return launch_pass_genes_logsum_tc(&P, 0, s);
-    };
-    auto rows = [&](cudaStream_t s) -> int {
-        if (!tc_eligible(&P)) return launch_pass_rows_simt(&P, 0, s);
-        ORI_TRY(launch_tc_prep_genes(&P, s));
-        return launch_pass_rows_tc(&P, 0, s);
-    };
-
     int b = 0;
     for (int64_t r0 = 0; r0 < n; r0 += slab, b ^= (nbuf - 1)) {
         const int64_t nr = (n - r0 < slab) ? n - r0 : slab;
@@ -651,7 +642,7 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         if (D) ORI_TRY(C->h2d_rows(dD, sizeof(float) * ldx, D + r0 * p, sizeof(float) * p, nr, s));
         ORI_CUDA(cudaMemcpyAsync(dlUs, logU + r0 * K, sizeof(float) * nr * K, cudaMemcpyHostToDevice, s));
         k_exp_pad<<<cdiv(nr * KP, 256), 256, 0, s>>>(dlUs, nullptr, 0, 0, deU, nr, (int)K, KP, C->as<float>(B::THRU0 + b));
-        if (D && quirk)   // zigap.py:94: weight of cell i for latent k is D_hat[i, k]
+        if (qw)   // zigap.py:94: weight of cell i for latent k is D_hat[i, k]
             k_exp_pad<<<cdiv(nr * KP, 256), 256, 0, s>>>(dlUs, dD, ldx, 0, deUw, nr, (int)K, KP);
         if (Z3_out)
             k_exp_pad<<<cdiv(nr * KP, 256), 256, 0, s>>>(dlUs, nullptr, 0, 1, deUl, nr, (int)K, KP);
@@ -669,7 +660,6 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         ORI_CUDA(cudaMemsetAsync(dZi, 0, sizeof(float) * nr * KP, s));
         P.n_rows = nr; P.n_total = n; P.flags = flags;
         P.eU[0] = deU; P.U_hat[0] = deU; P.U_hat[1] = deU;
-        if (sparse) P.eUl[0] = deUl;
         P.Zi = dZi;
         P.thrU = C->as<float>(B::THRU0 + b);
         P.tc_ws = tensor ? C->as<float>(B::WS0 + b) : nullptr;
@@ -677,17 +667,17 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
         // row sums (zigap.py:93)
         P.X = x;
         (tc_eligible(&P) ? C->tensor_slabs : C->simt_slabs) += 1;
-        ORI_TRY(rows(s));
+        ORI_TRY(pass_rows_any(&P, 0, s));
         k_scale_unpad<<<cdiv(nr * K, 256), 256, 0, s>>>(dZi, deU, nullptr, nullptr, dOutI, nr, (int)K, KP);
         ORI_CUDA(cudaMemcpyAsync(Zi_out + r0 * K, dOutI, sizeof(float) * nr * K, cudaMemcpyDeviceToHost, s));
-        // gene sums (zigap.py:94)
-        if (D && quirk) { P.X = xq; P.flags = ORI_F_QUIRK; P.eUw = deUw; }
+        // gene sums (zigap.py:94): both streams add into the same accumulators with atomics
         P.red32 = dZj;
-        ORI_TRY(genes(s));
-        if (Z3_out && !sparse) {  // zigap.py:95 = eV * (R_D^T (eU*logU)) + logV * [eV * (R_D^T eU)]
-            P.X = x; P.flags = ORI_F_QUIRK; P.eUw = deUl; P.red32 = dZj3a;
-            ORI_TRY(genes(s));
-            if (D && quirk) { P.flags = 0; P.red32 = dZj3b; ORI_TRY(genes(s)); }
+        P.eUl[0] = Z3_out && !sweep3 ? deUl : nullptr;
+        if (qw) { P.X = xq; P.flags = ORI_F_QUIRK; P.eUw = deUw; }
+        ORI_TRY(gene_sums(&P, 0, s));
+        if (sweep3) {
+            P.X = x; P.flags = flags; P.eUl[0] = deUl; P.red32 = dZ3;
+            ORI_TRY(gene_sums(&P, 0, s));
         }
         ORI_CUDA(cudaEventRecord(C->ev[b], s));
     }
@@ -695,10 +685,8 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     ORI_CUDA(cudaStreamWaitEvent(st, C->ev[1 % nbuf], 0));
     k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(dZj, deV, nullptr, nullptr, dOutJ, p, (int)K, KP);
     ORI_CUDA(cudaMemcpyAsync(Zj_out, dOutJ, sizeof(float) * p * K, cudaMemcpyDeviceToHost, st));
-    if (Z3_out) {   // sparse_zigap.py:116 likewise: eVd * Zl + logV * DZ_hat
-        const float* plain = (D && quirk) ? dZj3b : dZj;
-        k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(sparse ? dZj + 2 * p * KP : dZj3a, deV, plain, dlogVraw, dOutJ, p,
-                                                        (int)K, KP);
+    if (Z3_out) {   // eV * Zl + logV * (eV * plain gene sums)
+        k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(dZ3 + 2 * p * KP, deV, dZ3, dlogVraw, dOutJ, p, (int)K, KP);
         ORI_CUDA(cudaMemcpyAsync(Z3_out, dOutJ, sizeof(float) * p * K, cudaMemcpyDeviceToHost, st));
     }
     ORI_TRY(check_launch("operator epilogue"));
@@ -752,16 +740,25 @@ int ori_ctx_stats(ori_ctx_t* ctx, unsigned long long* calls, unsigned long long*
     return ORI_OK;
 }
 
+// The operator entry points check their arguments before any device work, so a bad *_host call creates no default
+// context; the *_host forms are the *_ctx ones on the process-wide default context.
+static int zigap_args(const float* DZ_hat_i, const float* DZ_hat_j, const float* log_U_hat, const float* log_V_hat,
+                      const float* D_hat, const float* X, int64_t n, int64_t p, int64_t K, int quirk) {
+    if (!D_hat) return set_error(ORI_EINVAL, "D_hat is NULL");
+    return z_operator_args(DZ_hat_i, DZ_hat_j, log_U_hat, log_V_hat, D_hat, X, n, p, K, quirk);
+}
+
 int ori_zigap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* DZ_hat_i, float* DZ_hat_j, float* DZ_exp_logsum_hat,
                                            const float* log_U_hat, const float* log_V_hat,
                                            const float* D_hat, const float* X,
                                            int64_t n, int64_t p, int64_t K, int quirk) {
-    if (!D_hat) return set_error(ORI_EINVAL, "D_hat is NULL");
+    ORI_TRY(zigap_args(DZ_hat_i, DZ_hat_j, log_U_hat, log_V_hat, D_hat, X, n, p, K, quirk));
     return z_operator_ctx(ctx, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, nullptr, nullptr, D_hat, X, n, p, K, quirk);
 }
 
 int ori_gap_compute_Z_q_expectations_ctx(ori_ctx_t* ctx, float* Z_hat_i, float* Z_hat_j, const float* log_U_hat,
                                          const float* log_V_hat, const float* X, int64_t n, int64_t p, int64_t K) {
+    ORI_TRY(z_operator_args(Z_hat_i, Z_hat_j, log_U_hat, log_V_hat, nullptr, X, n, p, K, 0));
     return z_operator_ctx(ctx, Z_hat_i, Z_hat_j, nullptr, log_U_hat, log_V_hat, nullptr, nullptr, nullptr, X, n, p, K, 0);
 }
 
@@ -769,23 +766,22 @@ int ori_zigap_compute_Z_q_expectations_host(float* DZ_hat_i, float* DZ_hat_j, fl
                                             const float* log_U_hat, const float* log_V_hat,
                                             const float* D_hat, const float* X,
                                             int64_t n, int64_t p, int64_t K, int quirk) {
-    if (!D_hat) return set_error(ORI_EINVAL, "D_hat is NULL");
+    ORI_TRY(zigap_args(DZ_hat_i, DZ_hat_j, log_U_hat, log_V_hat, D_hat, X, n, p, K, quirk));
     int rc;
     ori_ctx* c = default_ctx(&rc);
-    if (!c) return rc;
-    return z_operator_ctx(c, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, nullptr, nullptr, D_hat, X, n, p, K, quirk);
+    return c ? ori_zigap_compute_Z_q_expectations_ctx(c, DZ_hat_i, DZ_hat_j, DZ_exp_logsum_hat, log_U_hat, log_V_hat, D_hat,
+                                                      X, n, p, K, quirk) : rc;
 }
 
 int ori_gap_compute_Z_q_expectations_host(float* Z_hat_i, float* Z_hat_j, const float* log_U_hat,
                                           const float* log_V_hat, const float* X, int64_t n, int64_t p, int64_t K) {
+    ORI_TRY(z_operator_args(Z_hat_i, Z_hat_j, log_U_hat, log_V_hat, nullptr, X, n, p, K, 0));
     int rc;
     ori_ctx* c = default_ctx(&rc);
-    if (!c) return rc;
-    return z_operator_ctx(c, Z_hat_i, Z_hat_j, nullptr, log_U_hat, log_V_hat, nullptr, nullptr, nullptr, X, n, p, K, 0);
+    return c ? ori_gap_compute_Z_q_expectations_ctx(c, Z_hat_i, Z_hat_j, log_U_hat, log_V_hat, X, n, p, K) : rc;
 }
 
-// sparse_zigap.py:100-116: D_hat, S_tilde, S_hat and the third output (read by the S-step, :155) are required; checked
-// with the shape before any device work
+// sparse_zigap.py:100-116: D_hat, S_tilde, S_hat and the third output (read by the S-step, :155) are required
 static int sparse_args(const float* DSZ_hat, const float* DZ_hat, const float* DZ_exp_logsum_hat, const float* log_U_hat,
                        const float* log_V_hat, const float* S_tilde, const float* S_hat, const float* D_hat, const float* X,
                        int64_t n, int64_t p, int64_t K) {
@@ -810,8 +806,8 @@ int ori_sparse_zigap_compute_Z_q_expectations_host(float* DSZ_hat, float* DZ_hat
     ORI_TRY(sparse_args(DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat, S_tilde, S_hat, D_hat, X, n, p, K));
     int rc;
     ori_ctx* c = default_ctx(&rc);
-    if (!c) return rc;
-    return z_operator_ctx(c, DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat, S_tilde, S_hat, D_hat, X, n, p, K, 0);
+    return c ? ori_sparse_zigap_compute_Z_q_expectations_ctx(c, DSZ_hat, DZ_hat, DZ_exp_logsum_hat, log_U_hat, log_V_hat,
+                                                             S_tilde, S_hat, D_hat, X, n, p, K) : rc;
 }
 
 }  // extern "C"

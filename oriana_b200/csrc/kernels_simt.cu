@@ -222,9 +222,10 @@ k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
 constexpr int PG_TG = 128;
 constexpr int PG_TR = 32;
 
-// SPARSE: eV = the masked denominator operand, Vh = the previous effective V_hat (see k_pass_rows), and a third
-// sum Zl[j,k] = sum_i R_ij eU_ik E[log U_ik] (sparse_zigap.py:116) with the sweep operand eUl = eU * E[log U].
-template <int KP, bool DROPOUT, bool QUIRK, bool SPARSE>
+// THIRD: a third sum Zl[j,k] = sum_i R_ij eU_ik E[log U_ik] (zigap.py:95, sparse_zigap.py:116) with the sweep operand
+// eUl = eU * E[log U].  The sparse model passes eV = its masked denominator operand and Vh = the previous effective
+// V_hat (see k_pass_rows).
+template <int KP, bool DROPOUT, bool QUIRK, bool THIRD>
 __global__ void __launch_bounds__(PG_TG)
 k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
              const float* __restrict__ eU, const float* __restrict__ eUw, const float* __restrict__ Uh,
@@ -238,7 +239,7 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
     // det_z (ORI_F_DETERMINISTIC): the sums of row chunk blockIdx.y are stored to det_z[blockIdx.y][Zj | b2s | Zl][p x KP]
     // instead of added atomically; k_det_sum_chunks adds the chunks in index order
     __shared__ float sthr[PG_TR];
-    __shared__ __align__(16) float sUl[SPARSE ? PG_TR : 1][KP];
+    __shared__ __align__(16) float sUl[THIRD ? PG_TR : 1][KP];
     __shared__ __align__(16) float sU[PG_TR][KP];
     __shared__ __align__(16) float sUw[QUIRK ? PG_TR : 1][KP];
     __shared__ __align__(16) float sUh[DROPOUT ? PG_TR : 1][KP];
@@ -250,12 +251,12 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
     const long long r_begin = (long long)blockIdx.y * rows_per_chunk;
     const long long r_end = min(n_rows, r_begin + rows_per_chunk);
 
-    float ev[KP], vh[DROPOUT ? KP : 1], zj[KP], bs[DROPOUT ? KP : 1], zl[SPARSE ? KP : 1];
+    float ev[KP], vh[DROPOUT ? KP : 1], zj[KP], bs[DROPOUT ? KP : 1], zl[THIRD ? KP : 1];
 #pragma unroll
     for (int k = 0; k < KP; ++k) {
         ev[k] = j_ok ? eV[(long long)j * KP + k] : 0.f;
         zj[k] = 0.f;
-        if (SPARSE) zl[k] = 0.f;
+        if (THIRD) zl[k] = 0.f;
         if (DROPOUT) { vh[k] = j_ok ? Vh[(long long)j * KP + k] : 0.f; bs[k] = 0.f; }
     }
     const float lpj = (DROPOUT && j_ok) ? lp[j] : 0.f;
@@ -272,7 +273,7 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
             const bool ok = idx / KP < rcount;
             sUf[idx] = ok ? eU[r0 * KP + idx] : 0.f;
             if (QUIRK) sUwf[idx] = ok ? eUw[r0 * KP + idx] : 0.f;
-            if (SPARSE) sUlf[idx] = ok ? eUl[r0 * KP + idx] : 0.f;
+            if (THIRD) sUlf[idx] = ok ? eUl[r0 * KP + idx] : 0.f;
             if (DROPOUT) {
                 sUhf[idx] = ok ? Uh[r0 * KP + idx] : 0.f;
                 sUnf[idx] = ok ? Un[r0 * KP + idx] : 0.f;
@@ -294,7 +295,7 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
                 const float4* w4 = reinterpret_cast<const float4*>(&sUw[QUIRK ? rr : 0][0]);
                 const float4* h4 = reinterpret_cast<const float4*>(&sUh[DROPOUT ? rr : 0][0]);
                 const float4* n4 = reinterpret_cast<const float4*>(&sUn[DROPOUT ? rr : 0][0]);
-                const float4* l4 = reinterpret_cast<const float4*>(&sUl[SPARSE ? rr : 0][0]);
+                const float4* l4 = reinterpret_cast<const float4*>(&sUl[THIRD ? rr : 0][0]);
 #pragma unroll
                 for (int q = 0; q < KP / 4; ++q) {
                     const float4 uu = u4[q];
@@ -318,7 +319,7 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
                     for (int k = 0; k < KP; ++k)
                         if (sU[rr][k] * ev[k] > T) {
                             zj[k] = fmaf(r2, QUIRK ? sUw[QUIRK ? rr : 0][k] : sU[rr][k], zj[k]);
-                            if (SPARSE) zl[k] = fmaf(r2, sUl[SPARSE ? rr : 0][k], zl[k]);
+                            if (THIRD) zl[k] = fmaf(r2, sUl[THIRD ? rr : 0][k], zl[k]);
                         }
                     R = 0.f;
                 }
@@ -338,7 +339,7 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
                         bs[4 * q + 0] = fmaf(D, nn.x, bs[4 * q + 0]); bs[4 * q + 1] = fmaf(D, nn.y, bs[4 * q + 1]);
                         bs[4 * q + 2] = fmaf(D, nn.z, bs[4 * q + 2]); bs[4 * q + 3] = fmaf(D, nn.w, bs[4 * q + 3]);
                     }
-                    if (SPARSE) {
+                    if (THIRD) {
                         const float4 ll = l4[q];
                         zl[4 * q + 0] = fmaf(R, ll.x, zl[4 * q + 0]); zl[4 * q + 1] = fmaf(R, ll.y, zl[4 * q + 1]);
                         zl[4 * q + 2] = fmaf(R, ll.z, zl[4 * q + 2]); zl[4 * q + 3] = fmaf(R, ll.w, zl[4 * q + 3]);
@@ -354,14 +355,14 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
         for (int k = 0; k < KP; ++k) {
             base[k] = zj[k];
             if (DROPOUT) base[pk + k] = bs[k];
-            if (SPARSE) base[2 * pk + k] = zl[k];
+            if (THIRD) base[2 * pk + k] = zl[k];
         }
     } else if (j_ok) {
 #pragma unroll
         for (int k = 0; k < KP; ++k) {
             atomicAdd(Zj + (long long)j * KP + k, zj[k]);
             if (DROPOUT) atomicAdd(b2s + (long long)j * KP + k, bs[k]);
-            if (SPARSE) atomicAdd(Zl + (long long)j * KP + k, zl[k]);
+            if (THIRD) atomicAdd(Zl + (long long)j * KP + k, zl[k]);
         }
     }
 }
@@ -1024,7 +1025,8 @@ template <int KP>
 static int pass_rows_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     const int bx = cdiv(P->n_rows, PR_TR);
     constexpr int TGS = KP <= 32 ? PR_TG : 16;         // tile width of the sparse variant
-    const int ntiles = cdiv(P->p, (P->flags & ORI_F_SPARSE) ? TGS : PR_TG);
+    const bool sparse = P->flags & ORI_F_SPARSE;
+    const int ntiles = cdiv(P->p, sparse ? TGS : PR_TG);
     int gy = 1;  // split the gene sweep until there are several waves of CTAs (3 resident per SM): a 1.8-wave grid idles
     while (bx * gy < 148 * 3 * 6 && gy * 2 <= ntiles) gy *= 2;   // most of the machine during its last wave
     const bool drop = P->flags & ORI_F_DROPOUT, elbo = P->flags & ORI_F_ELBO;
@@ -1046,27 +1048,22 @@ static int pass_rows_kp(const ori_problem_t* P, int g, cudaStream_t st) {
         return nk ? check_launch("k_det_sum_cols", nk) : ORI_OK;
     };
     dim3 grid(bx, gy);
-    if (P->flags & ORI_F_SPARSE) {      // without ORI_F_DROPOUT: the operator seam (api.cu), D_hat folded into X
-#define ORI_LAUNCH_PRS(D)                                                                                       \
-        k_pass_rows<KP, D, false, true, TGS><<<grid, PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->eU[g],    \
-            P->U_hat[g], P->eVd, P->Vh_old, P->eVz, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part,     \
-            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,    \
-            det_cs, det_part)
-        if (drop) ORI_LAUNCH_PRS(true);
-        else ORI_LAUNCH_PRS(false);
-#undef ORI_LAUNCH_PRS
-        if (check_launch("k_pass_rows(sparse)") != ORI_OK) return ORI_ECUDA;
-        return det_sums();
-    }
-#define ORI_LAUNCH_PR(D, E)                                                                              \
-    k_pass_rows<KP, D, E, false><<<grid, PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->eU[g], P->U_hat[g], \
-                                                  P->eV, P->V_hat, P->eV, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part, \
-                                                  (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, \
-                                                  P->thrU ? P->thrV : nullptr, det_cs, det_part)
-    if (drop && elbo) ORI_LAUNCH_PR(true, true);
-    else if (drop) ORI_LAUNCH_PR(true, false);
-    else if (elbo) ORI_LAUNCH_PR(false, true);
-    else ORI_LAUNCH_PR(false, false);
+    // sparse model (without ORI_F_DROPOUT: the operator seam, api.cu, D_hat folded into X): the masked operands of
+    // k_pass_rows; ORI_F_SPARSE excludes ORI_F_ELBO
+    const float* eV = sparse ? P->eVd : P->eV;
+    const float* Vh = sparse ? P->Vh_old : P->V_hat;
+    const float* eVz = sparse ? P->eVz : P->eV;
+#define ORI_LAUNCH_PR(D, E, S)                                                                                  \
+    k_pass_rows<KP, D, E, S, S ? TGS : PR_TG><<<grid, PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->eU[g],   \
+        P->U_hat[g], eV, Vh, eVz, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part,                       \
+        (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,        \
+        det_cs, det_part)
+    if (sparse && drop) ORI_LAUNCH_PR(true, false, true);
+    else if (sparse) ORI_LAUNCH_PR(false, false, true);
+    else if (drop && elbo) ORI_LAUNCH_PR(true, true, false);
+    else if (drop) ORI_LAUNCH_PR(true, false, false);
+    else if (elbo) ORI_LAUNCH_PR(false, true, false);
+    else ORI_LAUNCH_PR(false, false, false);
 #undef ORI_LAUNCH_PR
     if (check_launch("k_pass_rows") != ORI_OK) return ORI_ECUDA;
     return det_sums();
@@ -1090,10 +1087,10 @@ static int pass_genes_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     long long rpc = (P->n_rows + chunks - 1) / chunks;
     rpc = (rpc + PG_TR - 1) / PG_TR * PG_TR;
     if (rpc > 8192) rpc = 8192;  // bound the fp32 running sums
-    const bool sparse_ = (P->flags & ORI_F_SPARSE) != 0;
+    const bool third = P->eUl[g] != nullptr;      // the third sum Zl into red32 block 2
     // ORI_F_DETERMINISTIC: nominal chunks only (their number bounds the scratch), every chunk stores to its own slot
     float* det_z = nullptr;
-    const long long det_stride = (long long)(sparse_ ? 3 : 2) * P->p * P->KP;
+    const long long det_stride = (long long)(third ? 3 : 2) * P->p * P->KP;
     if ((P->flags & ORI_F_DETERMINISTIC) && P->det_ws) {
         if (!det_simt_ok(P->n_rows, P->p)) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC on the CUDA-core kernels: problem too large");
         rpc = 8192;
@@ -1112,29 +1109,22 @@ static int pass_genes_kp(const ori_problem_t* P, int g, cudaStream_t st) {
         k_det_sum_chunks_strided<<<cdiv(total, 256), 256, 0, st>>>(P->red32, det_z, gy, total, det_stride);
         return check_launch("k_det_sum_chunks");
     };
-    if (P->flags & ORI_F_SPARSE) {      // without ORI_F_DROPOUT: the operator seam (api.cu), D_hat folded into X
-#define ORI_LAUNCH_PGS(D)                                                                                       \
-        k_pass_genes<KP, D, false, true><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc,        \
-            P->eU[g], nullptr, P->U_hat[g], P->U_hat[1 - g], P->eUl[g], P->eVd, P->Vh_old, P->lp, P->pfloor,    \
-            Zj, b2s, P->red32 + 2ll * P->p * P->KP,                                                              \
-            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,    \
-            det_z, det_stride)
-        if (drop) ORI_LAUNCH_PGS(true);
-        else ORI_LAUNCH_PGS(false);
-#undef ORI_LAUNCH_PGS
-        if (check_launch("k_pass_genes(sparse)") != ORI_OK) return ORI_ECUDA;
-        return det_sums();
-    }
-#define ORI_LAUNCH_PG(D, Q)                                                                             \
-    k_pass_genes<KP, D, Q, false><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, P->eU[g], \
-                                                   P->eUw, P->U_hat[g], P->U_hat[1 - g], nullptr, P->eV, P->V_hat, \
-                                                   P->lp, P->pfloor, Zj, b2s, nullptr, \
-                                                   (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, \
-                                                   P->thrU ? P->thrV : nullptr, det_z, det_stride)
-    if (drop && quirk) ORI_LAUNCH_PG(true, true);
-    else if (drop) ORI_LAUNCH_PG(true, false);
-    else if (quirk) ORI_LAUNCH_PG(false, true);
-    else ORI_LAUNCH_PG(false, false);
+    // sparse model (without ORI_F_DROPOUT: the operator seam, api.cu, D_hat folded into X): the masked denominator
+    // operand and the previous effective V_hat; the quirk weight and the third sum are never asked for together
+    const bool sparse = P->flags & ORI_F_SPARSE;
+    const float* eV = sparse ? P->eVd : P->eV;
+    const float* Vh = sparse ? P->Vh_old : P->V_hat;
+#define ORI_LAUNCH_PG(D, Q, T)                                                                                  \
+    k_pass_genes<KP, D, Q, T><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, P->eU[g], P->eUw, \
+        P->U_hat[g], P->U_hat[1 - g], P->eUl[g], eV, Vh, P->lp, P->pfloor, Zj, b2s, P->red32 + 2ll * P->p * P->KP, \
+        (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,        \
+        det_z, det_stride)
+    if (third && drop) ORI_LAUNCH_PG(true, false, true);
+    else if (third) ORI_LAUNCH_PG(false, false, true);
+    else if (drop && quirk) ORI_LAUNCH_PG(true, true, false);
+    else if (drop) ORI_LAUNCH_PG(true, false, false);
+    else if (quirk) ORI_LAUNCH_PG(false, true, false);
+    else ORI_LAUNCH_PG(false, false, false);
 #undef ORI_LAUNCH_PG
     if (check_launch("k_pass_genes") != ORI_OK) return ORI_ECUDA;
     return det_sums();

@@ -108,6 +108,13 @@ def test_bad_arguments_raise(cuda_lib):
     with pytest.raises(_lib.OrianaB200Error):   # quirk needs p >= K
         z_op(cuda_lib, np.zeros((2, 5), np.float32), np.zeros((3, 5), np.float32), np.zeros((2, 3), np.float32),
              np.ones((2, 3), np.float32), quirk=True)
+    # the third gene sum (eUl) belongs to the sparse model: a ZIGaP problem that asks for it is refused
+    from oriana.models import ZIGaP
+    P = _lib.OriProblem.from_buffer_copy(ZIGaP(np.ones((4, 6)), k=2, use_factors=False)._P)
+    _lib.check(cuda_lib.ori_problem_check(ctypes.byref(P)))
+    P.eUl[0] = P.eU[0]
+    with pytest.raises(_lib.OrianaB200Error):
+        _lib.check(cuda_lib.ori_problem_check(ctypes.byref(P)))
 
 
 def _stats(lib, ctx=None):
@@ -118,13 +125,15 @@ def _stats(lib, ctx=None):
 
 
 @pytest.mark.parametrize('quirk', [True, False])
-def test_tensor_sized_slabs_take_the_tcgen05_passes(cuda_lib, quirk):
+@pytest.mark.parametrize('K', [10, 40])
+def test_tensor_sized_slabs_take_the_tcgen05_passes(cuda_lib, K, quirk):
     """Slabs of >= 2^21 entries go through the tcgen05 / TMA kernels (TF32 operands: 1e-3 against the sequential float32
     loop of the reference, restated in C), through an explicit context with three ragged slabs; a second call of the
-    same shape allocates nothing and gives the same answer up to the order of the float atomics."""
+    same shape allocates nothing and gives the same answer up to the order of the float atomics.  K = 10 runs the
+    KP = 32 plan, K = 40 the KP = 64 one."""
     from oracle import zloop
     from oriana_b200 import _lib
-    n, p, K = 2900, 1500, 10
+    n, p = 2900, 1500
     rng = np.random.default_rng(5)
     lU = rng.normal(-0.5, 1.0, (n, K)).astype(np.float32)
     lV = rng.normal(-0.5, 1.0, (p, K)).astype(np.float32)
