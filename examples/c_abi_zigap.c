@@ -58,13 +58,13 @@ int main(int argc, char** argv) {
     for (int g = 0; g < 2; ++g) { P.U_hat[g] = (float*)dalloc(rowf); P.eU[g] = (float*)dalloc(rowf); }
     P.Zi = (float*)dalloc(rowf); P.a2s = (float*)dalloc(rowf);
     P.b1 = (float*)dalloc(genef); P.b2 = (float*)dalloc(genef); P.V_hat = (float*)dalloc(genef); P.eV = (float*)dalloc(genef);
-    P.red32 = (float*)dalloc(2 * genef);
+    P.red32 = (float*)dalloc(sizeof(float) * (size_t)ORI_RED32_FLOATS(p, KP, 0));
     P.lp = (float*)dalloc(sizeof(float) * p); P.pfloor = (float*)dalloc(sizeof(float) * p);
     P.hyper = (double*)dalloc(sizeof(double) * 4 * K);
-    P.red64 = (double*)dalloc(sizeof(double) * (p + 2 * KP + 8));
-    P.gsum = (double*)dalloc(sizeof(double) * (2 * KP + 8));
+    P.red64 = (double*)dalloc(sizeof(double) * (size_t)ORI_RED64_DOUBLES(p, KP));
+    P.gsum = (double*)dalloc(sizeof(double) * ORI_GSUM_DOUBLES(KP));
     P.pi_d = (double*)dalloc(sizeof(double) * p);
-    P.scal = (double*)dalloc(sizeof(double) * 16);
+    P.scal = (double*)dalloc(sizeof(double) * ORI_SC_NSLOTS);
     P.elbo_trace = (double*)dalloc(sizeof(double) * P.trace_cap);
     P.tc_ws_floats = ori_tc_workspace_floats(n, p, KP) + 32;
     P.tc_ws = (float*)dalloc(sizeof(float) * (size_t)P.tc_ws_floats);

@@ -43,8 +43,8 @@ extern "C" {
 #define ORI_F_NO_TENSOR 8u    /* force the CUDA-core kernels (tests); default picks tcgen05 when it can   */
 #define ORI_F_SPARSE 16u      /* SparseZIGaP: spike-and-slab layer S on V (sparse_zigap.py:100-204); needs
                                  ORI_F_DROPOUT, the `sparse` block below, K <= 64 (tensor kernels: K <= 32), no ELBO */
-#define ORI_F_DEVICE_ITER 32u /* the iteration count (index into elbo_trace) is read from scal[5] on the device
-                                 instead of ori_problem_t::iter, so that one captured CUDA graph of a whole
+#define ORI_F_DEVICE_ITER 32u /* the iteration count (index into elbo_trace) is read from scal[ORI_SC_ITER] on the
+                                 device instead of ori_problem_t::iter, so that one captured CUDA graph of a whole
                                  step can be replayed for every iteration                                   */
 
 #define ORI_F_PRECISE 64u     /* tensor path only (K <= 32): the accumulating contractions R.eV, D.V_hat and their transposes
@@ -68,6 +68,37 @@ extern "C" {
 #define ORI_M_INIT_KEEP 2     /* same but keep the caller's alpha/beta (state copied from a model)        */
 #define ORI_M_FINALIZE 3      /* flush: pi(t) and ELBO(t) of the CURRENT state, nothing else changes      */
 #define ORI_M_REFRESH 4       /* after ori_init_expectations on edited (a,b): only the pending ELBO terms  */
+
+/* Layout of the reduction buffers of ori_problem_t (the caller allocates them at these sizes):
+ *   red32 = [Zj | b2s | Zl]               float32, blocks of p x KP; the block Zl only with eUl (ORI_F_SPARSE)
+ *   red64 = [colsum D_hat (p) | sum_i log U_hat (KP) | sum_i U_hat (KP) | ELBO partials (ORI_R64_NSLOTS)]
+ *   gsum  = [sum_j log V_hat (KP) | sum_j V_hat (KP) | gene partials (ORI_GSUM_NSLOTS)]
+ *   scal  = ORI_SC_NSLOTS per-model scalars                                                                 */
+#define ORI_RED32_FLOATS(p, KP, third) (((third) ? 3 : 2) * (int64_t)(p) * (KP))
+#define ORI_RED64_DOUBLES(p, KP) ((int64_t)(p) + 2 * (KP) + ORI_R64_NSLOTS)
+#define ORI_GSUM_DOUBLES(KP) (2 * (KP) + ORI_GSUM_NSLOTS)
+
+/* slots of the ELBO partials of red64 (summed over ranks with it) */
+#define ORI_R64_XLOGDEN 0     /* sum_{X>0} X log den                                                      */
+#define ORI_R64_ENT 1         /* sum_{X==0} entropy of q(D_ij)                                            */
+#define ORI_R64_PUV 2         /* sum_ij D_hat_ij (U_hat V_hat^T)_ij                                       */
+#define ORI_R64_HROW 3        /* sum_ik entropy of q(U_ik)                                                */
+#define ORI_R64_LGAMX 4       /* sum_{X>0} lgamma(X+1)   (ori_count_stats)                                */
+#define ORI_R64_NNZ 5         /* number of non-zero entries   (ori_count_stats)                           */
+#define ORI_R64_NSLOTS 8
+
+/* slots of the gene partials of gsum */
+#define ORI_GSUM_HGENE 0      /* sum_jk entropy of q(V_jk)                                                */
+#define ORI_GSUM_NSLOTS 8
+
+/* slots of scal (float64 scalars that persist between calls); slot 3 and slots 7.. are unused */
+#define ORI_SC_LGAMX 0        /* sum_{X>0} lgamma(X+1)         (constant, all ranks)                      */
+#define ORI_SC_NNZ 1          /* number of non-zero entries    (constant, all ranks)                      */
+#define ORI_SC_PENDING 2      /* K-, p- and nK-sized ELBO terms of the current state, entropies included  */
+#define ORI_SC_ELBO_LAST 4    /* last finalised ELBO                                                      */
+#define ORI_SC_ITER 5         /* completed iterations (read by ORI_F_DEVICE_ITER)                         */
+#define ORI_SC_UVSUM 6        /* sum_k (sum_i U_hat_ik)(sum_j V_hat_jk) of the current state (GaP's ELBO)  */
+#define ORI_SC_NSLOTS 16
 
 /* One rank's view of the problem.  Factor arrays are row-major with row stride KP (K padded to a
  * multiple of 8, pad columns hold zeros).  "gen" arrays are ping-pong generations of the row factors:
@@ -99,19 +130,18 @@ typedef struct ori_problem {
     float* b2;             /* zigap.py:124 */
     float* V_hat;
     float* eV;
-    float* red32;          /* [2 x p x KP]: Zj partial | b2s partial -- allreduce(sum) buffer #1; [3 x p x KP]
-                              with eUl (ORI_F_SPARSE) */
+    float* red32;          /* [ORI_RED32_FLOATS(p, KP, eUl != NULL)] Zj | b2s (| Zl) -- allreduce(sum) buffer #1 */
 
     float* lp;             /* [p] logit(pi) generating the CURRENT D_hat; -inf: D_hat=(X>0) (zigap.py:77) */
     float* pfloor;         /* [p] 1e-10 where pi<=0 (zigap.py:133), else 0               */
 
     /* float64 small state */
     double* hyper;         /* [4 x K] alpha1 | alpha2 | beta1 | beta2                    */
-    double* red64;         /* [p + 2KP + 8] colsum D_hat | sum_i log U_hat | sum_i U_hat | ELBO partials
-                              -- allreduce(sum) buffer #2                                 */
-    double* gsum;          /* [2KP + 8] sum_j log V_hat | sum_j V_hat | entropy           */
+    double* red64;         /* [ORI_RED64_DOUBLES(p, KP)] colsum D_hat | sum_i log U_hat | sum_i U_hat |
+                              ORI_R64_* partials -- allreduce(sum) buffer #2              */
+    double* gsum;          /* [ORI_GSUM_DOUBLES(KP)] sum_j log V_hat | sum_j V_hat | ORI_GSUM_* partials */
     double* pi_d;          /* [p] Bernoulli prior pi(t)  zigap.py:158                    */
-    double* scal;          /* [16] see ScalSlot in csrc/common.cuh                       */
+    double* scal;          /* [ORI_SC_NSLOTS] the ORI_SC_* scalars                       */
     double* elbo_trace;    /* [trace_cap]                                                */
 
     /* tensor path (tcgen05/TMA kernels, csrc/kernels_tc.cu): caller-owned scratch of at least
@@ -121,8 +151,8 @@ typedef struct ori_problem {
     int64_t tc_ws_floats;
 
     /* SparseZIGaP (ORI_F_SPARSE).  With this flag b1, b2 parametrise V' (sparse_zigap.py:24-28), eV holds
-     * exp(E[log V']) without the mask, V_hat holds the EFFECTIVE factor S_hat * V'_hat (:140) and red32 is
-     * [3 x p x KP]: Zj | b2s | Zl, the third block being sum_i R_ij eU_ik E[log U_ik] (:116).
+     * exp(E[log V']) without the mask, V_hat holds the EFFECTIVE factor S_hat * V'_hat (:140) and red32
+     * has its third block, Zl = sum_i R_ij eU_ik E[log U_ik] (:116).
      * Gene-side arrays are [p x KP] float32. */
     float* p_s;            /* Bernoulli parameter of q(S) = S_hat (float32(p_s), bernoulli.py:45)          */
     float* logV;           /* E[log V'] (read by :116 and :157)                                            */
@@ -184,7 +214,8 @@ int64_t ori_det_workspace_doubles(int64_t n_rows, int32_t p, int32_t KP);
 int ori_uses_tensor_path(const ori_problem_t* P);
 /* Validate a problem description (shapes, alignment, null pointers). */
 int ori_problem_check(const ori_problem_t* P);
-/* Constant data statistics: sum lgamma(X+1), nnz -> scal; column sums of (X>0) -> red64[0..p). */
+/* Constant data statistics: sum lgamma(X+1), nnz -> red64 slots ORI_R64_LGAMX, ORI_R64_NNZ (ori_mstep ORI_M_INIT and
+ * ORI_M_INIT_KEEP copy them to scal); column sums of (X>0) -> red64[0..p). */
 int ori_count_stats(const ori_problem_t* P, void* stream);
 /* Expectations of generation `gen` from (a1,a2,b1,b2) (zigap.py:160-165) + their column sums. */
 int ori_init_expectations(const ori_problem_t* P, int gen, void* stream);

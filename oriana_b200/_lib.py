@@ -13,8 +13,24 @@ ORI_F_DROPOUT, ORI_F_QUIRK, ORI_F_ELBO, ORI_F_NO_TENSOR, ORI_F_SPARSE, ORI_F_DEV
 ORI_F_FIXED_CHAIN = 128
 ORI_F_DETERMINISTIC = 256
 ORI_M_STEP, ORI_M_INIT, ORI_M_INIT_KEEP, ORI_M_FINALIZE, ORI_M_REFRESH = 0, 1, 2, 3, 4
-R64_NSLOTS = 8
-SCAL_SLOTS = 16
+
+# layout of the reduction buffers of `ori_problem_t` (the ORI_R64_* / ORI_GSUM_* / ORI_SC_* slots and size macros)
+ORI_R64_XLOGDEN, ORI_R64_ENT, ORI_R64_PUV, ORI_R64_HROW, ORI_R64_LGAMX, ORI_R64_NNZ, ORI_R64_NSLOTS = 0, 1, 2, 3, 4, 5, 8
+ORI_GSUM_HGENE, ORI_GSUM_NSLOTS = 0, 8
+ORI_SC_LGAMX, ORI_SC_NNZ, ORI_SC_PENDING, ORI_SC_ELBO_LAST, ORI_SC_ITER, ORI_SC_UVSUM, ORI_SC_NSLOTS = 0, 1, 2, 4, 5, 6, 16
+
+
+def ORI_RED32_FLOATS(p, KP, third):
+    return (3 if third else 2) * p * KP
+
+
+def ORI_RED64_DOUBLES(p, KP):
+    return p + 2 * KP + ORI_R64_NSLOTS
+
+
+def ORI_GSUM_DOUBLES(KP):
+    return 2 * KP + ORI_GSUM_NSLOTS
+
 
 _fp = C.POINTER(C.c_float)
 _dp = C.POINTER(C.c_double)

@@ -173,7 +173,7 @@ int ori_problem_check(const ori_problem_t* P) {
     if (P->flags & ORI_F_DETERMINISTIC) {
         if (!P->tc_ws && !det_simt_ok(P->n_rows, P->p))
             return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC on the CUDA-core kernels is limited to 2^26 matrix entries");
-        if (!P->det_ws || P->det_ws_doubles < det_workspace_doubles(P->n_rows, P->p, P->KP))
+        if (!P->det_ws || P->det_ws_doubles < det_carve(nullptr, P->n_rows, P->p).doubles)
             return set_error(ORI_EINVAL, "ORI_F_DETERMINISTIC needs det_ws of ori_det_workspace_doubles() doubles");
     }
     if (P->ldx < P->p || (P->ldx & 3)) return set_error(ORI_EINVAL, "ldx=%lld must be >= p and a multiple of 4", (long long)P->ldx);
@@ -204,8 +204,8 @@ int ori_problem_check(const ori_problem_t* P) {
     return ORI_OK;
 }
 
-static size_t red64_bytes(const ori_problem_t* P) { return sizeof(double) * (size_t)(P->p + 2 * P->KP + R64_NSLOTS); }
-static size_t gsum_bytes(const ori_problem_t* P) { return sizeof(double) * (size_t)(2 * P->KP + 8); }
+static size_t red64_bytes(const ori_problem_t* P) { return sizeof(double) * (size_t)ORI_RED64_DOUBLES(P->p, P->KP); }
+static size_t gsum_bytes(const ori_problem_t* P) { return sizeof(double) * (size_t)ORI_GSUM_DOUBLES(P->KP); }
 static size_t rowf_bytes(const ori_problem_t* P) { return sizeof(float) * (size_t)P->n_rows * P->KP; }
 
 int ori_count_stats(const ori_problem_t* P, void* stream) {
@@ -247,7 +247,7 @@ static int pass_genes_any(const ori_problem_t* P, int gen_old, cudaStream_t st) 
 }
 
 int64_t ori_tc_workspace_floats(int64_t n_rows, int32_t p, int32_t KP) { return tc_workspace_floats(n_rows, p, KP); }
-int64_t ori_det_workspace_doubles(int64_t n_rows, int32_t p, int32_t KP) { return det_workspace_doubles(n_rows, p, KP); }
+int64_t ori_det_workspace_doubles(int64_t n_rows, int32_t p, int32_t KP) { (void)KP; return det_carve(nullptr, n_rows, p).doubles; }
 
 int ori_uses_tensor_path(const ori_problem_t* P) { return (P && tc_eligible(P)) ? 1 : 0; }
 
@@ -287,7 +287,7 @@ static int zero_accumulators(const ori_problem_t* P, cudaStream_t st, bool genes
         ORI_CUDA(cudaMemsetAsync(P->Zi, 0, rowf_bytes(P), st));
         if (P->flags & ORI_F_DROPOUT) ORI_CUDA(cudaMemsetAsync(P->a2s, 0, rowf_bytes(P), st));
     }
-    if (genes) ORI_CUDA(cudaMemsetAsync(P->red32, 0, sizeof(float) * (P->eUl[0] ? 3 : 2) * (size_t)P->p * P->KP, st));
+    if (genes) ORI_CUDA(cudaMemsetAsync(P->red32, 0, sizeof(float) * (size_t)ORI_RED32_FLOATS(P->p, P->KP, P->eUl[0] != nullptr), st));
     ORI_CUDA(cudaMemsetAsync(P->red64, 0, red64_bytes(P), st));
     return ORI_OK;
 }
@@ -565,8 +565,8 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     // into ZJ3 = [plain gene sums | (unused) | Zl]; otherwise it comes out of the Zj sweep, into ZJ's third block
     const bool qw = D && quirk;
     const bool sweep3 = Z3_out && qw;
-    const size_t gblk = sizeof(float) * p * KP;
-    const size_t zj_bytes = (Z3_out && !sweep3 ? 3 : 2) * gblk;
+    const size_t zj_bytes = sizeof(float) * ORI_RED32_FLOATS(p, KP, Z3_out && !sweep3);
+    const size_t zj3_bytes = sizeof(float) * ORI_RED32_FLOATS(p, KP, 1);
 
     typedef ori_ctx B;
     for (int b = 0; b < nbuf; ++b) {
@@ -584,13 +584,13 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     ORI_TRY(C->need(B::LVRAW, sizeof(float) * p * K));
     ORI_TRY(C->need(B::EV, sizeof(float) * p * KP));
     ORI_TRY(C->need(B::ZJ, zj_bytes));
-    if (sweep3) ORI_TRY(C->need(B::ZJ3, 3 * gblk));
+    if (sweep3) ORI_TRY(C->need(B::ZJ3, zj3_bytes));
     if (sparse) {
         ORI_TRY(C->need(B::EVZ, sizeof(float) * p * KP));
         ORI_TRY(C->need(B::SRAW, sizeof(float) * 2 * p * K));
     }
     ORI_TRY(C->need(B::OUTJ, sizeof(float) * p * K));
-    ORI_TRY(C->need(B::D64, sizeof(double) * (p + 2 * KP + R64_NSLOTS)));
+    ORI_TRY(C->need(B::D64, sizeof(double) * ORI_RED64_DOUBLES(p, KP)));
     ORI_TRY(C->need(B::THRV, sizeof(float) * p));
 
     float* dlogVraw = C->as<float>(B::LVRAW);
@@ -614,7 +614,7 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     }
     ORI_TRY(check_launch("k_exp_pad"));
     ORI_CUDA(cudaMemsetAsync(dZj, 0, zj_bytes, st));
-    if (sweep3) ORI_CUDA(cudaMemsetAsync(dZ3, 0, 3 * gblk, st));
+    if (sweep3) ORI_CUDA(cudaMemsetAsync(dZ3, 0, zj3_bytes, st));
     // [0],[1]: last work on each stream; [2]: gene-side operands ready
     ORI_CUDA(cudaEventRecord(C->ev[2], st));
     ORI_CUDA(cudaStreamWaitEvent(st2, C->ev[2], 0));
@@ -686,7 +686,9 @@ static int z_operator_ctx(ori_ctx* C, float* Zi_out, float* Zj_out, float* Z3_ou
     k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(dZj, deV, nullptr, nullptr, dOutJ, p, (int)K, KP);
     ORI_CUDA(cudaMemcpyAsync(Zj_out, dOutJ, sizeof(float) * p * K, cudaMemcpyDeviceToHost, st));
     if (Z3_out) {   // eV * Zl + logV * (eV * plain gene sums)
-        k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(dZ3 + 2 * p * KP, deV, dZ3, dlogVraw, dOutJ, p, (int)K, KP);
+        P.red32 = dZ3;
+        const RedBufs z3 = red_carve(P);
+        k_scale_unpad<<<cdiv(p * K, 256), 256, 0, st>>>(z3.Zl, deV, z3.Zj, dlogVraw, dOutJ, p, (int)K, KP);
         ORI_CUDA(cudaMemcpyAsync(Z3_out, dOutJ, sizeof(float) * p * K, cudaMemcpyDeviceToHost, st));
     }
     ORI_TRY(check_launch("operator epilogue"));

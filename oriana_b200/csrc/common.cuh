@@ -10,24 +10,26 @@ namespace ori {
 int set_error(int code, const char* fmt, ...);
 int check_launch(const char* what, int n_kernels = 1);   // also counts the kernels launched (ori_kernel_launches)
 
-// slots of ori_problem_t::red64 after the p column sums and the 2K row-side sums
-enum Red64Slot {
-    R64_XLOGDEN = 0,  // sum_{X>0} X log den
-    R64_ENT = 1,      // sum_{X==0} entropy of q(D_ij)
-    R64_PUV = 2,      // sum_ij D_hat_ij (U_hat V_hat^T)_ij
-    R64_HROW = 3,     // sum_ik entropy of q(U_ik)
-    R64_NSLOTS = 8
+// The regions of the reduction buffers red32, red64 and gsum (layout: include/oriana_b200.h).  Zl exists only with eUl.
+struct RedBufs {
+    float *Zj, *b2s, *Zl;                   // red32
+    double *colsum, *SlogU, *SU, *part;     // red64; part: the ORI_R64_* slots
+    double *SlogV, *SV, *gpart;             // gsum; gpart: the ORI_GSUM_* slots
 };
-// slots of ori_problem_t::scal (per-model persistent scalars, float64)
-enum ScalSlot {
-    SC_LGAMX = 0,     // sum_{X>0} lgamma(X+1)      (constant, all ranks)
-    SC_NNZ = 1,       // number of non-zero entries (constant, all ranks)
-    SC_PENDING = 2,   // K-/p-/nK-sized ELBO terms of the current state
-    SC_HGENE = 3,     // sum_jk entropy of q(V_jk) of the current state
-    SC_ELBO_LAST = 4, // last finalised ELBO
-    SC_ITER = 5,      // number of completed iterations
-    SC_NSLOTS = 16
-};
+__host__ __device__ inline RedBufs red_carve(const ori_problem_t& P) {
+    RedBufs r;
+    r.Zj = P.red32;
+    r.b2s = P.red32 + (long long)P.p * P.KP;
+    r.Zl = P.red32 + 2ll * P.p * P.KP;
+    r.colsum = P.red64;
+    r.SlogU = P.red64 + P.p;
+    r.SU = P.red64 + P.p + P.KP;
+    r.part = P.red64 + P.p + 2 * P.KP;
+    r.SlogV = P.gsum;
+    r.SV = P.gsum + P.KP;
+    r.gpart = P.gsum + 2 * P.KP;
+    return r;
+}
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
@@ -49,20 +51,26 @@ int launch_deviance(const ori_problem_t* P, int gen, const double* pi, const dou
 // kernels_tc.cu
 long long tc_workspace_floats(long long n_rows, int p, int KP);
 
-// ORI_F_DETERMINISTIC scratch (ori_problem_t::det_ws), in doubles:
-//   [0, DET_FU_BLOCKS * DET_FU_SLOTS)   per-block partial sums of k_factor_update (sum log E | sum E | entropy | D.uv)
-//   [.., + pad128(p))                    column sums of D_hat of the second column slice of the tensor gene pass
-//   [.., + det_max_items * DET_ITEM_SLOTS)  per-item, per-CTA, per-warp ELBO terms of the tensor gene pass
-//   [.., + tickets)                      one int per own tile of the running tensor pass (chunk order of the accumulator adds)
-constexpr int DET_FU_BLOCKS = 148 * 8;
+// ORI_F_DETERMINISTIC scratch (ori_problem_t::det_ws): the regions det_carve places
+constexpr int DET_FU_BLOCKS = 148 * 8;             // the most blocks of k_factor_update / k_sparse_gene_update
 constexpr int DET_FU_SLOTS = 2 * 64 + 2;
 constexpr int DET_ITEM_SLOTS = 2 * 8 * 2;          // CTAs of a pair x element-wise warps x (x log den, entropy)
-//   CUDA-core kernels (problems up to DET_SIMT_MAX entries), from det_simt_offset():
-//   [nb x p] column sums per row block | [nb x 2] ELBO terms per row block | [chunks x 3 x p x KP] floats: gene sums per row chunk
+// CUDA-core kernels (problems up to DET_SIMT_MAX entries): row blocks of k_pass_rows, row chunks of k_pass_genes
 constexpr long long DET_SIMT_MAX = 1ll << 26;
-long long det_max_items(long long n_rows, int p);
-long long det_workspace_doubles(long long n_rows, int p, int KP);
-long long det_simt_offset(long long n_rows, int p);
+constexpr int DET_SIMT_BLOCK_ROWS = 128;
+constexpr int DET_SIMT_CHUNK_ROWS = 8192;
+struct DetWs {
+    double* fu_part;      // [DET_FU_BLOCKS x DET_FU_SLOTS] per-block sums of the factor updates (sum log E | sum E | entropy | D.uv)
+    double* colsum2;      // [p, padded to 128] column sums of D_hat of the second column slice of the tensor gene pass
+    double* item_part;    // [items x DET_ITEM_SLOTS] per-item, per-CTA, per-warp ELBO terms of the tensor gene pass
+    int* tickets;         // one per own tile of the running tensor pass (chunk order of the accumulator adds)
+    double* simt_colsum;  // [row blocks x p] column sums of D_hat per row block     } CUDA-core kernels,
+    double* simt_elbo;    // [row blocks x 2] ELBO terms per row block               } NULL above
+    float* simt_gene;     // [row chunks x red32] gene sums per row chunk             } DET_SIMT_MAX entries
+    long long doubles;    // size of the whole scratch: ori_det_workspace_doubles
+};
+// ws == NULL: every pointer NULL, the size all the same
+DetWs det_carve(double* ws, long long n_rows, int p);
 inline bool det_simt_ok(long long n_rows, int p) { return n_rows * (long long)p <= DET_SIMT_MAX; }
 // src[n][2] added in index order by one block: *dst0 += sum src[.][0], *dst1 += sum src[.][1]
 int launch_det_sum_pairs(const double* src, long long n, double* dst0, double* dst1, cudaStream_t st);

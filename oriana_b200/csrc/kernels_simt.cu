@@ -41,6 +41,7 @@ __device__ __forceinline__ double block_reduce_sum(double v, double* sbuf) {
 // accumulators in registers and sweeps gene tiles of 32; the X tile is staged (coalesced) through smem.
 constexpr int PR_TR = 128;
 constexpr int PR_TG = 32;
+static_assert(PR_TR == DET_SIMT_BLOCK_ROWS, "det_carve sizes the per-row-block scratch by DET_SIMT_BLOCK_ROWS");
 
 // SPARSE (sparse_zigap.py:100-116, :140-142, :166): the denominator operand eV carries the mask S_tilde, the row
 // sums contract with eVz = eV * S_hat, D_hat is rebuilt from Vh = the PREVIOUS effective V_hat and the rate sums
@@ -210,7 +211,7 @@ k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
         const double s2 = block_reduce_sum(acc_ent, sred);
         if (tid == 0) {
             if (det_part) { det_part[2 * blockIdx.x] = s1; det_part[2 * blockIdx.x + 1] = s2; }
-            else { atomicAdd(part64 + R64_XLOGDEN, s1); atomicAdd(part64 + R64_ENT, s2); }
+            else { atomicAdd(&part64[ORI_R64_XLOGDEN], s1); atomicAdd(&part64[ORI_R64_ENT], s2); }
         }
     }
 }
@@ -522,16 +523,12 @@ k_mstep(ori_problem_t P, int mode)
 {
     __shared__ double sbuf[32];
     const int tid = threadIdx.x;
-    const int p = P.p, K = P.K, KP = P.KP;
+    const int p = P.p, K = P.K;
     const double n = (double)P.n_total;
     const bool dropout = (P.flags & ORI_F_DROPOUT) != 0;
-    double* colsum = P.red64;
-    double* SlogU = P.red64 + p;
-    double* SU = P.red64 + p + KP;
-    double* part = P.red64 + p + 2 * KP;
-    double* SlogV = P.gsum;
-    double* SV = P.gsum + KP;
-    double* gpart = P.gsum + 2 * KP;
+    const RedBufs red = red_carve(P);
+    double* colsum = red.colsum, *SlogU = red.SlogU, *SU = red.SU, *part = red.part;
+    double* SlogV = red.SlogV, *SV = red.SV, *gpart = red.gpart;
 
     // ---- phase 1: pi(t) and ELBO(t) of the state the row pass has just swept
     if (mode == ORI_M_STEP || mode == ORI_M_FINALIZE) {
@@ -551,16 +548,16 @@ k_mstep(ori_problem_t P, int mode)
         }
         const double b = block_reduce_sum(bern, sbuf);
         if (tid == 0) {
-            double e = part[R64_XLOGDEN] - P.scal[SC_LGAMX] + P.scal[SC_PENDING];
+            double e = part[ORI_R64_XLOGDEN] - P.scal[ORI_SC_LGAMX] + P.scal[ORI_SC_PENDING];
             if (dropout) {
                 const double q = 1e-10;  // p_d of a non-zero entry is 1 - 1e-10 (zigap.py:135)
                 const double h_nz = -(1.0 - q) * log1p(-q) - q * log(q);
-                e += -part[R64_PUV] + part[R64_ENT] + P.scal[SC_NNZ] * h_nz + b;
+                e += -part[ORI_R64_PUV] + part[ORI_R64_ENT] + P.scal[ORI_SC_NNZ] * h_nz + b;
             } else {
-                e -= P.scal[6];  // sum_k (sum_i U_hat_ik)(sum_j V_hat_jk) of the swept state
+                e -= P.scal[ORI_SC_UVSUM];  // sum_k (sum_i U_hat_ik)(sum_j V_hat_jk) of the swept state
             }
-            P.scal[SC_ELBO_LAST] = e;
-            const int it = (P.flags & ORI_F_DEVICE_ITER) ? (int)P.scal[SC_ITER] : P.iter;
+            P.scal[ORI_SC_ELBO_LAST] = e;
+            const int it = (P.flags & ORI_F_DEVICE_ITER) ? (int)P.scal[ORI_SC_ITER] : P.iter;
             if (it >= 0 && it < P.trace_cap) P.elbo_trace[it] = e;
         }
         __syncthreads();
@@ -569,7 +566,7 @@ k_mstep(ori_problem_t P, int mode)
 
     // ---- phase 2: M-step on the new expectations (zigap.py:143-155); alpha1 uses the OLD alpha2
     if (mode == ORI_M_INIT || mode == ORI_M_INIT_KEEP) {
-        if (tid == 0) { P.scal[SC_LGAMX] = part[4]; P.scal[SC_NNZ] = part[5]; }
+        if (tid == 0) { P.scal[ORI_SC_LGAMX] = part[ORI_R64_LGAMX]; P.scal[ORI_SC_NNZ] = part[ORI_R64_NNZ]; }
         if (dropout)
             for (int j = tid; j < p; j += blockDim.x) {
                 P.pi_d[j] = colsum[j] / n;        // column means of p_d = (X>0)  (base.py:52 -> zigap.py:158)
@@ -599,10 +596,10 @@ k_mstep(ori_problem_t P, int mode)
     const double ps = block_reduce_sum(pend, sbuf);
     const double us = block_reduce_sum(uvs, sbuf);
     if (tid == 0) {
-        P.scal[SC_PENDING] = ps + part[R64_HROW] + gpart[0];
-        P.scal[6] = us;
-        const int it = (P.flags & ORI_F_DEVICE_ITER) ? (int)P.scal[SC_ITER] : P.iter;
-        P.scal[SC_ITER] = (double)(mode == ORI_M_STEP ? it + 1 : it);
+        P.scal[ORI_SC_PENDING] = ps + part[ORI_R64_HROW] + gpart[ORI_GSUM_HGENE];
+        P.scal[ORI_SC_UVSUM] = us;
+        const int it = (P.flags & ORI_F_DEVICE_ITER) ? (int)P.scal[ORI_SC_ITER] : P.iter;
+        P.scal[ORI_SC_ITER] = (double)(mode == ORI_M_STEP ? it + 1 : it);
     }
 }
 
@@ -625,7 +622,7 @@ k_count_stats(const float* __restrict__ X, long long ldx, long long n_rows, int 
     if (j < p && cnt != 0.f) atomicAdd(colsum + j, (double)cnt);
     const double s1 = block_reduce_sum(lg, sred);
     const double s2 = block_reduce_sum((double)cnt, sred);
-    if (threadIdx.x == 0) { atomicAdd(part64 + 4, s1); atomicAdd(part64 + 5, s2); }
+    if (threadIdx.x == 0) { atomicAdd(&part64[ORI_R64_LGAMX], s1); atomicAdd(&part64[ORI_R64_NNZ], s2); }
 }
 
 // eUw[i,k] = eU[i,k] * D_hat[i, gene k]   (the operand that reproduces zigap.py:94)
@@ -696,10 +693,9 @@ k_sparse_gene_update(ori_problem_t P, double* __restrict__ blk_part)
     double dL[32], dE[32];               // this gene's contributions (K <= 32), kept for the ordered sums
 #pragma unroll
     for (int k = 0; k < 32; ++k) { dL[k] = 0.0; dE[k] = 0.0; }
+    const RedBufs red = red_carve(P);
     if (j < p) {
-        const float* Zj = P.red32;
-        const float* b2s = P.red32 + (long long)p * KP;
-        const float* Zl = P.red32 + 2ll * p * KP;
+        const float* Zj = red.Zj, *b2s = red.b2s, *Zl = red.Zl;
         const double* beta1 = P.hyper + 2 * K, *beta2 = P.hyper + 3 * K;
         const double pis = P.pi_s[j];
         const double lps = logit_f64(pis);
@@ -778,8 +774,8 @@ k_sparse_gene_update(ori_problem_t P, double* __restrict__ blk_part)
     }
     __syncthreads();
     if (threadIdx.x < K) {
-        atomicAdd(P.gsum + threadIdx.x, sSlog[threadIdx.x]);
-        atomicAdd(P.gsum + KP + threadIdx.x, sShat[threadIdx.x]);
+        atomicAdd(&red.SlogV[threadIdx.x], sSlog[threadIdx.x]);
+        atomicAdd(&red.SV[threadIdx.x], sShat[threadIdx.x]);
     }
 }
 
@@ -1030,21 +1026,23 @@ static int pass_rows_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     int gy = 1;  // split the gene sweep until there are several waves of CTAs (3 resident per SM): a 1.8-wave grid idles
     while (bx * gy < 148 * 3 * 6 && gy * 2 <= ntiles) gy *= 2;   // most of the machine during its last wave
     const bool drop = P->flags & ORI_F_DROPOUT, elbo = P->flags & ORI_F_ELBO;
-    double* colsum = P->red64;
-    double* part = P->red64 + P->p + 2 * P->KP;
+    const RedBufs red = red_carve(*P);
+    double* colsum = red.colsum;
+    double* part = red.part;
     // ORI_F_DETERMINISTIC: one CTA per row block (a single add per Zi / a2s element), per-CTA slots for the rest
     double* det_cs = nullptr; double* det_part = nullptr;
     if ((P->flags & ORI_F_DETERMINISTIC) && P->det_ws) {
         if (!det_simt_ok(P->n_rows, P->p)) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC on the CUDA-core kernels: problem too large");
         gy = 1;
-        det_cs = P->det_ws + det_simt_offset(P->n_rows, P->p);
-        det_part = det_cs + (long long)bx * P->p;
+        const DetWs d = det_carve(P->det_ws, P->n_rows, P->p);
+        det_cs = d.simt_colsum;
+        det_part = d.simt_elbo;
     }
     auto det_sums = [&]() -> int {
         if (!det_cs) return ORI_OK;
         int nk = 0;
         if (drop) { k_det_sum_cols<<<cdiv(P->p, 128), 128, 0, st>>>(colsum, det_cs, bx, P->p); ++nk; }
-        if (elbo) { if (launch_det_sum_pairs(det_part, bx, part + R64_XLOGDEN, part + R64_ENT, st) != ORI_OK) return ORI_ECUDA; }
+        if (elbo) { if (launch_det_sum_pairs(det_part, bx, part + ORI_R64_XLOGDEN, part + ORI_R64_ENT, st) != ORI_OK) return ORI_ECUDA; }
         return nk ? check_launch("k_det_sum_cols", nk) : ORI_OK;
     };
     dim3 grid(bx, gy);
@@ -1090,23 +1088,21 @@ static int pass_genes_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     const bool third = P->eUl[g] != nullptr;      // the third sum Zl into red32 block 2
     // ORI_F_DETERMINISTIC: nominal chunks only (their number bounds the scratch), every chunk stores to its own slot
     float* det_z = nullptr;
-    const long long det_stride = (long long)(third ? 3 : 2) * P->p * P->KP;
+    const long long det_stride = ORI_RED32_FLOATS(P->p, P->KP, third);
     if ((P->flags & ORI_F_DETERMINISTIC) && P->det_ws) {
         if (!det_simt_ok(P->n_rows, P->p)) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC on the CUDA-core kernels: problem too large");
-        rpc = 8192;
-        const long long nb = cdiv(P->n_rows, PR_TR);
-        det_z = reinterpret_cast<float*>(P->det_ws + det_simt_offset(P->n_rows, P->p) + nb * P->p + 2 * nb + 2);
+        rpc = DET_SIMT_CHUNK_ROWS;
+        det_z = det_carve(P->det_ws, P->n_rows, P->p).simt_gene;
     }
     const int gy = cdiv(P->n_rows, rpc);
     dim3 grid(bx, gy);
     const bool drop = P->flags & ORI_F_DROPOUT, quirk = (P->flags & ORI_F_QUIRK) != 0;
-    float* Zj = P->red32;
-    float* b2s = P->red32 + (long long)P->p * P->KP;
+    const RedBufs red = red_carve(*P);
     auto det_sums = [&]() -> int {
         if (!det_z) return ORI_OK;
         // blocks of the [Zj | b2s | Zl] scratch that this launch did not write (no dropout) are never read: sum what exists
         const long long total = drop ? det_stride : (long long)P->p * P->KP;
-        k_det_sum_chunks_strided<<<cdiv(total, 256), 256, 0, st>>>(P->red32, det_z, gy, total, det_stride);
+        k_det_sum_chunks_strided<<<cdiv(total, 256), 256, 0, st>>>(red.Zj, det_z, gy, total, det_stride);
         return check_launch("k_det_sum_chunks");
     };
     // sparse model (without ORI_F_DROPOUT: the operator seam, api.cu, D_hat folded into X): the masked denominator
@@ -1116,7 +1112,7 @@ static int pass_genes_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     const float* Vh = sparse ? P->Vh_old : P->V_hat;
 #define ORI_LAUNCH_PG(D, Q, T)                                                                                  \
     k_pass_genes<KP, D, Q, T><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, P->eU[g], P->eUw, \
-        P->U_hat[g], P->U_hat[1 - g], P->eUl[g], eV, Vh, P->lp, P->pfloor, Zj, b2s, P->red32 + 2ll * P->p * P->KP, \
+        P->U_hat[g], P->U_hat[1 - g], P->eUl[g], eV, Vh, P->lp, P->pfloor, red.Zj, red.b2s, red.Zl,              \
         (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,        \
         det_z, det_stride)
     if (third && drop) ORI_LAUNCH_PG(true, false, true);
@@ -1157,35 +1153,34 @@ __global__ void k_det_sum_blocks(const double* __restrict__ blk_part, int nblock
 
 static int update_grid(long long total) {
     long long b = (total + 255) / 256;
-    return (int)(b < 1 ? 1 : (b > 148 * 8 ? 148 * 8 : b));
+    return (int)(b < 1 ? 1 : (b > DET_FU_BLOCKS ? DET_FU_BLOCKS : b));
 }
 
 // write_state: 1 = regular update into generation 1-gen_old; 0 = only the ELBO term sum D_hat*uv of
 // the swept state (finalize); 2 = expectations of generation gen_old from (a1,a2) with their column sums
 // (init); 3 = the same expectations without touching any sum (host-streamed slabs).
 int launch_row_update(const ori_problem_t* P, int g, int write_state, cudaStream_t st) {
-    const int p = P->p, K = P->K, KP = P->KP;
-    double* SlogU = P->red64 + p;
-    double* SU = P->red64 + p + KP;
-    double* part = P->red64 + p + 2 * KP;
+    const int K = P->K, KP = P->KP;
+    const RedBufs red = red_carve(*P);
+    double* Hrow = red.part + ORI_R64_HROW;
     const bool drop = P->flags & ORI_F_DROPOUT, sparse = P->flags & ORI_F_SPARSE;
     const bool det = (P->flags & ORI_F_DETERMINISTIC) && P->det_ws;
+    double* fu = det ? det_carve(P->det_ws, P->n_rows, P->p).fu_part : nullptr;
     const int grid = update_grid(P->n_rows * KP);
     if (write_state >= 2) {
         const bool sums = write_state == 2;
         k_factor_update<true><<<grid, 256, 0, st>>>(P->n_rows, K, KP, nullptr, nullptr, nullptr, nullptr,
             nullptr, nullptr, nullptr, P->a1, P->a2, P->U_hat[g], P->eU[g], sparse ? P->eUl[g] : nullptr, P->xrow,
-            sums ? SlogU : nullptr, SU, part + R64_HROW, nullptr, 1, P->thrU ? P->thrU + (long long)g * P->n_rows : nullptr,
-            (det && sums) ? P->det_ws : nullptr);
-        if (det && sums) k_det_sum_blocks<<<1, 256, 0, st>>>(P->det_ws, grid, K, SlogU, SU, part + R64_HROW, nullptr);
+            sums ? red.SlogU : nullptr, red.SU, Hrow, nullptr, 1, P->thrU ? P->thrU + (long long)g * P->n_rows : nullptr,
+            sums ? fu : nullptr);
+        if (det && sums) k_det_sum_blocks<<<1, 256, 0, st>>>(fu, grid, K, red.SlogU, red.SU, Hrow, nullptr);
     } else {
-        // GaP: rate = alpha2 + sum_j V_hat_jk (gap.py:98); the column sums live in gsum[KP..2KP)
+        // GaP: rate = alpha2 + sum_j V_hat_jk (gap.py:98)
         k_factor_update<false><<<grid, 256, 0, st>>>(P->n_rows, K, KP, P->Zi, P->eU[g],
-            drop ? P->a2s : nullptr, P->gsum + KP, P->hyper, P->hyper + K, P->U_hat[g],
-            P->a1, P->a2, P->U_hat[1 - g], P->eU[1 - g], sparse ? P->eUl[1 - g] : nullptr, P->xrow, SlogU, SU,
-            part + R64_HROW, part + R64_PUV, write_state, P->thrU ? P->thrU + (long long)(1 - g) * P->n_rows : nullptr,
-            det ? P->det_ws : nullptr);
-        if (det) k_det_sum_blocks<<<1, 256, 0, st>>>(P->det_ws, grid, K, SlogU, SU, part + R64_HROW, part + R64_PUV);
+            drop ? P->a2s : nullptr, red.SV, P->hyper, P->hyper + K, P->U_hat[g],
+            P->a1, P->a2, P->U_hat[1 - g], P->eU[1 - g], sparse ? P->eUl[1 - g] : nullptr, P->xrow, red.SlogU, red.SU,
+            Hrow, red.part + ORI_R64_PUV, write_state, P->thrU ? P->thrU + (long long)(1 - g) * P->n_rows : nullptr, fu);
+        if (det) k_det_sum_blocks<<<1, 256, 0, st>>>(fu, grid, K, red.SlogU, red.SU, Hrow, red.part + ORI_R64_PUV);
     }
     return check_launch("k_factor_update(rows)", det ? 2 : 1);
 }
@@ -1193,32 +1188,30 @@ int launch_row_update(const ori_problem_t* P, int g, int write_state, cudaStream
 int launch_gene_update(const ori_problem_t* P, int write_state, cudaStream_t st) {
     const int p = P->p, K = P->K, KP = P->KP;
     const bool drop = P->flags & ORI_F_DROPOUT;
-    double* SlogV = P->gsum; double* SV = P->gsum + KP; double* gpart = P->gsum + 2 * KP;
-    const bool det = (P->flags & ORI_F_DETERMINISTIC) && P->det_ws && !(P->flags & ORI_F_SPARSE);
+    const RedBufs red = red_carve(*P);
+    double* Hgene = red.gpart + ORI_GSUM_HGENE;
+    const bool det = (P->flags & ORI_F_DETERMINISTIC) && P->det_ws;
+    double* fu = det ? det_carve(P->det_ws, P->n_rows, P->p).fu_part : nullptr;
     const int grid = update_grid((long long)p * KP);
     if (P->flags & ORI_F_SPARSE) {
         const int gs = cdiv(p, 128);
-        const bool sdet = (P->flags & ORI_F_DETERMINISTIC) && P->det_ws;
-        if (sdet && gs > DET_FU_BLOCKS) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC: too many genes for the sparse update");
-        double* bp = sdet ? P->det_ws : nullptr;
-        if (write_state == 2) k_sparse_gene_update<true><<<gs, 128, 0, st>>>(*P, bp);
-        else k_sparse_gene_update<false><<<gs, 128, 0, st>>>(*P, bp);
-        if (sdet) k_det_sum_blocks<<<1, 256, 0, st>>>(P->det_ws, gs, K, SlogV, SV, nullptr, nullptr);
-        return check_launch("k_sparse_gene_update", sdet ? 2 : 1);
+        if (det && gs > DET_FU_BLOCKS) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC: too many genes for the sparse update");
+        if (write_state == 2) k_sparse_gene_update<true><<<gs, 128, 0, st>>>(*P, fu);
+        else k_sparse_gene_update<false><<<gs, 128, 0, st>>>(*P, fu);
+        if (det) k_det_sum_blocks<<<1, 256, 0, st>>>(fu, gs, K, red.SlogV, red.SV, nullptr, nullptr);
+        return check_launch("k_sparse_gene_update", det ? 2 : 1);
     }
     if (write_state == 2) {
         k_factor_update<true><<<grid, 256, 0, st>>>(p, K, KP, nullptr, nullptr, nullptr, nullptr,
-            nullptr, nullptr, nullptr, P->b1, P->b2, P->V_hat, P->eV, nullptr, P->xcol, SlogV, SV, gpart, nullptr, 1, P->thrV,
-            det ? P->det_ws : nullptr);
+            nullptr, nullptr, nullptr, P->b1, P->b2, P->V_hat, P->eV, nullptr, P->xcol, red.SlogV, red.SV, Hgene, nullptr, 1,
+            P->thrV, fu);
     } else {
-        // GaP: rate = beta2 + sum_i U_hat_ik (gap.py:106) with the NEW U_hat: red64[p+KP ..)
-        float* Zj = P->red32; float* b2s = P->red32 + (long long)p * KP;
-        k_factor_update<false><<<grid, 256, 0, st>>>(p, K, KP, Zj, P->eV, drop ? b2s : nullptr,
-            P->red64 + p + KP, P->hyper + 2 * K, P->hyper + 3 * K, nullptr,
-            P->b1, P->b2, P->V_hat, P->eV, nullptr, P->xcol, SlogV, SV, gpart, nullptr, write_state, P->thrV,
-            det ? P->det_ws : nullptr);
+        // GaP: rate = beta2 + sum_i U_hat_ik (gap.py:106) with the NEW U_hat
+        k_factor_update<false><<<grid, 256, 0, st>>>(p, K, KP, red.Zj, P->eV, drop ? red.b2s : nullptr,
+            red.SU, P->hyper + 2 * K, P->hyper + 3 * K, nullptr,
+            P->b1, P->b2, P->V_hat, P->eV, nullptr, P->xcol, red.SlogV, red.SV, Hgene, nullptr, write_state, P->thrV, fu);
     }
-    if (det) k_det_sum_blocks<<<1, 256, 0, st>>>(P->det_ws, grid, K, SlogV, SV, gpart, nullptr);
+    if (det) k_det_sum_blocks<<<1, 256, 0, st>>>(fu, grid, K, red.SlogV, red.SV, Hgene, nullptr);
     return check_launch("k_factor_update(genes)", det ? 2 : 1);
 }
 
@@ -1233,8 +1226,8 @@ int launch_count_stats(const ori_problem_t* P, cudaStream_t st) {
     while (bx * chunks < 148 * 4 && P->n_rows / (chunks * 2) >= 16) chunks *= 2;
     const long long rpc = (P->n_rows + chunks - 1) / chunks;
     dim3 grid(bx, cdiv(P->n_rows, rpc));
-    k_count_stats<<<grid, 128, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, P->red64,
-                                        P->red64 + P->p + 2 * P->KP);
+    const RedBufs red = red_carve(*P);
+    k_count_stats<<<grid, 128, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, red.colsum, red.part);
     return check_launch("k_count_stats");
 }
 

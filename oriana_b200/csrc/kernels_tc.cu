@@ -916,8 +916,8 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                             slot[0] = acc_xl * (double)LN2;
                             slot[1] = DROPOUT ? acc_ent * (double)LN2 : 0.0;
                         } else {
-                            atomicAdd(a.part64 + R64_XLOGDEN, acc_xl * (double)LN2);
-                            if (DROPOUT) atomicAdd(a.part64 + R64_ENT, acc_ent * (double)LN2);
+                            atomicAdd(&a.part64[ORI_R64_XLOGDEN], acc_xl * (double)LN2);
+                            if (DROPOUT) atomicAdd(&a.part64[ORI_R64_ENT], acc_ent * (double)LN2);
                         }
                     }
                 }
@@ -1084,7 +1084,7 @@ __global__ void k_det_add(double* __restrict__ dst, const double* __restrict__ s
 #endif
 static long long pad128(long long v) { return (v + 127) / 128 * 128; }
 
-long long det_max_items(long long n_rows, int p) {
+static long long det_max_items(long long n_rows, int p) {
     // items = own units x sweep chunks; the shortest nominal chunk is ORI_TC_CHUNK_PRECISE sweep entries, own units are at
     // least 128 wide, and the small-problem splitting of tc_partition stops below one item per SM
     const long long np = pad128(n_rows), pp = pad128(p);
@@ -1092,18 +1092,31 @@ long long det_max_items(long long n_rows, int p) {
     long long m = a > b ? a : b;
     return m > 2 * 148 ? m : 2 * 148;
 }
-long long det_simt_offset(long long n_rows, int p) {
-    const long long tiles = (pad128(n_rows) + pad128(p)) / 128 + 64;
-    return (long long)DET_FU_BLOCKS * DET_FU_SLOTS + pad128(p) + det_max_items(n_rows, p) * DET_ITEM_SLOTS + (tiles + 1) / 2 + 2;
-}
-long long det_workspace_doubles(long long n_rows, int p, int KP) {
-    (void)KP;
-    long long simt = 0;
+// The regions are sized in doubles.  Three terms are larger than what the kernels use (the ticket region's 64 spare
+// tiles and its 2 doubles, the 2 doubles after the ELBO terms, the 8 after the gene sums); they are kept so that
+// ori_det_workspace_doubles returns the size it always has.
+DetWs det_carve(double* ws, long long n_rows, int p) {
+    DetWs d;
+    long long at = 0;
+    auto take = [&](long long doubles) { double* r = ws ? ws + at : nullptr; at += doubles; return r; };
+    const long long np = pad128(n_rows), pp = pad128(p);
+    d.fu_part = take((long long)DET_FU_BLOCKS * DET_FU_SLOTS);
+    d.colsum2 = take(pp);
+    d.item_part = take(det_max_items(n_rows, p) * DET_ITEM_SLOTS);
+    // a pass uses n_own_tiles + 2 tickets, n_own_tiles <= max(np, pp) / 128
+    const long long tiles = (np + pp) / 128 + 64;
+    d.tickets = reinterpret_cast<int*>(take((tiles + 1) / 2 + 2));
+    d.simt_colsum = d.simt_elbo = nullptr;
+    d.simt_gene = nullptr;
     if (det_simt_ok(n_rows, p)) {
-        const long long nb = (n_rows + 127) / 128, chunks = (n_rows + 8191) / 8192;
-        simt = nb * p + 2 * nb + 2 + (chunks * 3 * p * 64 + 1) / 2 + 8;
+        const long long nb = (n_rows + DET_SIMT_BLOCK_ROWS - 1) / DET_SIMT_BLOCK_ROWS;
+        const long long chunks = (n_rows + DET_SIMT_CHUNK_ROWS - 1) / DET_SIMT_CHUNK_ROWS;
+        d.simt_colsum = take(nb * p);
+        d.simt_elbo = take(2 * nb + 2);
+        d.simt_gene = reinterpret_cast<float*>(take((chunks * 3 * p * 64 + 1) / 2 + 8));   // floats, at any KP <= 64
     }
-    return det_simt_offset(n_rows, p) + simt;
+    d.doubles = at;
+    return d;
 }
 int launch_det_sum_pairs(const double* src, long long n, double* dst0, double* dst1, cudaStream_t st) {
     k_det_sum_items<<<1, 1024, 0, st>>>(src, n, dst0, dst1);
@@ -1269,6 +1282,7 @@ template <bool GENES, int KP, bool PRECISE>
 static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st, bool logsum = false) {
     using C = Cfg<KP, PRECISE>;
     const TcWs w = tc_carve(P);
+    const RedBufs red = red_carve(*P);
     const bool sparse = P->flags & ORI_F_SPARSE;
     const bool drop = (P->flags & ORI_F_DROPOUT) && !logsum, elbo = (P->flags & ORI_F_ELBO) && !logsum;
     constexpr int SW = C::SW;
@@ -1290,7 +1304,7 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
              make_tmap_f32(&maps.X, P->X, P->n_rows, P->p, P->ldx, 32, SW);
         a.own_total = P->p; a.sw_total = P->n_rows; a.sw_pad = w.np;
         a.own_e = sparse ? P->eVd : P->eV; a.own_E = sparse ? P->Vh_old : P->V_hat;
-        a.acc1 = P->red32 + (logsum ? 2ll * P->p * KP : 0ll); a.acc2 = P->red32 + (long long)P->p * KP;
+        a.acc1 = logsum ? red.Zl : red.Zj; a.acc2 = red.b2s;
     }
     if (!ok) return set_error(ORI_ECUDA, "cuTensorMapEncodeTiled failed");
     a.lp2w = w.lp2w; a.flw = w.flw; a.cw = w.cw; a.any_floor = w.flags;
@@ -1299,7 +1313,7 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
     a.thr_own = ufl ? (GENES ? P->thrV : thr_rows) : nullptr;
     a.thr_sw = ufl ? (GENES ? thr_rows : P->thrV) : nullptr;
     a.thr_sw_max = ufl ? reinterpret_cast<const float*>(w.flags + (GENES ? 2 : 1)) : nullptr;
-    a.colsum = P->red64; a.part64 = P->red64 + P->p + 2 * P->KP;
+    a.colsum = red.colsum; a.part64 = red.part;
     a.n_own_tiles = cdiv(a.own_total, TC_OWN);
     a.n_own_units = cdiv(a.n_own_tiles, NCTA);
     a.n_sw_tiles = cdiv(a.sw_total, SW);
@@ -1311,13 +1325,14 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
     if (det) {
         if (ufl) return set_error(ORI_EUNSUPPORTED, "ORI_F_DETERMINISTIC and the underflow thresholds cannot be combined on the tensor path");
         if (a.n_items > det_max_items(P->n_rows, P->p)) return set_error(ORI_EINVAL, "det_ws too small for %d items", a.n_items);
-        a.colsum2 = P->det_ws + (long long)DET_FU_BLOCKS * DET_FU_SLOTS;
-        a.item_part = a.colsum2 + pad128(P->p);
+        const DetWs d = det_carve(P->det_ws, P->n_rows, P->p);
+        a.colsum2 = d.colsum2;
+        a.item_part = d.item_part;
         if (GENES && drop) {
             const cudaError_t e2 = cudaMemsetAsync(a.colsum2, 0, sizeof(double) * (size_t)P->p, st);
             if (e2 != cudaSuccess) return set_error(ORI_ECUDA, "cudaMemsetAsync(colsum2): %s", cudaGetErrorString(e2));
         }
-        a.tickets = reinterpret_cast<int*>(a.item_part + det_max_items(P->n_rows, P->p) * DET_ITEM_SLOTS);
+        a.tickets = d.tickets;
         cudaError_t e_ = cudaMemsetAsync(a.tickets, 0, sizeof(int) * (size_t)(a.n_own_tiles + 2), st);
         if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaMemsetAsync(tickets): %s", cudaGetErrorString(e_));
         if (!(GENES && elbo)) a.item_part = nullptr;
@@ -1331,10 +1346,10 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
                        : launch_tc_flags<GENES, KP, PRECISE, false, false>(drop, elbo, maps, a, grid, st);
     if (rc != ORI_OK) return rc;
     int extra = 0;
-    if (det && GENES && drop) { k_det_add<<<cdiv(P->p, 256), 256, 0, st>>>(P->red64, a.colsum2, P->p); ++extra; }
+    if (det && GENES && drop) { k_det_add<<<cdiv(P->p, 256), 256, 0, st>>>(red.colsum, a.colsum2, P->p); ++extra; }
     if (a.item_part) {
-        double* part = P->red64 + P->p + 2 * P->KP;
-        k_det_sum_items<<<1, 1024, 0, st>>>(a.item_part, (long long)a.n_items * (DET_ITEM_SLOTS / 2), part + R64_XLOGDEN, part + R64_ENT);
+        k_det_sum_items<<<1, 1024, 0, st>>>(a.item_part, (long long)a.n_items * (DET_ITEM_SLOTS / 2), red.part + ORI_R64_XLOGDEN,
+                                            red.part + ORI_R64_ENT);
         ++extra;
     }
     if (extra) return check_launch("k_tc_pass + deterministic sums", 1 + extra);

@@ -258,7 +258,7 @@ class HostStreamedCAVI:
         self.pi_d = host(np.zeros(p), torch.float64, (p,))
         self.lp = host(np.full(p, -np.inf), torch.float32, (p,))
         self.pfloor = host(np.zeros(p), torch.float32, (p,))
-        self.scal = host(np.zeros(_lib.SCAL_SLOTS), torch.float64, (_lib.SCAL_SLOTS,))
+        self.scal = host(np.zeros(_lib.ORI_SC_NSLOTS), torch.float64, (_lib.ORI_SC_NSLOTS,))
         self.elbo_trace = []
         self.iterations = 0
 
@@ -331,7 +331,7 @@ class HostStreamedCAVI:
         g['hyper'].copy_(self.hyper, non_blocking=True)
         g['lp'].copy_(self.lp, non_blocking=True); g['pfloor'].copy_(self.pfloor, non_blocking=True)
         g['scal'].copy_(self.scal, non_blocking=True)
-        self.h2d_bytes += 2 * self.p * K * 4 + 4 * K * 8 + self.p * 8 + _lib.SCAL_SLOTS * 8
+        self.h2d_bytes += 2 * self.p * K * 4 + 4 * K * 8 + self.p * 8 + _lib.ORI_SC_NSLOTS * 8
 
     def _copy_slab(self, s, r0, rows):
         """Host -> device copies of one slab (current stream = the copy stream): X in the form the host holds it, the escape
@@ -449,7 +449,7 @@ class HostStreamedCAVI:
         g, K = self._g, self.k
         self.hyper.copy_(g['hyper'], non_blocking=True)
         self.scal.copy_(g['scal'], non_blocking=True)
-        self.d2h_bytes += 4 * K * 8 + _lib.SCAL_SLOTS * 8
+        self.d2h_bytes += 4 * K * 8 + _lib.ORI_SC_NSLOTS * 8
         if self.dropout:
             self.pi_d.copy_(g['pi_d'], non_blocking=True)
             self.lp.copy_(g['lp'], non_blocking=True); self.pfloor.copy_(g['pfloor'], non_blocking=True)
@@ -485,7 +485,7 @@ class HostStreamedCAVI:
         self._download_genes()
         torch.cuda.current_stream().synchronize()                   # results are on the host when we return
         self.iterations += 1
-        e = float(self.scal[4])
+        e = float(self.scal[_lib.ORI_SC_ELBO_LAST])
         self.elbo_trace.append(e)
         return e
 

@@ -332,7 +332,7 @@ class FactorModel(metaclass=ABCMeta):
             self.update_prior_hyper_parameters()
             return
         if g == 'warm':
-            self._scal[5] = float(self._iter)             # SC_ITER: the device-side count the captured kernels read
+            self._scal[_lib.ORI_SC_ITER] = float(self._iter)      # the device-side count the captured kernels read
             torch.cuda.synchronize()
             before = int(self._lib.ori_kernel_launches())
             g = torch.cuda.CUDAGraph()
@@ -440,7 +440,7 @@ class FactorModel(metaclass=ABCMeta):
     def elbo(self):
         """Evidence lower bound of the current state (float64 accumulation on the device)."""
         self._finalize()
-        return float(self._scal[4].item())
+        return float(self._scal[_lib.ORI_SC_ELBO_LAST].item())
 
     @property
     def elbo_trace(self):
@@ -524,7 +524,7 @@ class FactorModel(metaclass=ABCMeta):
         self._after_load_state(state)
         # the device-side iteration count (ORI_F_DEVICE_ITER: index of the next ELBO trace entry under graph replay) and
         # the trace follow the host-side count of the loaded state
-        self._scal[5] = float(self._iter)
+        self._scal[_lib.ORI_SC_ITER] = float(self._iter)
         self._trace.zero_()
         if self._graphs is not None:
             self._graphs.clear()

@@ -47,11 +47,11 @@ def gene_buffers(p, K, KP, device, dropout, sparse, trace_cap):
     f32, f64 = dict(dtype=torch.float32, device=device), dict(dtype=torch.float64, device=device)
     return dict(
         b1=torch.zeros((p, KP), **f32), b2=torch.zeros((p, KP), **f32), V_hat=torch.zeros((p, KP), **f32),
-        eV=torch.zeros((p, KP), **f32), red32=torch.zeros((3 if sparse else 2, p, KP), **f32),
+        eV=torch.zeros((p, KP), **f32), red32=torch.zeros((_lib.ORI_RED32_FLOATS(p, KP, sparse),), **f32).view(-1, p, KP),
         lp=torch.full((p,), float('-inf'), **f32) if dropout else None,
         pfloor=torch.zeros((p,), **f32) if dropout else None, pi_d=torch.zeros((p,), **f64) if dropout else None,
-        hyper=torch.ones((4, K), **f64), red64=torch.zeros((p + 2 * KP + _lib.R64_NSLOTS,), **f64),
-        gsum=torch.zeros((2 * KP + 8,), **f64), scal=torch.zeros((_lib.SCAL_SLOTS,), **f64),
+        hyper=torch.ones((4, K), **f64), red64=torch.zeros((_lib.ORI_RED64_DOUBLES(p, KP),), **f64),
+        gsum=torch.zeros((_lib.ORI_GSUM_DOUBLES(KP),), **f64), scal=torch.zeros((_lib.ORI_SC_NSLOTS,), **f64),
         elbo_trace=torch.zeros((trace_cap,), **f64))
 
 

@@ -76,8 +76,8 @@ def test_row_pitch_and_gene_buffer_sizes():
         for name in ('b1', 'b2', 'V_hat', 'eV'):
             assert g[name].shape == (p, KP) and g[name].dtype == torch.float32
         assert g['red32'].shape == (3 if sparse else 2, p, KP)
-        assert g['red64'].shape == (p + 2 * KP + _lib.R64_NSLOTS,) and g['red64'].dtype == torch.float64
-        assert g['gsum'].shape == (2 * KP + 8,) and g['scal'].shape == (_lib.SCAL_SLOTS,)
+        assert g['red64'].shape == (p + 2 * KP + _lib.ORI_R64_NSLOTS,) and g['red64'].dtype == torch.float64
+        assert g['gsum'].shape == (2 * KP + _lib.ORI_GSUM_NSLOTS,) and g['scal'].shape == (_lib.ORI_SC_NSLOTS,)
         assert g['hyper'].shape == (4, K) and bool((g['hyper'] == 1).all()) and g['elbo_trace'].shape == (7,)
         if dropout:
             assert g['lp'].shape == g['pfloor'].shape == g['pi_d'].shape == (p,) and bool(torch.isinf(g['lp']).all())
