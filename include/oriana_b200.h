@@ -61,6 +61,10 @@ extern "C" {
                                  ticket per block); per-item ELBO terms and per-block factor sums go through scratch arrays
                                  that are summed in index order.  CUDA-core kernels (up to 2^26 matrix entries): one CTA per
                                  row block, per-CTA / per-row-chunk slots summed in index order.  Needs det_ws.             */
+#define ORI_F_X_U16 512u      /* X holds the counts as uint16_t (the caller casts the pointer): half the bytes of float32 in HBM.
+                                 ldx (elements) must be a multiple of 8, so that a row starts on 16 bytes for TMA.  Every kernel
+                                 widens a count to float32 exactly (u < 2^23) as it reads it, so the results are those of the
+                                 float32 matrix of the same counts                                                          */
 
 /* modes of ori_mstep */
 #define ORI_M_STEP 0          /* regular end of iteration t+1: finalise ELBO(t), pi(t); M-step; next lp   */
@@ -106,7 +110,7 @@ extern "C" {
 typedef struct ori_problem {
     int64_t n_rows;        /* cells owned by this rank                                   */
     int64_t n_total;       /* cells over all ranks (denominator of the M-step means)     */
-    int64_t ldx;           /* row stride of X in elements (multiple of 4)                */
+    int64_t ldx;           /* row stride of X in elements (multiple of 4; of 8 with ORI_F_X_U16) */
     int32_t p;             /* genes                                                      */
     int32_t K;             /* latent dimension                                           */
     int32_t KP;            /* padded latent dimension: 8, 16, 32 or 64, >= K             */
@@ -114,7 +118,7 @@ typedef struct ori_problem {
     int32_t iter;          /* completed iterations (index into elbo_trace)               */
     int32_t trace_cap;     /* capacity of elbo_trace                                     */
 
-    const float* X;        /* [n_rows x ldx] counts as float32 (zigap.py:112)            */
+    const float* X;        /* [n_rows x ldx] counts as float32 (zigap.py:112), or uint16_t with ORI_F_X_U16 */
 
     /* row side, [n_rows x KP] float32 */
     float* a1;             /* Gamma shape of q(U)   zigap.py:115                         */
@@ -252,6 +256,9 @@ int ori_dropout_posterior_f32(const ori_problem_t* P, int gen, float* out, int64
 int ori_row_sums_f32(const float* X, int64_t ldx, int64_t n_rows, int32_t p, float* out, void* stream);
 /* out[c] = sum_i X[i, c] over this rank's rows, float64 (device pointers). */
 int ori_column_sums_f64(const float* X, int64_t ldx, int64_t n_rows, int32_t p, double* out, void* stream);
+/* The same two sums of a uint16 count matrix (ORI_F_X_U16 storage; ldx in elements). */
+int ori_row_sums_u16_f32(const uint16_t* X, int64_t ldx, int64_t n_rows, int32_t p, float* out, void* stream);
+int ori_column_sums_u16_f64(const uint16_t* X, int64_t ldx, int64_t n_rows, int32_t p, double* out, void* stream);
 /* The three zero-inflated Poisson log-likelihood sums behind reconstruction_deviance / explained_deviance for
  * this rank's rows: rate = U_hat V_hat^T masked where round(D_hat) == 0 (base.py:64-67), rate = X (saturated,
  * :68), rate = column means of X (:76; col_mean [p] float64, all ranks).  pi [p] float64 = the finalised pi_d.

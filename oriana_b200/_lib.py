@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get('ORIANA_B200_LIB') or os.path.join(_HERE, 'lib', 'libo
 ORI_F_DROPOUT, ORI_F_QUIRK, ORI_F_ELBO, ORI_F_NO_TENSOR, ORI_F_SPARSE, ORI_F_DEVICE_ITER, ORI_F_PRECISE = 1, 2, 4, 8, 16, 32, 64
 ORI_F_FIXED_CHAIN = 128
 ORI_F_DETERMINISTIC = 256
+ORI_F_X_U16 = 512
 ORI_M_STEP, ORI_M_INIT, ORI_M_INIT_KEEP, ORI_M_FINALIZE, ORI_M_REFRESH = 0, 1, 2, 3, 4
 
 # layout of the reduction buffers of `ori_problem_t` (the ORI_R64_* / ORI_GSUM_* / ORI_SC_* slots and size macros)
@@ -84,6 +85,8 @@ _SIGNATURES = {
     'ori_dropout_posterior_f32': ([_PP, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p], C.c_int),
     'ori_row_sums_f32': ([C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p], C.c_int),
     'ori_column_sums_f64': ([C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p], C.c_int),
+    'ori_row_sums_u16_f32': ([C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p], C.c_int),
+    'ori_column_sums_u16_f64': ([C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p], C.c_int),
     'ori_deviance_sums': ([_PP, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     'ori_zigap_compute_Z_q_expectations_host': ([C.c_void_p] * 7 + [C.c_int64] * 3 + [C.c_int], C.c_int),
     'ori_gap_compute_Z_q_expectations_host': ([C.c_void_p] * 5 + [C.c_int64] * 3, C.c_int),

@@ -177,6 +177,8 @@ int ori_problem_check(const ori_problem_t* P) {
             return set_error(ORI_EINVAL, "ORI_F_DETERMINISTIC needs det_ws of ori_det_workspace_doubles() doubles");
     }
     if (P->ldx < P->p || (P->ldx & 3)) return set_error(ORI_EINVAL, "ldx=%lld must be >= p and a multiple of 4", (long long)P->ldx);
+    if ((P->flags & ORI_F_X_U16) && (P->ldx & 7))     // uint16 rows start on 16 bytes (TMA)
+        return set_error(ORI_EINVAL, "ORI_F_X_U16: ldx=%lld must be a multiple of 8", (long long)P->ldx);
     if (P->n_total < P->n_rows || P->n_total <= 0) return set_error(ORI_EINVAL, "n_total=%lld < n_rows", (long long)P->n_total);
     if ((P->flags & ORI_F_QUIRK) && P->p < P->K) return set_error(ORI_EINVAL, "quirk mode needs p >= K (zigap.py:94 reads D_hat[i, k])");
     const void* need[] = {P->a1, P->a2, P->U_hat[0], P->U_hat[1], P->eU[0], P->eU[1], P->Zi, P->b1, P->b2,
@@ -348,6 +350,17 @@ int ori_row_sums_f32(const float* X, int64_t ldx, int64_t n_rows, int32_t p, flo
 
 int ori_column_sums_f64(const float* X, int64_t ldx, int64_t n_rows, int32_t p, double* out, void* stream) {
     if (n_rows < 0 || p <= 0 || ldx < p || !out || (n_rows > 0 && !X)) return set_error(ORI_EINVAL, "ori_column_sums_f64: bad argument");
+    ORI_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)p, (cudaStream_t)stream));
+    return launch_col_sums(X, ldx, n_rows, p, out, (cudaStream_t)stream);
+}
+
+int ori_row_sums_u16_f32(const uint16_t* X, int64_t ldx, int64_t n_rows, int32_t p, float* out, void* stream) {
+    if (n_rows < 0 || p <= 0 || ldx < p || (n_rows > 0 && (!X || !out))) return set_error(ORI_EINVAL, "ori_row_sums_u16_f32: bad argument");
+    return launch_row_sums(X, ldx, n_rows, p, out, (cudaStream_t)stream);
+}
+
+int ori_column_sums_u16_f64(const uint16_t* X, int64_t ldx, int64_t n_rows, int32_t p, double* out, void* stream) {
+    if (n_rows < 0 || p <= 0 || ldx < p || !out || (n_rows > 0 && !X)) return set_error(ORI_EINVAL, "ori_column_sums_u16_f64: bad argument");
     ORI_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)p, (cudaStream_t)stream));
     return launch_col_sums(X, ldx, n_rows, p, out, (cudaStream_t)stream);
 }

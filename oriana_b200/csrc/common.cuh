@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 #include "../../include/oriana_b200.h"
 
 namespace ori {
@@ -33,6 +34,20 @@ __host__ __device__ inline RedBufs red_carve(const ori_problem_t& P) {
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// Counts stored as uint16 (ORI_F_X_U16) are widened to float32 as they are read, exactly (u < 2^23): the bits
+// 0x4B000000 | u are the float 2^23 + u, and one FADD takes 2^23 off.  Integer / FMA pipes only -- no I2F, which would
+// add to the XU / MIO path that bounds the tensor passes (DESIGN.md 4.1).  float32 counts pass through unchanged.
+__device__ __forceinline__ float u16_to_f32(uint32_t u) { return __uint_as_float(0x4B000000u | u) - 8388608.f; }
+__device__ __forceinline__ float count_f32(float x) { return x; }
+__device__ __forceinline__ float count_f32(uint16_t x) { return u16_to_f32(x); }
+// the count at p through the read-only cache
+template <class XT> __device__ __forceinline__ float ldg_count(const XT* p) { return count_f32(__ldg(p)); }
+// f(X) with the problem's X pointer in its storage type (const float* or const uint16_t*)
+template <class F> static inline int with_counts(const ori_problem_t* P, F&& f) {
+    return (P->flags & ORI_F_X_U16) ? f(reinterpret_cast<const uint16_t*>(P->X)) : f(P->X);
+}
+template <class Ptr> using count_t = std::remove_const_t<std::remove_pointer_t<Ptr>>;
+
 // kernels_simt.cu
 int launch_pass_rows_simt(const ori_problem_t* P, int gen_old, cudaStream_t st);
 int launch_pass_genes_simt(const ori_problem_t* P, int gen_old, cudaStream_t st);
@@ -43,8 +58,8 @@ int launch_count_stats(const ori_problem_t* P, cudaStream_t st);
 int launch_quirk_weights(const ori_problem_t* P, int gen_old, cudaStream_t st);
 int launch_dropout_posterior(const ori_problem_t* P, int gen, float* out, long long ldo,
                              long long row0, long long nrows, cudaStream_t st);
-int launch_row_sums(const float* X, long long ldx, long long n_rows, int p, float* out, cudaStream_t st);
-int launch_col_sums(const float* X, long long ldx, long long n_rows, int p, double* out, cudaStream_t st);
+template <class XT> int launch_row_sums(const XT* X, long long ldx, long long n_rows, int p, float* out, cudaStream_t st);
+template <class XT> int launch_col_sums(const XT* X, long long ldx, long long n_rows, int p, double* out, cudaStream_t st);
 int launch_deviance(const ori_problem_t* P, int gen, const double* pi, const double* col_mean, long long* out_int,
                     double* out_f64, cudaStream_t st);
 

@@ -48,9 +48,10 @@ static_assert(PR_TR == DET_SIMT_BLOCK_ROWS, "det_carve sizes the per-row-block s
 // contract with Vc = the current one.  Otherwise eVz == eV and Vc == Vh (not read).  SPARSE without DROPOUT (the
 // operator seam, D_hat folded into X): Vh and Vc are not read.
 // TG: genes per tile (32; 16 for the sparse model at KP = 64, whose four gene-side operand tiles would not fit 48 KB)
-template <int KP, bool DROPOUT, bool ELBO, bool SPARSE, int TG = PR_TG>
+// XT: element type of X (float, or uint16_t under ORI_F_X_U16)
+template <int KP, bool DROPOUT, bool ELBO, bool SPARSE, int TG, class XT>
 __global__ void __launch_bounds__(PR_TR)
-k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
+k_pass_rows(const XT* __restrict__ X, long long ldx, long long n_rows, int p,
             const float* __restrict__ eU, const float* __restrict__ Uh,
             const float* __restrict__ eV, const float* __restrict__ Vh,
             const float* __restrict__ eVz, const float* __restrict__ Vc,
@@ -96,7 +97,7 @@ k_pass_rows(const float* __restrict__ X, long long ldx, long long n_rows, int p,
         for (int rr = warp; rr < PR_TR; rr += PR_TR / 32) {
             const long long r = row0 + rr;
             float v = 0.f;
-            if (r < n_rows && lane < gcount) v = __ldg(X + r * ldx + j0 + lane);
+            if (r < n_rows && lane < gcount) v = ldg_count(X + r * ldx + j0 + lane);
             if (lane < TG) sX[rr][lane] = v;
         }
         float* sVf = &sV[0][0];
@@ -226,9 +227,9 @@ constexpr int PG_TR = 32;
 // THIRD: a third sum Zl[j,k] = sum_i R_ij eU_ik E[log U_ik] (zigap.py:95, sparse_zigap.py:116) with the sweep operand
 // eUl = eU * E[log U].  The sparse model passes eV = its masked denominator operand and Vh = the previous effective
 // V_hat (see k_pass_rows).
-template <int KP, bool DROPOUT, bool QUIRK, bool THIRD>
+template <int KP, bool DROPOUT, bool QUIRK, bool THIRD, class XT>
 __global__ void __launch_bounds__(PG_TG)
-k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
+k_pass_genes(const XT* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
              const float* __restrict__ eU, const float* __restrict__ eUw, const float* __restrict__ Uh,
              const float* __restrict__ Un, const float* __restrict__ eUl,
              const float* __restrict__ eV, const float* __restrict__ Vh,
@@ -286,7 +287,7 @@ k_pass_genes(const float* __restrict__ X, long long ldx, long long n_rows, int p
             float xs[8];
 #pragma unroll
             for (int u = 0; u < 8; ++u)
-                xs[u] = (j_ok && rb + u < rcount) ? __ldg(X + (r0 + rb + u) * ldx + j) : 0.f;
+                xs[u] = (j_ok && rb + u < rcount) ? ldg_count(X + (r0 + rb + u) * ldx + j) : 0.f;
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
                 const int rr = rb + u;
@@ -605,8 +606,9 @@ k_mstep(ori_problem_t P, int mode)
 
 // ------------------------------------------------------------------------------------------------
 // Constant statistics of X: sum lgamma(X+1), nnz, column sums of (X>0).
+template <class XT>
 __global__ void __launch_bounds__(128)
-k_count_stats(const float* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
+k_count_stats(const XT* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
               double* __restrict__ colsum, double* __restrict__ part64)
 {
     __shared__ double sred[4];
@@ -616,7 +618,7 @@ k_count_stats(const float* __restrict__ X, long long ldx, long long n_rows, int 
     double lg = 0.0; float cnt = 0.f;
     if (j < p)
         for (long long r = r0; r < r1; ++r) {
-            const float x = __ldg(X + r * ldx + j);
+            const float x = ldg_count(X + r * ldx + j);
             if (x > 0.f) { cnt += 1.f; lg += (double)lgammaf(x + 1.f); }
         }
     if (j < p && cnt != 0.f) atomicAdd(colsum + j, (double)cnt);
@@ -626,8 +628,9 @@ k_count_stats(const float* __restrict__ X, long long ldx, long long n_rows, int 
 }
 
 // eUw[i,k] = eU[i,k] * D_hat[i, gene k]   (the operand that reproduces zigap.py:94)
+template <class XT>
 __global__ void __launch_bounds__(256)
-k_quirk_weights(const float* __restrict__ X, long long ldx, long long n_rows, int K, int KP,
+k_quirk_weights(const XT* __restrict__ X, long long ldx, long long n_rows, int K, int KP,
                 const float* __restrict__ eU, const float* __restrict__ Uh, const float* __restrict__ Vh,
                 const float* __restrict__ lp, const float* __restrict__ pfloor, float* __restrict__ eUw)
 {
@@ -635,7 +638,7 @@ k_quirk_weights(const float* __restrict__ X, long long ldx, long long n_rows, in
     if (idx >= n_rows * KP) return;
     const long long i = idx / KP; const int k = (int)(idx % KP);
     if (k >= K) { eUw[idx] = 0.f; return; }
-    const float x = X[i * ldx + k];
+    const float x = count_f32(X[i * ldx + k]);
     float D = 1.f;
     if (x == 0.f) {
         float uv = 0.f;
@@ -647,8 +650,9 @@ k_quirk_weights(const float* __restrict__ X, long long ldx, long long n_rows, in
 }
 
 // D_hat slab (tests / API access to model.D_hat): zigap.py:131-136
+template <class XT>
 __global__ void __launch_bounds__(256)
-k_dropout_posterior(const float* __restrict__ X, long long ldx, int p, int K, int KP,
+k_dropout_posterior(const XT* __restrict__ X, long long ldx, int p, int K, int KP,
                     const float* __restrict__ Uh, const float* __restrict__ Vh,
                     const float* __restrict__ lp, const float* __restrict__ pfloor,
                     float* __restrict__ out, long long ldo, long long row0, long long nrows)
@@ -656,7 +660,7 @@ k_dropout_posterior(const float* __restrict__ X, long long ldx, int p, int K, in
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= nrows * p) return;
     const long long i = row0 + idx / p; const int j = (int)(idx % p);
-    const float x = X[i * ldx + j];
+    const float x = count_f32(X[i * ldx + j]);
     float D = 1.f;
     if (x == 0.f) {
         float uv = 0.f;
@@ -781,8 +785,9 @@ k_sparse_gene_update(ori_problem_t P, double* __restrict__ blk_part)
 
 // ------------------------------------------------------------------------------------------------
 // Column sums of X in float64 (column means for explained_deviance, base.py:76).
+template <class XT>
 __global__ void __launch_bounds__(128)
-k_col_sums(const float* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
+k_col_sums(const XT* __restrict__ X, long long ldx, long long n_rows, int p, int rows_per_chunk,
            double* __restrict__ out)
 {
     const int j = blockIdx.x * 128 + threadIdx.x;
@@ -790,19 +795,20 @@ k_col_sums(const float* __restrict__ X, long long ldx, long long n_rows, int p, 
     const long long r0 = (long long)blockIdx.y * rows_per_chunk;
     const long long r1 = min(n_rows, r0 + rows_per_chunk);
     double s = 0.0;
-    for (long long r = r0; r < r1; ++r) s += (double)__ldg(X + r * ldx + j);
+    for (long long r = r0; r < r1; ++r) s += (double)ldg_count(X + r * ldx + j);
     if (s != 0.0) atomicAdd(out + j, s);
 }
 
 // Row sums of X (float32): one warp per cell.
+template <class XT>
 __global__ void __launch_bounds__(256)
-k_row_sums(const float* __restrict__ X, long long ldx, long long n_rows, int p, float* __restrict__ out)
+k_row_sums(const XT* __restrict__ X, long long ldx, long long n_rows, int p, float* __restrict__ out)
 {
     const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
     if (row >= n_rows) return;
     const int lane = threadIdx.x & 31;
     float s = 0.f;
-    for (int j = lane; j < p; j += 32) s += __ldg(X + row * ldx + j);
+    for (int j = lane; j < p; j += 32) s += ldg_count(X + row * ldx + j);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
     if (lane == 0) out[row] = s;
@@ -823,9 +829,9 @@ __device__ __forceinline__ long long trunc_like_numpy(double v) {
 // table, and zero entries whose terms all truncate to 0 are skipped.
 constexpr int DEV_LOGX = 1024;
 
-template <int KP, bool EXACT>
+template <int KP, bool EXACT, class XT>
 __global__ void __launch_bounds__(PR_TR)
-k_deviance(const float* __restrict__ X, long long ldx, long long n_rows, int p,
+k_deviance(const XT* __restrict__ X, long long ldx, long long n_rows, int p,
            const float* __restrict__ Uh, const float* __restrict__ b1, const float* __restrict__ b2,
            const float* __restrict__ Sh, const float* __restrict__ Vo,
            const float* __restrict__ lp, const float* __restrict__ pfloor,
@@ -865,7 +871,7 @@ k_deviance(const float* __restrict__ X, long long ldx, long long n_rows, int p,
         for (int rr = warp; rr < PR_TR; rr += PR_TR / 32) {
             const long long r = row0 + rr;
             float v = 0.f;
-            if (r < n_rows && lane < gcount) v = __ldg(X + r * ldx + j0 + lane);
+            if (r < n_rows && lane < gcount) v = ldg_count(X + r * ldx + j0 + lane);
             sX[rr][lane] = v;
         }
         float* sVof = &sVo[0][0];
@@ -1051,18 +1057,21 @@ static int pass_rows_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     const float* eV = sparse ? P->eVd : P->eV;
     const float* Vh = sparse ? P->Vh_old : P->V_hat;
     const float* eVz = sparse ? P->eVz : P->eV;
+    with_counts(P, [&](auto X) {
 #define ORI_LAUNCH_PR(D, E, S)                                                                                  \
-    k_pass_rows<KP, D, E, S, S ? TGS : PR_TG><<<grid, PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->eU[g],   \
-        P->U_hat[g], eV, Vh, eVz, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part,                       \
-        (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,        \
-        det_cs, det_part)
-    if (sparse && drop) ORI_LAUNCH_PR(true, false, true);
-    else if (sparse) ORI_LAUNCH_PR(false, false, true);
-    else if (drop && elbo) ORI_LAUNCH_PR(true, true, false);
-    else if (drop) ORI_LAUNCH_PR(true, false, false);
-    else if (elbo) ORI_LAUNCH_PR(false, true, false);
-    else ORI_LAUNCH_PR(false, false, false);
+        k_pass_rows<KP, D, E, S, S ? TGS : PR_TG, count_t<decltype(X)>><<<grid, PR_TR, 0, st>>>(X, P->ldx,         \
+            P->n_rows, P->p, P->eU[g], P->U_hat[g], eV, Vh, eVz, P->V_hat, P->lp, P->pfloor, P->Zi, P->a2s, colsum, part, \
+            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,    \
+            det_cs, det_part)
+        if (sparse && drop) ORI_LAUNCH_PR(true, false, true);
+        else if (sparse) ORI_LAUNCH_PR(false, false, true);
+        else if (drop && elbo) ORI_LAUNCH_PR(true, true, false);
+        else if (drop) ORI_LAUNCH_PR(true, false, false);
+        else if (elbo) ORI_LAUNCH_PR(false, true, false);
+        else ORI_LAUNCH_PR(false, false, false);
 #undef ORI_LAUNCH_PR
+        return ORI_OK;
+    });
     if (check_launch("k_pass_rows") != ORI_OK) return ORI_ECUDA;
     return det_sums();
 }
@@ -1110,18 +1119,21 @@ static int pass_genes_kp(const ori_problem_t* P, int g, cudaStream_t st) {
     const bool sparse = P->flags & ORI_F_SPARSE;
     const float* eV = sparse ? P->eVd : P->eV;
     const float* Vh = sparse ? P->Vh_old : P->V_hat;
+    with_counts(P, [&](auto X) {
 #define ORI_LAUNCH_PG(D, Q, T)                                                                                  \
-    k_pass_genes<KP, D, Q, T><<<grid, PG_TG, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, P->eU[g], P->eUw, \
-        P->U_hat[g], P->U_hat[1 - g], P->eUl[g], eV, Vh, P->lp, P->pfloor, red.Zj, red.b2s, red.Zl,              \
-        (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,        \
-        det_z, det_stride)
-    if (third && drop) ORI_LAUNCH_PG(true, false, true);
-    else if (third) ORI_LAUNCH_PG(false, false, true);
-    else if (drop && quirk) ORI_LAUNCH_PG(true, true, false);
-    else if (drop) ORI_LAUNCH_PG(true, false, false);
-    else if (quirk) ORI_LAUNCH_PG(false, true, false);
-    else ORI_LAUNCH_PG(false, false, false);
+        k_pass_genes<KP, D, Q, T, count_t<decltype(X)>><<<grid, PG_TG, 0, st>>>(X, P->ldx, P->n_rows, P->p, (int)rpc, \
+            P->eU[g], P->eUw, P->U_hat[g], P->U_hat[1 - g], P->eUl[g], eV, Vh, P->lp, P->pfloor, red.Zj, red.b2s, red.Zl, \
+            (P->thrU && P->thrV) ? P->thrU + (long long)g * P->n_rows : nullptr, P->thrU ? P->thrV : nullptr,    \
+            det_z, det_stride)
+        if (third && drop) ORI_LAUNCH_PG(true, false, true);
+        else if (third) ORI_LAUNCH_PG(false, false, true);
+        else if (drop && quirk) ORI_LAUNCH_PG(true, true, false);
+        else if (drop) ORI_LAUNCH_PG(true, false, false);
+        else if (quirk) ORI_LAUNCH_PG(false, true, false);
+        else ORI_LAUNCH_PG(false, false, false);
 #undef ORI_LAUNCH_PG
+        return ORI_OK;
+    });
     if (check_launch("k_pass_genes") != ORI_OK) return ORI_ECUDA;
     return det_sums();
 }
@@ -1227,14 +1239,20 @@ int launch_count_stats(const ori_problem_t* P, cudaStream_t st) {
     const long long rpc = (P->n_rows + chunks - 1) / chunks;
     dim3 grid(bx, cdiv(P->n_rows, rpc));
     const RedBufs red = red_carve(*P);
-    k_count_stats<<<grid, 128, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, (int)rpc, red.colsum, red.part);
+    with_counts(P, [&](auto X) {
+        k_count_stats<<<grid, 128, 0, st>>>(X, P->ldx, P->n_rows, P->p, (int)rpc, red.colsum, red.part);
+        return ORI_OK;
+    });
     return check_launch("k_count_stats");
 }
 
 int launch_quirk_weights(const ori_problem_t* P, int g, cudaStream_t st) {
     const long long total = P->n_rows * P->KP;
-    k_quirk_weights<<<cdiv(total, 256), 256, 0, st>>>(P->X, P->ldx, P->n_rows, P->K, P->KP, P->eU[g],
-                                                      P->U_hat[g], P->V_hat, P->lp, P->pfloor, P->eUw);
+    with_counts(P, [&](auto X) {
+        k_quirk_weights<<<cdiv(total, 256), 256, 0, st>>>(X, P->ldx, P->n_rows, P->K, P->KP, P->eU[g],
+                                                          P->U_hat[g], P->V_hat, P->lp, P->pfloor, P->eUw);
+        return ORI_OK;
+    });
     return check_launch("k_quirk_weights");
 }
 
@@ -1242,13 +1260,17 @@ int launch_dropout_posterior(const ori_problem_t* P, int g, float* out, long lon
                              long long nrows, cudaStream_t st) {
     const long long total = nrows * P->p;
     if (total == 0) return ORI_OK;
-    k_dropout_posterior<<<cdiv(total, 256), 256, 0, st>>>(P->X, P->ldx, P->p, P->K, P->KP, P->U_hat[g],
-                                                          (P->flags & ORI_F_SPARSE) ? P->Vh_old : P->V_hat, P->lp,
-                                                          P->pfloor, out, ldo, row0, nrows);
+    with_counts(P, [&](auto X) {
+        k_dropout_posterior<<<cdiv(total, 256), 256, 0, st>>>(X, P->ldx, P->p, P->K, P->KP, P->U_hat[g],
+                                                              (P->flags & ORI_F_SPARSE) ? P->Vh_old : P->V_hat, P->lp,
+                                                              P->pfloor, out, ldo, row0, nrows);
+        return ORI_OK;
+    });
     return check_launch("k_dropout_posterior");
 }
 
-int launch_col_sums(const float* X, long long ldx, long long n_rows, int p, double* out, cudaStream_t st) {
+template <class XT>
+int launch_col_sums(const XT* X, long long ldx, long long n_rows, int p, double* out, cudaStream_t st) {
     if (n_rows == 0) return ORI_OK;
     const int bx = cdiv(p, 128);
     long long chunks = 1;
@@ -1259,11 +1281,16 @@ int launch_col_sums(const float* X, long long ldx, long long n_rows, int p, doub
     return check_launch("k_col_sums");
 }
 
-int launch_row_sums(const float* X, long long ldx, long long n_rows, int p, float* out, cudaStream_t st) {
+template <class XT>
+int launch_row_sums(const XT* X, long long ldx, long long n_rows, int p, float* out, cudaStream_t st) {
     if (n_rows == 0) return ORI_OK;
     k_row_sums<<<cdiv(n_rows, 8), 256, 0, st>>>(X, ldx, n_rows, p, out);
     return check_launch("k_row_sums");
 }
+template int launch_col_sums(const float*, long long, long long, int, double*, cudaStream_t);
+template int launch_col_sums(const uint16_t*, long long, long long, int, double*, cudaStream_t);
+template int launch_row_sums(const float*, long long, long long, int, float*, cudaStream_t);
+template int launch_row_sums(const uint16_t*, long long, long long, int, float*, cudaStream_t);
 
 template <int KP>
 static int deviance_kp(const ori_problem_t* P, int g, const double* pi, const double* cmean, long long* out_int,
@@ -1275,14 +1302,18 @@ static int deviance_kp(const ori_problem_t* P, int g, const double* pi, const do
     int gy = 1;
     while (bx * gy < 148 * 4 * 8 && gy * 2 <= ntiles) gy *= 2;
     const bool sparse = P->flags & ORI_F_SPARSE;
-    if (out_f64)
-        k_deviance<KP, true><<<dim3(bx, gy), PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->U_hat[g], P->b1, P->b2,
-            sparse ? P->p_s : nullptr, sparse ? P->Vh_old : P->V_hat, P->lp, P->pfloor, pi, cmean,
-            (unsigned long long*)out_int, out_f64);
-    else
-        k_deviance<KP, false><<<dim3(bx, gy), PR_TR, 0, st>>>(P->X, P->ldx, P->n_rows, P->p, P->U_hat[g], P->b1, P->b2,
-            sparse ? P->p_s : nullptr, sparse ? P->Vh_old : P->V_hat, P->lp, P->pfloor, pi, cmean,
-            (unsigned long long*)out_int, nullptr);
+    with_counts(P, [&](auto X) {
+        using XT = count_t<decltype(X)>;
+        if (out_f64)
+            k_deviance<KP, true, XT><<<dim3(bx, gy), PR_TR, 0, st>>>(X, P->ldx, P->n_rows, P->p, P->U_hat[g], P->b1, P->b2,
+                sparse ? P->p_s : nullptr, sparse ? P->Vh_old : P->V_hat, P->lp, P->pfloor, pi, cmean,
+                (unsigned long long*)out_int, out_f64);
+        else
+            k_deviance<KP, false, XT><<<dim3(bx, gy), PR_TR, 0, st>>>(X, P->ldx, P->n_rows, P->p, P->U_hat[g], P->b1, P->b2,
+                sparse ? P->p_s : nullptr, sparse ? P->Vh_old : P->V_hat, P->lp, P->pfloor, pi, cmean,
+                (unsigned long long*)out_int, nullptr);
+        return ORI_OK;
+    });
     return check_launch("k_deviance");
 }
 

@@ -52,7 +52,8 @@ constexpr int NCTA = 2;               // CTAs of a cluster (pair)
 // as tf32 hi plus a bf16 [hi | lo] . [lo | hi] chain for the two cross terms, like den / uv -- so every sum is fp32-grade
 // (~2^-21) instead of TF32-grade (~2^-12 per term).  The tile keeps R16 / D16 (the packed bf16 pairs) beside R / D in TMEM,
 // which halves the sweep width (32) to stay inside 512 columns.
-template <int KP, bool PRECISE = false, bool DEVI = false>
+// XB: bytes per count of X (4: float32; 2: uint16, ORI_F_X_U16) -- only the X ring's stages change size.
+template <int KP, bool PRECISE = false, bool DEVI = false, int XB = 4>
 struct Cfg {
     static_assert(KP == 32 || KP == 64, "tensor path: KP is 32 or 64");
     static_assert(!PRECISE || KP == 32, "the fp32-grade plan exists for KP = 32");
@@ -69,7 +70,7 @@ struct Cfg {
     static constexpr uint32_t T_CHUNK = (KP / NCTA) * 128;
     static constexpr uint32_t T_ARR = (SW / 32) * T_CHUNK;
     static constexpr uint32_t T_STAGE = NTA * T_ARR;      // transposed e and transposed E (+ their bf16 [lo | hi] pairs)
-    static constexpr uint32_t X_STAGE = TC_OWN * SW * 4;  // X tile
+    static constexpr uint32_t X_STAGE = TC_OWN * SW * XB; // X tile
     // per-gene constants of a tile: lp2[SW] | floor[SW] | (1-pi)/pi [SW]; deviance pass: 8 arrays (k_tc_prep_dev)
     static constexpr uint32_t LP_STAGE = (DEVI ? 8 : 3) * SW * 4;
     static constexpr uint32_t OFF_K = 0;
@@ -151,6 +152,23 @@ __device__ __forceinline__ float lds32(uint32_t a) {
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
     return v;
 }
+// two biased counts (0x4B000000 | u, see u16_to_f32) -> their float32 values with one packed add (add.f32x2)
+__device__ __forceinline__ void unbias2(uint32_t b0, uint32_t b1, float& f0, float& f1) {
+    uint32_t r0, r1;
+    asm("{\n\t.reg .b64 t, c, d;\n\tmov.b64 t, {%2, %3};\n\tmov.b64 c, {%4, %4};\n\tadd.rn.f32x2 d, t, c;\n\t"
+        "mov.b64 {%0, %1}, d;\n\t}" : "=r"(r0), "=r"(r1) : "r"(b0), "r"(b1), "r"(0xCB000000u));
+    f0 = __uint_as_float(r0); f1 = __uint_as_float(r1);
+}
+__device__ __forceinline__ uint4 lds128u(uint32_t a) {
+    uint4 v;
+    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ uint32_t lds16(uint32_t a) {
+    uint16_t v;
+    asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(a));
+    return v;
+}
 // x != 0 ? a : b, twice with differently spelled tests: each predicate dies at its select, so sixteen of them
 // never have to be parked in a bit mask across the MUFU latency
 __device__ __forceinline__ float sel_nz_a(float x, float a, float b) {
@@ -210,11 +228,17 @@ struct TileIter {
 // loop cost the plain kernels 7 % (row pass) / 3 % (gene pass) when the hooks were runtime-switched.
 // DET: the ORI_F_DETERMINISTIC epilogue (TcArgs::tickets / item_part), a separate instantiation for the same reason (runtime-
 // switched it cost the plain kernels 2.6 % / 3.4 %).
-template <bool GENES, bool DROPOUT, bool ELBO, int KP, bool PRECISE, bool DEVI = false, bool UFL = false, bool DET = false>
+// XT: element type of X -- float, or uint16_t (ORI_F_X_U16: half the X bytes per tile, widened exactly as it is read
+// from shared memory; row pass: one [128 cells][SW genes] box per tile, 128- or 64-byte swizzled rows; gene pass:
+// [SW cells][32 genes] boxes of 64-byte rows, 64-byte swizzle).
+template <bool GENES, bool DROPOUT, bool ELBO, int KP, bool PRECISE, bool DEVI = false, bool UFL = false, bool DET = false,
+          class XT = float>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
 {
-    using C = Cfg<KP, PRECISE, DEVI>;
+    constexpr int XB = (int)sizeof(XT);
+    constexpr bool U16 = XB == 2;
+    using C = Cfg<KP, PRECISE, DEVI, XB>;
     static_assert(!DEVI || (!GENES && DROPOUT && !ELBO && !PRECISE), "deviance pass: row orientation, two contractions");
     constexpr int SW = C::SW, NS = C::NS;
     constexpr uint32_t TM_UV = C::TM_UV;
@@ -319,10 +343,14 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     const int sw0 = ik.t * SW;
                     mbar_expect_tx(bar, X_STAGE + ((!GENES && DROPOUT) ? LP_STAGE : 0));
                     if (DEVI) bulk_load(smem + OFF_LP + s * LP_STAGE, a.devlp + (long long)ik.t * (8 * SW), LP_STAGE, bar);
-                    if (!GENES) {          // [128 cells][32 genes] boxes
+                    if (!GENES) {          // [128 cells][32 genes] boxes (uint16: one [128 cells][SW genes] box)
+                        if constexpr (U16) {
+                            tma_load_2d_hint(st, &maps.X, bar, sw0, ik.own0, L2_EVICT_FIRST);
+                        } else {
 #pragma unroll
-                        for (int c = 0; c < SW / 32; ++c)
-                            tma_load_2d_hint(st + c * (TC_OWN * 128), &maps.X, bar, sw0 + 32 * c, ik.own0, L2_EVICT_FIRST);
+                            for (int c = 0; c < SW / 32; ++c)
+                                tma_load_2d_hint(st + c * (TC_OWN * 128), &maps.X, bar, sw0 + 32 * c, ik.own0, L2_EVICT_FIRST);
+                        }
                         if (DROPOUT && !DEVI) {
                             bulk_load(smem + OFF_LP + s * LP_STAGE, a.lp2w + sw0, SW * 4, bar);
                             bulk_load(smem + OFF_LP + s * LP_STAGE + SW * 4, a.flw + sw0, SW * 4, bar);
@@ -331,7 +359,7 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
                     } else {               // [SW cells][32 genes] boxes, one per TMEM lane quarter
 #pragma unroll
                         for (int c = 0; c < 4; ++c)
-                            tma_load_2d_hint(st + c * (SW * 128), &maps.X, bar, ik.own0 + 32 * c, sw0, L2_EVICT_FIRST);
+                            tma_load_2d_hint(st + c * (SW * 32 * XB), &maps.X, bar, ik.own0 + 32 * c, sw0, L2_EVICT_FIRST);
                     }
                 }
                 __syncwarp();
@@ -510,10 +538,13 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             if (lane == 0) mbar_arrive_cluster(&bars[B_A_READY], 0);
         };
 
-        // gene pass: X is staged [cell][gene]; lane (gene) reads one float per cell, 128-byte swizzle undone here
-        uint32_t xoff[8];
+        // gene pass: X is staged [cell][gene]; lane (gene) reads one count per cell, the swizzle undone here (float32:
+        // 128-byte rows, chunk ^ (cell & 7); uint16: 64-byte rows, chunk ^ ((cell >> 1) & 3))
+        uint32_t xoff[U16 ? 4 : 8];
 #pragma unroll
-        for (int k = 0; k < 8; ++k) xoff[k] = (uint32_t)(quarter * (SW * 128) + ((((lane >> 2) ^ k)) << 4) + (lane & 3) * 4);
+        for (int k = 0; k < (U16 ? 4 : 8); ++k)
+            xoff[k] = U16 ? (uint32_t)(quarter * (SW * 64) + (((lane >> 3) ^ k) << 4) + (lane & 7) * 2)
+                          : (uint32_t)(quarter * (SW * 128) + ((((lane >> 2) ^ k)) << 4) + (lane & 3) * 4);
 
         TileIter ti;
         ti.init(a, NCTA, rank);
@@ -589,12 +620,36 @@ k_tc_pass(const __grid_constant__ TcMaps maps, const TcArgs a)
             auto load_x = [&](const Tile& c, int g, int b) {
                 const int c0 = colbase + g * 16;
                 if (!GENES) {
-                    const uint32_t base = c.xs_addr + (c0 >> 5) * (TC_OWN * 128) + lrow * 128;
-                    const int cb = (c0 & 31) >> 2;
+                    if constexpr (U16) {
+                        // row of SW counts = 128 bytes (SW = 64, 128-byte swizzle) or 64 bytes (SW = 32, 64-byte swizzle);
+                        // the 16 counts of the group are two 16-byte chunks
+                        constexpr int RB = SW * 2;
+                        const uint32_t base = c.xs_addr + lrow * RB;
+                        const int sw = RB == 128 ? (lrow & 7) : ((lrow >> 1) & 3);
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const float4 v = lds128(base + (((cb + q) ^ (lrow & 7)) << 4));
-                        x[b][4 * q] = v.x; x[b][4 * q + 1] = v.y; x[b][4 * q + 2] = v.z; x[b][4 * q + 3] = v.w;
+                        for (int q = 0; q < 2; ++q) {
+                            const uint4 w = lds128u(base + ((((c0 >> 3) + q) ^ sw) << 4));
+                            const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+                            for (int h = 0; h < 4; ++h)
+                                unbias2(__byte_perm(ws[h], 0x4B000000u, 0x7610), __byte_perm(ws[h], 0x4B000000u, 0x7632),
+                                        x[b][8 * q + 2 * h], x[b][8 * q + 2 * h + 1]);
+                        }
+                    } else {
+                        const uint32_t base = c.xs_addr + (c0 >> 5) * (TC_OWN * 128) + lrow * 128;
+                        const int cb = (c0 & 31) >> 2;
+#pragma unroll
+                        for (int q = 0; q < 4; ++q) {
+                            const float4 v = lds128(base + (((cb + q) ^ (lrow & 7)) << 4));
+                            x[b][4 * q] = v.x; x[b][4 * q + 1] = v.y; x[b][4 * q + 2] = v.z; x[b][4 * q + 3] = v.w;
+                        }
+                    }
+                } else if constexpr (U16) {
+#pragma unroll
+                    for (int e = 0; e < 16; e += 2) {
+                        const int i = c0 + e;
+                        unbias2(0x4B000000u | lds16(c.xs_addr + xoff[(i >> 1) & 3] + i * 64),
+                                0x4B000000u | lds16(c.xs_addr + xoff[((i + 1) >> 1) & 3] + (i + 1) * 64), x[b][e], x[b][e + 1]);
                     }
                 } else {
 #pragma unroll
@@ -1247,10 +1302,10 @@ static void tc_partition(TcArgs& a, bool genes, int units, int sw, bool precise,
     a.n_items = a.n_own_units * a.n_chunks;
 }
 
-template <bool GENES, bool D, bool E, int KP, bool PRECISE, bool DEVI, bool UFL, bool DET>
+template <bool GENES, bool D, bool E, int KP, bool PRECISE, bool DEVI, bool UFL, bool DET, class XT>
 static int launch_tc_variant(const TcMaps& maps, const TcArgs& a, int grid, cudaStream_t st) {
-    auto kern = k_tc_pass<GENES, D, E, KP, PRECISE, DEVI, UFL, DET>;
-    constexpr uint32_t smem = Cfg<KP, PRECISE, DEVI>::SMEM_BYTES;
+    auto kern = k_tc_pass<GENES, D, E, KP, PRECISE, DEVI, UFL, DET, XT>;
+    constexpr uint32_t smem = Cfg<KP, PRECISE, DEVI, (int)sizeof(XT)>::SMEM_BYTES;
     static bool attr_done = false;
     if (!attr_done) {
         cudaError_t e_ = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
@@ -1269,12 +1324,21 @@ static int launch_tc_variant(const TcMaps& maps, const TcArgs& a, int grid, cuda
 }
 
 // the instance of a pass for its (dropout, ELBO) flags
-template <bool GENES, int KP, bool PRECISE, bool UFL, bool DET>
+template <bool GENES, int KP, bool PRECISE, bool UFL, bool DET, class XT>
 static int launch_tc_flags(bool drop, bool elbo, const TcMaps& maps, const TcArgs& a, int grid, cudaStream_t st) {
-    if (drop && elbo) return launch_tc_variant<GENES, true, true, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
-    if (drop) return launch_tc_variant<GENES, true, false, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
-    if (elbo) return launch_tc_variant<GENES, false, true, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
-    return launch_tc_variant<GENES, false, false, KP, PRECISE, false, UFL, DET>(maps, a, grid, st);
+    if (drop && elbo) return launch_tc_variant<GENES, true, true, KP, PRECISE, false, UFL, DET, XT>(maps, a, grid, st);
+    if (drop) return launch_tc_variant<GENES, true, false, KP, PRECISE, false, UFL, DET, XT>(maps, a, grid, st);
+    if (elbo) return launch_tc_variant<GENES, false, true, KP, PRECISE, false, UFL, DET, XT>(maps, a, grid, st);
+    return launch_tc_variant<GENES, false, false, KP, PRECISE, false, UFL, DET, XT>(maps, a, grid, st);
+}
+
+// X's tensor map: float32 [128 cells][32 genes] / [SW cells][32 genes] boxes (128-byte rows); uint16 (ORI_F_X_U16)
+// [128 cells][SW genes] in the row orientation (one box per tile), [SW cells][32 genes] in the gene orientation
+static bool make_x_map(CUtensorMap* map, const ori_problem_t* P, bool genes, int SW) {
+    if (P->flags & ORI_F_X_U16)
+        return make_tmap_u16(map, reinterpret_cast<const uint16_t*>(P->X), P->n_rows, P->p, P->ldx, genes ? 32 : SW,
+                             genes ? SW : TC_OWN);
+    return make_tmap_f32(map, P->X, P->n_rows, P->p, P->ldx, 32, genes ? SW : TC_OWN);
 }
 
 // logsum: the dropout-free sweep of the sparse model's third gene-side sum into red32 block 2
@@ -1294,14 +1358,14 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
     if (!GENES) {
         ok = make_tmap_f32(&maps.swK, w.geneK, 4 * w.pp, KP, KP, 32, SW / NCTA) &&
              make_tmap_f32(&maps.swT, w.geneT, C::NTA * KP, w.pp, w.pp, 32, KP / NCTA) &&
-             make_tmap_f32(&maps.X, P->X, P->n_rows, P->p, P->ldx, 32, TC_OWN);
+             make_x_map(&maps.X, P, false, SW);
         a.own_total = P->n_rows; a.sw_total = P->p; a.sw_pad = w.pp;
         a.own_e = P->eU[gen_old]; a.own_E = P->U_hat[gen_old];
         a.acc1 = P->Zi; a.acc2 = P->a2s;
     } else {
         ok = make_tmap_f32(&maps.swK, w.rowK, 4 * w.np, KP, KP, 32, SW / NCTA) &&
              make_tmap_f32(&maps.swT, w.rowT, C::NTA * KP, w.np, w.np, 32, KP / NCTA) &&
-             make_tmap_f32(&maps.X, P->X, P->n_rows, P->p, P->ldx, 32, SW);
+             make_x_map(&maps.X, P, true, SW);
         a.own_total = P->p; a.sw_total = P->n_rows; a.sw_pad = w.np;
         a.own_e = sparse ? P->eVd : P->eV; a.own_E = sparse ? P->Vh_old : P->V_hat;
         a.acc1 = logsum ? red.Zl : red.Zj; a.acc2 = red.b2s;
@@ -1341,9 +1405,12 @@ static int launch_tc_pass_p(const ori_problem_t* P, int gen_old, cudaStream_t st
             if (e_ != cudaSuccess) return set_error(ORI_ECUDA, "cudaMemsetAsync(item_part): %s", cudaGetErrorString(e_));
         }
     }
-    const int rc = det ? launch_tc_flags<GENES, KP, PRECISE, false, true>(drop, elbo, maps, a, grid, st)
-                 : ufl ? launch_tc_flags<GENES, KP, PRECISE, true, false>(drop, elbo, maps, a, grid, st)
-                       : launch_tc_flags<GENES, KP, PRECISE, false, false>(drop, elbo, maps, a, grid, st);
+    const int rc = with_counts(P, [&](auto X) {
+        using XT = count_t<decltype(X)>;
+        return det ? launch_tc_flags<GENES, KP, PRECISE, false, true, XT>(drop, elbo, maps, a, grid, st)
+             : ufl ? launch_tc_flags<GENES, KP, PRECISE, true, false, XT>(drop, elbo, maps, a, grid, st)
+                   : launch_tc_flags<GENES, KP, PRECISE, false, false, XT>(drop, elbo, maps, a, grid, st);
+    });
     if (rc != ORI_OK) return rc;
     int extra = 0;
     if (det && GENES && drop) { k_det_add<<<cdiv(P->p, 256), 256, 0, st>>>(red.colsum, a.colsum2, P->p); ++extra; }
@@ -1387,7 +1454,7 @@ static int launch_deviance_tc_kp(const ori_problem_t* P, int g, const double* pi
     memset(&a, 0, sizeof(a));
     const bool ok = make_tmap_f32(&maps.swK, w.geneK, 4 * w.pp, KP, KP, 32, SW / NCTA) &&
                     make_tmap_f32(&maps.swT, w.geneT, C::NTA * KP, w.pp, w.pp, 32, KP / NCTA) &&
-                    make_tmap_f32(&maps.X, P->X, P->n_rows, P->p, P->ldx, 32, TC_OWN);
+                    make_x_map(&maps.X, P, false, SW);
     if (!ok) return set_error(ORI_ECUDA, "cuTensorMapEncodeTiled failed");
     a.own_total = P->n_rows; a.sw_total = P->p; a.sw_pad = w.pp;
     a.own_e = P->U_hat[g]; a.own_E = P->U_hat[g];
@@ -1406,7 +1473,9 @@ static int launch_deviance_tc_kp(const ori_problem_t* P, int g, const double* pi
     a.n_chunks = cdiv(a.n_sw_tiles, a.tiles_per_chunk);
     a.n_items = a.n_own_units * a.n_chunks;
     const int grid = NCTA * (a.n_items < units ? a.n_items : units);
-    const int rc = launch_tc_variant<false, true, false, KP, false, true, false, false>(maps, a, grid, st);
+    const int rc = with_counts(P, [&](auto X) {
+        return launch_tc_variant<false, true, false, KP, false, true, false, false, count_t<decltype(X)>>(maps, a, grid, st);
+    });
     if (rc != ORI_OK) return rc;
     return check_launch("k_tc_pass(deviance)");
 }

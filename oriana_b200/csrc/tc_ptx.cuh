@@ -280,4 +280,19 @@ inline bool make_tmap_f32(CUtensorMap* map, const float* base, uint64_t rows, ui
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// uint16 row-major [rows x cols] (counts stored as uint16, ORI_F_X_U16); box = box_cols x box_rows with box_cols * 2 = 128
+// bytes (128-byte swizzle) or 64 bytes (64-byte swizzle).  Out-of-bounds elements are filled with zeros.
+inline bool make_tmap_u16(CUtensorMap* map, const uint16_t* base, uint64_t rows, uint64_t cols, uint64_t ld,
+                          uint32_t box_cols, uint32_t box_rows) {
+    EncodeTiledFn fn = get_encode_fn();
+    if (!fn) return false;
+    cuuint64_t dims[2] = {cols, rows};
+    cuuint64_t strides[1] = {ld * sizeof(uint16_t)};
+    cuuint32_t box[2] = {box_cols, box_rows};
+    cuuint32_t estr[2] = {1, 1};
+    return fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, (void*)base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+              box_cols * 2 == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 }  // namespace tc

@@ -23,6 +23,7 @@ import numpy as np
 import torch
 
 from .. import _lib
+from .. import problem as _problem
 from ..dims import Dimensions
 from ..nodes import Einsum
 from ..parameters import Parameter
@@ -70,6 +71,7 @@ class FactorModel(metaclass=ABCMeta):
 
     _dropout = False     # ZIGaP sets this
     _sparse = False      # SparseZIGaP sets this
+    _X_SLAB_ENTRIES = 1 << 25   # matrix entries per row slab of the metrics and of the uint16 NMF warm start
 
     def __init__(self, cmatrix, k=2, use_factors=True, *, state=None, compat_quirk=False, sharded=False,
                  process_group=None, elbo=True, trace_cap=4096, force_simt=False, tensor=None, nmf=None, graphs=False,
@@ -154,18 +156,23 @@ class FactorModel(metaclass=ABCMeta):
         dev, n, p, K, KP = self._dev, self.n, self.p, self.k, self._KP
         f32 = dict(dtype=torch.float32, device=dev)
         f64 = dict(dtype=torch.float64, device=dev)
-        ldx = row_pitch(p)
+        # counts handed in as uint16 stay uint16 in HBM (ORI_F_X_U16, half the bytes) when float32 would not fit the device
+        u16 = _problem.counts_storage(cmatrix.is_uint16(), n, p, KP, torch.cuda.mem_get_info(dev)[0]) == torch.uint16
+        xdt, esz = (torch.uint16, 2) if u16 else (torch.float32, 4)
+        if u16:
+            self._flags |= _lib.ORI_F_X_U16
+        ldx = row_pitch(p, esz)
         src = cmatrix.as_tensor()
-        if isinstance(src, torch.Tensor) and src.is_cuda and src.dtype == torch.float32 \
-                and src.shape[1] == p and src.stride(1) == 1 and src.stride(0) % 4 == 0 \
+        if isinstance(src, torch.Tensor) and src.is_cuda and src.dtype == xdt \
+                and src.shape[1] == p and src.stride(1) == 1 and src.stride(0) % (16 // esz) == 0 \
                 and src.stride(0) >= p and src.data_ptr() % 16 == 0:
             self._X = src                      # adopt a resident row block without copying it
             ldx = src.stride(0) if n > 1 else max(ldx, src.stride(0))
             self._Xfull = None
         else:
-            # ingest (cmatrix.py -> HBM): slabs cross PCIe in the narrowest integer type that holds the counts and are
-            # widened on the device; no n x p float32 copy on the host
-            self._X = cmatrix.to_device(dev)
+            # ingest (cmatrix.py -> HBM): float32 storage: slabs cross PCIe in the narrowest integer type that holds the
+            # counts and are widened on the device; no n x p float32 copy on the host.  uint16 storage: copied as is
+            self._X = cmatrix.to_device(dev, dtype=xdt)
             self._Xfull = self._X
         self._ldx = ldx
 
@@ -187,8 +194,7 @@ class FactorModel(metaclass=ABCMeta):
         if self._flags & _lib.ORI_F_ELBO:
             self._xrow = torch.zeros((max(n, 1),), **f32)
             cs = torch.zeros((p,), **f64)
-            _lib.check(self._lib.ori_row_sums_f32(self._X.data_ptr(), ldx, n, p, self._xrow.data_ptr(), _lib.stream_ptr()))
-            _lib.check(self._lib.ori_column_sums_f64(self._X.data_ptr(), ldx, n, p, cs.data_ptr(), _lib.stream_ptr()))
+            self._x_sums(cs, rows=self._xrow)
             xcol = self._shard.allreduce_sum(cs).to(torch.float32)
         under = self.emulate_underflow
         # every array the problem points at: this dict owns the memory of those the model has no name for
@@ -215,6 +221,38 @@ class FactorModel(metaclass=ABCMeta):
         self.alpha2 = DeviceView(self, lambda: self._hyper[1])
         self.beta1 = DeviceView(self, lambda: self._hyper[2])
         self.beta2 = DeviceView(self, lambda: self._hyper[3])
+
+    @property
+    def counts_dtype(self):
+        """Storage of the count matrix in HBM: torch.uint16 for counts handed in as uint16, torch.float32 otherwise."""
+        return torch.uint16 if self._flags & _lib.ORI_F_X_U16 else torch.float32
+
+    def _x_sums(self, cols, rows=None):
+        """Column sums (float64) of this rank's X into `cols` and, given `rows`, its row sums (float32), by the entry
+        points of X's storage type."""
+        u16 = bool(self._flags & _lib.ORI_F_X_U16)
+        args = (self._X.data_ptr(), self._ldx, self.n, self.p)
+        if rows is not None:
+            fn = self._lib.ori_row_sums_u16_f32 if u16 else self._lib.ori_row_sums_f32
+            _lib.check(fn(*args, rows.data_ptr(), _lib.stream_ptr()))
+        fn = self._lib.ori_column_sums_u16_f64 if u16 else self._lib.ori_column_sums_f64
+        _lib.check(fn(*args, cols.data_ptr(), _lib.stream_ptr()))
+
+    def _x_slabs(self, rows):
+        """(first row, float32 [r, p] block) over this rank's X.  float32 storage: views of X, `rows` ignored (one block).
+        uint16 storage: slabs of at most `rows` cells widened by `ori_widen_counts_f32` into one float32 scratch that
+        every slab reuses -- the whole matrix is never widened at once."""
+        if not self._flags & _lib.ORI_F_X_U16:
+            yield 0, self._X
+            return
+        rows = max(1, min(int(rows), self.n))
+        ldw = row_pitch(self.p)
+        scratch = torch.empty((rows, ldw), dtype=torch.float32, device=self._dev)
+        for r in range(0, self.n, rows):
+            nr = min(rows, self.n - r)
+            _lib.check(self._lib.ori_widen_counts_f32(self._X[r:].data_ptr(), 2, self._ldx, scratch.data_ptr(), ldw, nr,
+                                                      self.p, _lib.stream_ptr()))
+            yield r, scratch[:nr, :self.p]
 
     def _extra_fields(self, rowf, genef):
         """Hook for model-specific device state (SparseZIGaP): further `ori_problem_t` fields by name."""
@@ -249,18 +287,23 @@ class FactorModel(metaclass=ABCMeta):
         over ranks.  Initialisation as sklearn's `init='random'`: sqrt(mean(X) / k) * |N(0, 1)|, seeded from
         `np.random` (rank 0's gene factors are broadcast).  Initialisation only: not part of the CAVI iteration."""
         dev, k = self._dev, self.k
-        X = self._X
+        slab = max(1, self._X_SLAB_ENTRIES // max(1, self.p))     # uint16 X: GEMMs over bounded float32 slabs
         gen = torch.Generator(device=dev)
         gen.manual_seed(int(np.random.randint(0, 2 ** 31 - 1)))
-        tot = self._shard.allreduce_sum(X.sum(dtype=torch.float64).reshape(1))[0]
+        tot = sum(X.sum(dtype=torch.float64) for _, X in self._x_slabs(slab))
+        tot = self._shard.allreduce_sum(torch.as_tensor(tot, dtype=torch.float64, device=dev).reshape(1))[0]
         scale = float(torch.sqrt(tot / (float(self.n_total) * self.p * k)).item()) or 1.0
         U = scale * torch.randn((self.n, k), device=dev, generator=gen).abs_()
         V = scale * torch.randn((self.p, k), device=dev, generator=gen).abs_()
         self._shard.broadcast(V)
         for _ in range(iters):
             VtV = V.T @ V
-            U *= (X @ V) / (U @ VtV + eps)
-            XtU = self._shard.allreduce_sum(X.T @ U)
+            XtU = None
+            for r, X in self._x_slabs(slab):
+                Ur = U[r:r + X.shape[0]]
+                Ur *= (X @ V) / (Ur @ VtV + eps)
+                XtU = X.T @ Ur if XtU is None else XtU + X.T @ Ur
+            XtU = self._shard.allreduce_sum(V.new_zeros(V.shape) if XtU is None else XtU)
             UtU = self._shard.allreduce_sum(U.T @ U)
             V *= XtU / (V @ UtU + eps)
         return U, V
@@ -537,10 +580,11 @@ class FactorModel(metaclass=ABCMeta):
         """base.py:84-87, evaluated in row slabs on the device (no n x p float64 temporary)."""
         tot = torch.zeros((), dtype=torch.float64, device=self._dev)
         U = self._Uhat[self._gen][:, :self.k]; V = self._Vhat[:, :self.k]
-        step = max(1, (1 << 25) // max(1, self.p))
-        for r in range(0, self.n, step):
-            d = (U[r:r + step] @ V.T) - self._X[r:r + step]
-            tot += (d.double() ** 2).sum()
+        step = max(1, self._X_SLAB_ENTRIES // max(1, self.p))
+        for r0, X in self._x_slabs(step):
+            for r in range(r0, r0 + X.shape[0], step):
+                d = (U[r:r + step] @ V.T) - X[r - r0:r - r0 + step]
+                tot += (d.double() ** 2).sum()
         tot = self._shard.allreduce_sum(tot.reshape(1))[0]
         return float(torch.sqrt(tot).item())
 
@@ -557,7 +601,14 @@ class FactorModel(metaclass=ABCMeta):
         self.V.buffer = self._Vhat[:, :self.k].double()
         self.UV.forward()
         try:
-            local = torch.tensor([self.U.loglikelihood() + x_ll()], dtype=torch.float64, device=self._dev)
+            if self._flags & _lib.ORI_F_X_U16:
+                # the Poisson terms of uint16 counts, slab by slab from a float32 widening (the node's own formula)
+                uv, xl = self.UV.tensor, 0.
+                for r, X in self._x_slabs(max(1, self._X_SLAB_ENTRIES // max(1, self.p))):
+                    xl += float(torch.nan_to_num(self.X._logp(X, uv[r:r + X.shape[0]])).sum().item())
+            else:
+                xl = x_ll()
+            local = torch.tensor([self.U.loglikelihood() + xl], dtype=torch.float64, device=self._dev)
         finally:
             self.UV._t = None
         return float(self._shard.allreduce_sum(local)[0].item()) + self.V.loglikelihood()

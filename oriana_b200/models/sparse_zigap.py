@@ -139,8 +139,7 @@ class SparseZIGaP(ZIGaP):
         dev = self._dev
         if self._col_mean is None:
             cs = torch.zeros((self.p,), dtype=torch.float64, device=dev)
-            _lib.check(self._lib.ori_column_sums_f64(self._X.data_ptr(), self._ldx, self.n, self.p, cs.data_ptr(),
-                                                     _lib.stream_ptr()))
+            self._x_sums(cs)
             self._shard.allreduce_sum(cs)
             self._col_mean = cs / float(self.n_total)
         out_i = torch.zeros((3,), dtype=torch.int64, device=dev)

@@ -7,9 +7,23 @@ import torch
 from . import _lib
 
 
-def row_pitch(p):
-    """Floats per row of X in HBM: p rounded up to 4, the 16-byte row pitch the kernels read."""
-    return (p + 3) // 4 * 4
+def row_pitch(p, elem_size=4):
+    """Elements per row of X in HBM: p rounded up to the 16-byte row pitch the kernels read (4 float32 counts, 8 uint16)."""
+    q = 16 // elem_size
+    return (p + q - 1) // q * q
+
+
+def counts_storage(uint16_counts, n, p, KP, free_bytes):
+    """Storage of an [n, p] count matrix in HBM: torch.uint16 (ORI_F_X_U16, half the bytes) or torch.float32.
+
+    Counts that came as uint16 stay uint16 only when the float32 matrix and the rest of the model's device state (row
+    factors, workspaces: about 4 * KP * (20 n + 16 p) bytes) would not fit `free_bytes`.  The uint16 passes are up to 11 %
+    slower than the float32 ones (profiles/r3_u16_counts.json), so uint16 storage serves problems it makes fit on the
+    device -- config 5 on one B200 -- and every problem that fits as float32 keeps the float32 passes."""
+    if not uint16_counts:
+        return torch.float32
+    need = n * row_pitch(p) * 4 + 4 * KP * (20 * n + 16 * p)
+    return torch.uint16 if need > free_bytes else torch.float32
 
 
 def pad_k(K):

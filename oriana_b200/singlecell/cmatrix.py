@@ -8,9 +8,9 @@ labels are kept beside them, so that the label-based calls (`cm['gene']`, `filte
 behave like the reference's without a pandas round trip of the matrix.
 
 Ingest helpers with no counterpart in the reference: `row_block` (the contiguous cell range a rank owns, SURVEY.md
-8e), `to_device` (float32 matrix in HBM with the 16-byte row pitch the kernels want, uploaded in slabs and widened on
-the device from the narrowest integer type that holds the counts), `to_compact` (saturating uint8 + escape list for
-host-streamed runs).
+8e), `to_device` (the matrix in HBM with the 16-byte row pitch the kernels want, uploaded in slabs: float32, widened on
+the device from the narrowest integer type that holds the counts, or uint16 as it is for counts handed in as uint16),
+`to_compact` (saturating uint8 + escape list for host-streamed runs).
 """
 import numpy as np
 import torch
@@ -129,6 +129,12 @@ class CountMatrix:
         return CountMatrix(self._data[r0:r1], row_names=None if self._rows is None else self._rows[r0:r1],
                            col_names=self._cols)
 
+    def is_uint16(self):
+        """True when the counts are a uint16 array or tensor: the device models may then keep them as uint16 in HBM
+        (`oriana_b200.problem.counts_storage`)."""
+        dt = self._data.dtype
+        return dt == torch.uint16 if isinstance(self._data, torch.Tensor) else dt == np.uint16
+
     def narrow_dtype(self):
         """Narrowest unsigned integer type that holds every count (None: the counts are not non-negative integers
         below 2^16, keep float32)."""
@@ -147,20 +153,41 @@ class CountMatrix:
             return None
         return torch.uint8 if hi < 256 else torch.uint16
 
-    def to_device(self, device='cuda', slab_rows=None):
-        """float32 [n, p] view of a [n, ldx] device buffer (ldx = p rounded up to 4: the kernels' row pitch), filled
-        slab by slab; integer counts cross PCIe in their narrow type and are widened by `ori_widen_counts_f32`."""
+    def to_device(self, device='cuda', slab_rows=None, dtype=torch.float32):
+        """[n, p] view of a [n, ldx] device buffer (ldx: the kernels' 16-byte row pitch), filled slab by slab.
+        dtype=torch.float32: integer counts cross PCIe in their narrow type and are widened by `ori_widen_counts_f32`.
+        dtype=torch.uint16 (counts that are uint16 already): the slabs are copied into the padded pitch as they are."""
         from .. import _lib
         from ..problem import row_pitch
         lib = _lib.load()
         dev = torch.device(device)
         n, p = self.shape
+        if dtype == torch.uint16:
+            if not self.is_uint16():
+                raise TypeError('to_device(dtype=torch.uint16) needs uint16 counts, got %s' % self._data.dtype)
+            # the copies go through int16 views: same bits, and every copy kernel handles int16
+            out = torch.zeros((n, row_pitch(p, 2)), dtype=torch.int16, device=dev)
+            step = slab_rows or max(1, (1 << 27) // max(1, p))
+            for r in range(0, n, step):
+                blk = self._data[r:r + step]
+                blk = blk if isinstance(blk, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(blk))
+                out[r:r + step, :p].copy_(blk.view(torch.int16))
+            return out.view(torch.uint16)[:, :p]
+        if dtype != torch.float32:
+            raise TypeError('to_device stores counts as float32 or uint16, not %s' % dtype)
         ldx = row_pitch(p)
         out = torch.zeros((n, ldx), dtype=torch.float32, device=dev)
         if isinstance(self._data, torch.Tensor) and self._data.is_cuda:
-            out[:, :p] = self._data.to(torch.float32)
+            if self.is_uint16():           # torch has no uint16 arithmetic: the library widens it
+                src = self._data if self._data.stride(1) == 1 else self._data.contiguous()
+                if n:
+                    _lib.check(lib.ori_widen_counts_f32(src.data_ptr(), 2, max(src.stride(0), p), out.data_ptr(), ldx, n, p,
+                                                        _lib.stream_ptr()))
+            else:
+                out[:, :p] = self._data.to(torch.float32)
             return out[:, :p]
-        nd = self.narrow_dtype()
+        # uint16 torch tensors cross as they are (every count fits; torch cannot scan them for a narrower type)
+        nd = torch.uint16 if isinstance(self._data, torch.Tensor) and self.is_uint16() else self.narrow_dtype()
         step = slab_rows or max(1, (1 << 26) // max(1, p))
         for r in range(0, n, step):
             blk = self._data[r:r + step]
