@@ -347,6 +347,21 @@ int ori_expand_bitmap_counts_f32(const uint32_t* bitmap, int64_t words_per_row, 
                                  const int64_t* rowoff, int64_t base, float* dst, int64_t ldd, int64_t rows,
                                  int32_t p, void* stream);
 
+/* CSR ingest, the device side of cmatrix.py:39-54 (as_sparse_matrix): rows [0, rows) of a CSR slab into a dense
+ * [rows x ldd] matrix.  Row r's non-zeros are [indptr[r] - base, indptr[r + 1] - base) of indices / values (device
+ * pointers; base = indptr of the slab's first row, so a slab cut from the middle of a matrix needs no rebasing).  The
+ * indices of a row are distinct (canonical CSR): idx_bytes = 2 (uint16, p <= 65536) or 4 (int32).  values: ORI_CSR_U8,
+ * ORI_CSR_U16 or ORI_CSR_F32 (the value type's size in bytes).  dst: dst_bytes = 4 (float32 X) or 2 (uint16 X, the
+ * ORI_F_X_U16 storage; ORI_CSR_F32 values are rejected there), 16-byte aligned, ldd a multiple of 16 / dst_bytes.
+ * EVERY element of the destination is written -- counts, zeros and the pad columns p..ldd-1 -- so it needs no memset.
+ * indices / values may be null when the rows hold no non-zero. */
+#define ORI_CSR_U8 1
+#define ORI_CSR_U16 2
+#define ORI_CSR_F32 4
+int ori_expand_csr_counts(const int64_t* indptr, int64_t base, const void* indices, int32_t idx_bytes,
+                          const void* values, int32_t val_type, void* dst, int32_t dst_bytes, int64_t ldd,
+                          int64_t rows, int32_t p, void* stream);
+
 /* Escapes of the saturating uint8 encoding: X[row[e] - row0, col[e]] = val[e] (device pointers; row = global
  * cell index, row0 = first cell of the slab held in X).  Entries outside the slab are ignored. */
 int ori_scatter_counts_f32(float* X, int64_t ldx, int64_t row0, int64_t rows, int32_t p, const int32_t* row,

@@ -13,6 +13,7 @@ ORI_F_DROPOUT, ORI_F_QUIRK, ORI_F_ELBO, ORI_F_NO_TENSOR, ORI_F_SPARSE, ORI_F_DEV
 ORI_F_FIXED_CHAIN = 128
 ORI_F_DETERMINISTIC = 256
 ORI_F_X_U16 = 512
+ORI_CSR_U8, ORI_CSR_U16, ORI_CSR_F32 = 1, 2, 4       # value types of ori_expand_csr_counts (their size in bytes)
 ORI_M_STEP, ORI_M_INIT, ORI_M_INIT_KEEP, ORI_M_FINALIZE, ORI_M_REFRESH = 0, 1, 2, 3, 4
 
 # layout of the reduction buffers of `ori_problem_t` (the ORI_R64_* / ORI_GSUM_* / ORI_SC_* slots and size macros)
@@ -100,6 +101,8 @@ _SIGNATURES = {
     'ori_widen_counts_f32': ([C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p], C.c_int),
     'ori_expand_bitmap_counts_f32': ([C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
                                       C.c_int32, C.c_void_p], C.c_int),
+    'ori_expand_csr_counts': ([C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,
+                               C.c_int64, C.c_int64, C.c_int32, C.c_void_p], C.c_int),
     'ori_scatter_counts_f32': ([C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int64, C.c_void_p], C.c_int),
     'ori_synth_counts_f32': ([C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_uint64,

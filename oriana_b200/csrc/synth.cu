@@ -211,6 +211,70 @@ extern "C" int ori_expand_bitmap_counts_f32(const uint32_t* bitmap, int64_t word
     return check_launch("k_expand_bitmap");
 }
 
+// ---- CSR row slab -> X (sparse count-matrix ingest, cmatrix.py:39-54 as_sparse_matrix) -------------------------------
+// Real single-cell matrices arrive as CSR (10x / Matrix Market, AnnData .X) with 2-10 % non-zeros: the host sends each
+// non-zero as a column index and a count instead of the whole row.  One CTA per row: zero-fill the row's ldd elements
+// with 16-byte stores (pad columns included, so the caller needs no memset), then scatter its non-zeros.  The indices of
+// a row are distinct (canonical CSR), so the scattered stores never collide; the column guard keeps every store in its
+// row's first p elements.  PCIe-bound where it is used (ingest, host-streamed slabs): no further tuning.
+template <typename I, typename V, typename D>
+__global__ void __launch_bounds__(256)
+k_expand_csr(const long long* __restrict__ indptr, long long base, const I* __restrict__ idx, const V* __restrict__ val,
+             D* __restrict__ dst, long long ldd, long long rows, int p)
+{
+    const int n16 = (int)(ldd * (long long)sizeof(D) / 16);        // ldd * sizeof(D) is a multiple of 16
+    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
+        D* drow = dst + r * ldd;
+        uint4* d16 = reinterpret_cast<uint4*>(drow);
+        for (int i = threadIdx.x; i < n16; i += blockDim.x) d16[i] = make_uint4(0u, 0u, 0u, 0u);
+        __syncthreads();
+        const long long lo = indptr[r] - base, hi = indptr[r + 1] - base;
+        for (long long e = lo + threadIdx.x; e < hi; e += blockDim.x) {
+            const long long c = (long long)idx[e];
+            if (c >= 0 && c < p) drow[c] = (D)val[e];
+        }
+    }
+}
+
+template <typename I, typename V, typename D>
+static void launch_expand_csr(const int64_t* indptr, int64_t base, const void* indices, const void* values, void* dst,
+                              int64_t ldd, int64_t rows, int32_t p, cudaStream_t st)
+{
+    const int grid = (int)(rows < 148 * 64 ? rows : 148 * 64);
+    k_expand_csr<I, V, D><<<grid, 256, 0, st>>>((const long long*)indptr, base, (const I*)indices, (const V*)values,
+                                                (D*)dst, ldd, rows, p);
+}
+
+template <typename I, typename D>
+static void launch_expand_csr_values(int32_t val_type, const int64_t* indptr, int64_t base, const void* indices,
+                                     const void* values, void* dst, int64_t ldd, int64_t rows, int32_t p, cudaStream_t st)
+{
+    if (val_type == ORI_CSR_U8) launch_expand_csr<I, uint8_t, D>(indptr, base, indices, values, dst, ldd, rows, p, st);
+    else if (val_type == ORI_CSR_U16) launch_expand_csr<I, uint16_t, D>(indptr, base, indices, values, dst, ldd, rows, p, st);
+    else launch_expand_csr<I, float, float>(indptr, base, indices, values, dst, ldd, rows, p, st);   // D = float (checked)
+}
+
+extern "C" int ori_expand_csr_counts(const int64_t* indptr, int64_t base, const void* indices, int32_t idx_bytes,
+                                     const void* values, int32_t val_type, void* dst, int32_t dst_bytes, int64_t ldd,
+                                     int64_t rows, int32_t p, void* stream)
+{
+    if (!indptr || !dst || p <= 0 || rows < 0 || ldd < p || (idx_bytes != 2 && idx_bytes != 4) ||
+        (val_type != ORI_CSR_U8 && val_type != ORI_CSR_U16 && val_type != ORI_CSR_F32) ||
+        (dst_bytes != 2 && dst_bytes != 4) || (ldd % (16 / dst_bytes)) || ((uintptr_t)dst & 15) ||
+        (val_type == ORI_CSR_F32 && dst_bytes == 2))
+        return set_error(ORI_EINVAL, "ori_expand_csr_counts: bad argument");
+    if (rows == 0) return ORI_OK;
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (idx_bytes == 2) {
+        if (dst_bytes == 4) launch_expand_csr_values<uint16_t, float>(val_type, indptr, base, indices, values, dst, ldd, rows, p, st);
+        else launch_expand_csr_values<uint16_t, uint16_t>(val_type, indptr, base, indices, values, dst, ldd, rows, p, st);
+    } else {
+        if (dst_bytes == 4) launch_expand_csr_values<int32_t, float>(val_type, indptr, base, indices, values, dst, ldd, rows, p, st);
+        else launch_expand_csr_values<int32_t, uint16_t>(val_type, indptr, base, indices, values, dst, ldd, rows, p, st);
+    }
+    return check_launch("k_expand_csr");
+}
+
 // Escapes of the saturating uint8 encoding: X[row[e] - row0, col[e]] = val[e] for the entries whose count does not
 // fit a byte (stored as 255 in the compact matrix).  row is the GLOBAL cell index, row0 the first cell of the slab.
 __global__ void __launch_bounds__(256)

@@ -104,6 +104,24 @@ class CompactCounts(_EscapeList):
             cls._gather_escapes(blk, r, parts)
         return cls(u8, *cls._join_escapes(parts, pin))
 
+    @classmethod
+    def from_csr(cls, csr, pin=True, chunk_entries=1 << 24):
+        """Encode a scipy CSR count matrix, densified in row chunks of about `chunk_entries` entries (the [n, p] uint8
+        matrix itself is inherent to this form)."""
+        n, p = csr.shape
+        pin = pin and torch.cuda.is_available()
+        u8 = torch.empty((n, p), dtype=torch.uint8, pin_memory=pin)
+        u8np, parts = u8.numpy(), []
+        step = max(1, chunk_entries // max(1, p))
+        for r in range(0, n, step):
+            blk = csr[r:r + step].toarray()
+            u8np[r:r + step] = np.minimum(blk, 255).astype(np.uint8)
+            idx = np.nonzero(blk >= 255)
+            if idx[0].size:
+                parts.append((torch.from_numpy((idx[0] + r).astype(np.int32)), torch.from_numpy(idx[1].astype(np.int32)),
+                              torch.from_numpy(blk[idx].astype(np.float32))))
+        return cls(u8, *cls._join_escapes(parts, pin))
+
     def dense(self):
         return self._with_escapes(self.u8.to(torch.float32))
 
@@ -174,6 +192,53 @@ class SparseCounts(_EscapeList):
             rowoff = rowoff.pin_memory()
         return cls((n, p), bitmap, nz, rowoff, *cls._join_escapes(parts, pin))
 
+    @classmethod
+    def from_csr(cls, csr, pin=True, chunk_nnz=1 << 24):
+        """Encode a scipy CSR count matrix in O(nnz + n p / 32), without densifying it: the bitmap from the column
+        indices, the saturating bytes and the escapes from the stored values.  Stored zeros are zeros (no bit); a CSR that
+        is not canonical (sorted, no duplicates) is made so on a copy first."""
+        from .singlecell.cmatrix import canonical_csr
+        csr = canonical_csr(csr)
+        n, p = csr.shape
+        pin = pin and torch.cuda.is_available()
+        W = (p + 31) // 32
+        ptr, ind, data = csr.indptr.astype(np.int64), csr.indices, csr.data
+        keep = data != 0
+        if keep.all():
+            rowoff = torch.from_numpy(ptr)
+        else:                                                      # the non-zeros of the rows before r
+            kept = np.zeros((keep.size + 1,), dtype=np.int64)
+            np.cumsum(keep, out=kept[1:])
+            rowoff = torch.from_numpy(kept[ptr])
+        total = int(rowoff[-1])
+        bitmap = torch.zeros((n, W), dtype=torch.int32, pin_memory=pin)
+        nz = torch.empty((total,), dtype=torch.uint8, pin_memory=pin and total > 0)
+        bm, nznp, off = bitmap.numpy().view(np.uint32).reshape(-1), nz.numpy(), rowoff.numpy()
+        parts, r0 = [], 0
+        while r0 < n:                                              # row chunks of at most chunk_nnz stored entries
+            r1 = max(r0 + 1, int(np.searchsorted(ptr, ptr[r0] + chunk_nnz, side='right')) - 1)
+            r1 = min(r1, n)
+            lo, hi = int(ptr[r0]), int(ptr[r1])
+            k = keep[lo:hi]
+            col = ind[lo:hi][k].astype(np.int64)
+            val = data[lo:hi][k]
+            row = np.repeat(np.arange(r0, r1, dtype=np.int64), np.diff(off[r0:r1 + 1]))
+            if col.size:
+                # (row, word) keys are non-decreasing in CSR order: OR the bits of each run of equal keys
+                key = row * W + (col >> 5)
+                bit = np.left_shift(np.uint32(1), (col & 31).astype(np.uint32))
+                start = np.flatnonzero(np.concatenate(([True], key[1:] != key[:-1])))
+                bm[key[start]] = np.bitwise_or.reduceat(bit, start)
+                nznp[off[r0]:off[r1]] = np.minimum(val, 255).astype(np.uint8)
+                esc = np.flatnonzero(val >= 255)
+                if esc.size:
+                    parts.append((torch.from_numpy(row[esc].astype(np.int32)), torch.from_numpy(col[esc].astype(np.int32)),
+                                  torch.from_numpy(val[esc].astype(np.float32))))
+            r0 = r1
+        if pin:
+            rowoff = rowoff.pin_memory()
+        return cls((n, p), bitmap, nz, rowoff, *cls._join_escapes(parts, pin))
+
     def byte_range(self, r0, r1):
         return int(self._off_np[r0]), int(self._off_np[r1])
 
@@ -196,6 +261,100 @@ class SparseCounts(_EscapeList):
         return float((blk != 0).float().mean()) < 0.85
 
 
+class CsrCounts:
+    """A count matrix held on the host in compressed sparse row form, the form single-cell data arrive in (10x / Matrix
+    Market, AnnData .X; cmatrix.py:39-54 `as_sparse_matrix`): per non-zero a column index and the count, no bitmap and no
+    escape list.  (index + value) bytes per non-zero cross PCIe per step -- 3 with uint16 indices and uint8 counts --
+    against SparseCounts' p / 8 + nnz bytes per cell, so it is the smaller form below 1/16 = 6.25 % non-zeros;
+    `ori_expand_csr_counts` rebuilds the float32 slab in HBM.  Lossless: `dense()` gives the counts back.
+
+        indptr   [n + 1] int64, row r's non-zeros = [indptr[r], indptr[r + 1])                        (pinned)
+        indices  [nnz] uint16 when p <= 65536, else int32: their genes, ascending within a row       (pinned)
+        values   [nnz] uint8 / uint16 / float32: the narrowest of the three that holds every count   (pinned)
+    """
+
+    _VAL_TYPES = {torch.uint8: _lib.ORI_CSR_U8, torch.uint16: _lib.ORI_CSR_U16, torch.float32: _lib.ORI_CSR_F32}
+
+    def __init__(self, shape, indptr, indices, values):
+        n, p = shape
+        assert indptr.dtype == torch.int64 and indptr.numel() == n + 1 and not indptr.is_cuda
+        assert indices.dtype == (torch.uint16 if p <= 65536 else torch.int32) and not indices.is_cuda
+        assert values.dtype in self._VAL_TYPES and values.numel() == indices.numel() and not values.is_cuda
+        self.shape = (int(n), int(p))
+        self.indptr, self.indices, self.values = indptr, indices, values
+        self._ptr_np = indptr.numpy()
+        assert int(self._ptr_np[0]) == 0 and int(self._ptr_np[-1]) == indices.numel() and (np.diff(self._ptr_np) >= 0).all()
+
+    @classmethod
+    def _build(cls, shape, indptr, indices, values, pin):
+        """From numpy arrays: stored zeros dropped, indices and counts in their narrow types, pinned."""
+        from .singlecell.cmatrix import narrow_count_dtype
+        n, p = shape
+        keep = values != 0
+        if not keep.all():
+            kept = np.zeros((keep.size + 1,), dtype=np.int64)
+            np.cumsum(keep, out=kept[1:])
+            indptr, indices, values = kept[indptr], indices[keep], values[keep]
+        vt = narrow_count_dtype(values) or torch.float32
+        vals = values.astype({torch.uint8: np.uint8, torch.uint16: np.uint16, torch.float32: np.float32}[vt])
+        idx = indices.astype(np.uint16 if p <= 65536 else np.int32)
+        pin = pin and torch.cuda.is_available()
+
+        def host(a):
+            t = torch.from_numpy(np.ascontiguousarray(a))
+            return t.pin_memory() if pin and t.numel() else t
+        return cls((n, p), host(np.asarray(indptr, dtype=np.int64)), host(idx), host(vals))
+
+    @classmethod
+    def from_csr(cls, csr, pin=True):
+        """Encode a scipy CSR count matrix (made canonical -- sorted, duplicates summed -- on a copy if it is not)."""
+        from .singlecell.cmatrix import canonical_csr
+        csr = canonical_csr(csr)
+        return cls._build(csr.shape, csr.indptr, csr.indices, csr.data, pin)
+
+    @classmethod
+    def from_tensor(cls, X, chunk_rows=1 << 13, pin=True):
+        """Encode a [n, p] count tensor (any real dtype, host or device; non-negative counts)."""
+        n, p = X.shape
+        counts, cols, vals = [], [], []
+        for r in range(0, n, chunk_rows):
+            blk = X[r:r + chunk_rows]
+            mask = blk != 0
+            counts.append(mask.sum(dim=1).cpu())
+            cols.append(mask.nonzero(as_tuple=False)[:, 1].cpu())
+            vals.append(blk[mask].cpu())
+        indptr = np.zeros((n + 1,), dtype=np.int64)
+        if n:
+            np.cumsum(torch.cat(counts).numpy(), out=indptr[1:])
+        cat = lambda parts, dt: torch.cat(parts).numpy() if parts else np.zeros((0,), dtype=dt)
+        return cls._build((n, p), indptr, cat(cols, np.int64), cat(vals, np.float32), pin)
+
+    def byte_range(self, r0, r1):
+        """[lo, hi) of the non-zeros of rows [r0, r1) in `indices` / `values`."""
+        return int(self._ptr_np[r0]), int(self._ptr_np[r1])
+
+    @property
+    def idx_bytes(self):
+        return self.indices.element_size()
+
+    @property
+    def val_type(self):
+        """The ori_expand_csr_counts value type of `values`."""
+        return self._VAL_TYPES[self.values.dtype]
+
+    def dense(self):
+        """The float32 matrix back on the host (numpy scatter; the device path is ori_expand_csr_counts)."""
+        n, p = self.shape
+        X = np.zeros((n, p), dtype=np.float32)
+        rows = np.repeat(np.arange(n), np.diff(self._ptr_np))
+        X[rows, self.indices.numpy().astype(np.int64)] = self.values.numpy().astype(np.float32)
+        return torch.from_numpy(X)
+
+    @property
+    def nbytes(self):
+        return 8 * self.indptr.numel() + self.indices.numel() * (self.idx_bytes + self.values.element_size())
+
+
 class HostStreamedCAVI:
 
     @staticmethod
@@ -212,16 +371,21 @@ class HostStreamedCAVI:
                  process_group=None, elbo=True, keep_hyper=True, precise=False):
         """X_host: CPU tensor [n, p] (pin it for asynchronous copies), float32 like the array the reference
         feeds its kernel (zigap.py:112) or the same counts kept compactly as uint16 / uint8 (half / a quarter of
-        the bytes per step over PCIe; widened to float32 on the device), or a `CompactCounts` (saturating uint8
-        plus an escape list for counts >= 255).  state: host arrays a1, a2 [n, k],
+        the bytes per step over PCIe; widened to float32 on the device), a `CompactCounts` (saturating uint8
+        plus an escape list for counts >= 255), a `SparseCounts` (bitmap + non-zero bytes) or a `CsrCounts` (column
+        index + count per non-zero).  state: host arrays a1, a2 [n, k],
         b1, b2 [p, k], alpha1, alpha2, beta1, beta2 [k] (a reference model's state vector)."""
         self._dev = _lib.require_cuda()
         self._lib = _lib.load()
         self._compact = X_host if isinstance(X_host, (CompactCounts, SparseCounts)) else None
         self._sparse = X_host if isinstance(X_host, SparseCounts) else None
+        self._csr = X_host if isinstance(X_host, CsrCounts) else None
         if self._sparse is not None:
             self.X, self._xbytes = None, 1             # bitmap + non-zero bytes per slab; the escapes follow each slab
             self.n, self.p = self._sparse.shape
+        elif self._csr is not None:
+            self.X, self._xbytes = None, 0             # row offsets, indices and counts of the slab's non-zeros
+            self.n, self.p = self._csr.shape
         else:
             if self._compact is not None:
                 X_host = self._compact.u8              # saturating bytes; the escapes follow each slab
@@ -283,6 +447,12 @@ class HostStreamedCAVI:
                 s['bm'] = torch.zeros((S, (p + 31) // 32), dtype=torch.int32, device=dev)
                 s['nz'] = torch.zeros((nzcap,), dtype=torch.uint8, device=dev)
                 s['off'] = torch.zeros((S + 1,), dtype=torch.int64, device=dev)
+            elif self._csr is not None:
+                cs, ptr = self._csr, self._csr._ptr_np
+                nnzcap = max(1, max(int(ptr[min(n, r + S)] - ptr[r]) for r in range(0, n, S)))
+                s['ptr'] = torch.zeros((S + 1,), dtype=torch.int64, device=dev)
+                s['ind'] = torch.zeros((nnzcap,), dtype=cs.indices.dtype, device=dev)
+                s['val'] = torch.zeros((nnzcap,), dtype=cs.values.dtype, device=dev)
             elif self._xbytes != 4:
                 s['Xq'] = torch.zeros((S, p), dtype=X_host.dtype, device=dev)      # compact counts as they arrive
             if self._compact is not None:
@@ -350,6 +520,17 @@ class HostStreamedCAVI:
             s['off'][:rows + 1].copy_(sp.rowoff[r0:r0 + rows + 1], non_blocking=True)
             info['lo'] = lo
             xbytes_sent = rows * s['bm'].shape[1] * 4 + (hi - lo) + (rows + 1) * 8
+        elif self._csr is not None:
+            cs = self._csr
+            lo, hi = cs.byte_range(r0, r0 + rows)
+            s['ptr'][:rows + 1].copy_(cs.indptr[r0:r0 + rows + 1], non_blocking=True)
+            if hi > lo:                                # 16-bit fields go through int16 views (same bits)
+                for dst, src in ((s['ind'], cs.indices), (s['val'], cs.values)):
+                    if src.dtype == torch.uint16:
+                        dst, src = dst.view(torch.int16), src.view(torch.int16)
+                    dst[:hi - lo].copy_(src[lo:hi], non_blocking=True)
+            info['lo'] = lo
+            xbytes_sent = (rows + 1) * 8 + (hi - lo) * (cs.idx_bytes + cs.values.element_size())
         else:
             s['Xq'][:rows].copy_(self.X[r0:r0 + rows], non_blocking=True)
         if self._compact is not None:
@@ -375,6 +556,10 @@ class HostStreamedCAVI:
             _lib.check(self._lib.ori_expand_bitmap_counts_f32(s['bm'].data_ptr(), s['bm'].shape[1], s['nz'].data_ptr(),
                                                               s['off'].data_ptr(), info['lo'], s['X'].data_ptr(), self._ldx,
                                                               rows, p, st))
+        elif self._csr is not None:
+            _lib.check(self._lib.ori_expand_csr_counts(s['ptr'].data_ptr(), info['lo'], s['ind'].data_ptr(),
+                                                       self._csr.idx_bytes, s['val'].data_ptr(), self._csr.val_type,
+                                                       s['X'].data_ptr(), 4, self._ldx, rows, p, st))
         elif self._xbytes != 4:
             _lib.check(self._lib.ori_widen_counts_f32(s['Xq'].data_ptr(), self._xbytes, p, s['X'].data_ptr(), self._ldx,
                                                       rows, p, st))

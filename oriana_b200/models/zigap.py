@@ -104,8 +104,13 @@ class ZIGaP(FactorModel):
             self._iter = int(state.get('iterations', 0))
         elif 'p_d' in state:
             pd = np.asarray(state['p_d'])
-            X = self.cmatrix.as_array()
-            zero = X == 0
-            if pd.shape != X.shape or (pd[zero] != 0).any() or (pd[~zero] < 0.5).any():
+            if self.cmatrix.is_sparse:         # the zero pattern from the CSR: p_d is >= 0.5 there and 0 elsewhere
+                r, c = self.cmatrix.as_sparse_matrix('csr').nonzero()
+                bad = pd.shape != self.cmatrix.shape or (pd[r, c] < 0.5).any() or np.count_nonzero(pd) != r.size
+            else:
+                X = self.cmatrix.as_array()
+                zero = X == 0
+                bad = pd.shape != X.shape or (pd[zero] != 0).any() or (pd[~zero] < 0.5).any()
+            if bad:
                 raise ValueError('state["p_d"] is not the indicator (X > 0) of a freshly constructed model; '
                                  'a mid-run snapshot must carry "pi_prev" (SURVEY.md section 8c)')
