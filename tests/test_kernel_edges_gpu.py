@@ -7,6 +7,10 @@ sit on an edge of the kernels -- own tile, CTA pair, sweep tile, 16-entry group,
 rare-path cases (dead cells, genes with pi <= 0 or pi = 1, zeros whose U_hat.V_hat passes the ELBO clamp) at group offsets
 0, 15, 16 and in the last ragged tile.  The edges are read from the kernel sources, so they move when the code moves.
 
+Each problem also runs with X stored as uint16 in HBM (ORI_F_X_U16, storage 'u16'): those are separate kernel instances,
+with their own TMA boxes, swizzles, widening and an 8-count row pitch.  Widening a count is exact, so they are held to the
+float32 tolerances.
+
 `test_probes_move_their_checks_far_beyond_every_tolerance` and `test_probes_of_the_other_gpu_problems_move_their_checks`
 (no GPU) apply each probe's mistake to the oracle's input on the very problems the GPU tests run, and show that it moves
 what the probe is checked by at least 20 times the tolerance of the plan that checks it.
@@ -117,15 +121,34 @@ def devi_chunk(n, p, sms=None):
     return tpc * sw
 
 
-def periods(n, p, K, plan, sms=None):
-    """Tile, pair, group and chunk lengths of the plan along the cells and along the genes."""
+# the lines of `launch_count_stats` / `launch_col_sums` (kernels_simt.cu) that `count_chunk_rows` restates (each launcher
+# has its own copy of the rule, `n_rows` there, `P->n_rows` here); 148 is written into them, not read from the device
+COUNT_SPLIT_RULE = [r'while (bx * chunks < 148 * 4 && P->n_rows / (chunks * 2) >= 16) chunks *= 2;',
+                    r'const long long rpc = (P->n_rows + chunks - 1) / chunks;',
+                    r'while (bx * chunks < 148 * 4 && n_rows / (chunks * 2) >= 16) chunks *= 2;',
+                    r'const long long rpc = (n_rows + chunks - 1) / chunks;']
+
+
+def count_chunk_rows(n, p):
+    """Rows per chunk of k_count_stats / k_col_sums: the row range is halved until 128-gene blocks x chunks fill 4 CTAs per
+    SM or a chunk would fall below 16 rows."""
+    bx, chunks = -(-p // 128), 1
+    while bx * chunks < 148 * 4 and n // (chunks * 2) >= 16:
+        chunks *= 2
+    return -(-n // chunks)
+
+
+def periods(n, p, K, plan, sms=None, esz=4):
+    """Tile, pair, group and chunk lengths of the plan along the cells and along the genes.  `esz`: bytes per count in
+    HBM (4: float32, 2: uint16); X rows start on 16 bytes, so the row pitch is 4 or 8 counts."""
+    pitch = 16 // esz
     if plan == 'simt':
-        return ([KC['PR_TR'], KC['PG_TR'], KC['SIMT_ROWS']], [KC['PR_TG'], KC['PG_TG'], 4])
+        return ([KC['PR_TR'], KC['PG_TR'], KC['SIMT_ROWS']], [KC['PR_TG'], KC['PG_TG'], pitch])
     KP = 32 if K <= 32 else 64
     sw = sweep_width(KP, plan == 'precise')
     own, pair, g = KC['TC_OWN'], KC['NCTA'] * KC['TC_OWN'], KC['GROUP']
     rows = [own, pair, sw, g, tc_chunk(p, n, True, sw, plan == 'precise', sms=sms)]
-    genes = [own, pair, sw, g, tc_chunk(n, p, False, sw, plan == 'precise', sms=sms), 4]       # 4: the row pitch
+    genes = [own, pair, sw, g, tc_chunk(n, p, False, sw, plan == 'precise', sms=sms), pitch]
     return rows, genes
 
 
@@ -199,7 +222,8 @@ def _base(n, p, K, model, start, seed, steps=2, dtype=np.float64):
     return s
 
 
-def edge_case(n, p, K, model, plan, start='mid', kind='edges', seed=None, steps=2, dtype=np.float64, sms=None, pers=None):
+def edge_case(n, p, K, model, plan, start='mid', kind='edges', seed=None, steps=2, dtype=np.float64, sms=None, pers=None,
+              esz=4):
     """(state, probes) of an edge-weighted problem.
 
     kind='edges': counts of 5000 on (edge cell, edge gene) pairs, the U_hat of one edge cell per edge gene and the V_hat
@@ -224,7 +248,7 @@ def edge_case(n, p, K, model, plan, start='mid', kind='edges', seed=None, steps=
         return i
 
     if kind == 'edges':
-        rp, gp = periods(n, p, K, plan, sms) if pers is None else pers
+        rp, gp = periods(n, p, K, plan, sms, esz) if pers is None else pers
         # an edge factor must dominate a sum over every cell / gene: the scale grows with the extent
         sr, sg = SCALE * max(1., n / 1024.), SCALE * max(1., p / 1024.)
         R, G = edges(n, rp), edges(p, gp)
@@ -367,6 +391,20 @@ PLANS = [('zigap', 'tf32', 20), ('zigap', 'tf32', 40), ('gap', 'tf32', 20), ('ga
 SPARSE_SHAPES = [(257, 66, 8), (2049, 33, 20), (129, 2049, 12)]
 NOMINAL = (4097, 3328, 12)       # fp32-grade gene pass: 13 gene pairs x 3 chunks fill the machine, no halving
 NOMINAL_PERIODS = ([KC['CHUNK_PRECISE']], [2 * KC['TC_OWN']])      # its chunk seams (cells), its CTA pairs (genes)
+# TF32 gene pass at its nominal 16384-cell chunk (configs 4 and 5 run it): 19 gene pairs x 2 chunks fill the machine
+NOMINAL_TF32 = (16385, 4609)
+NOMINAL_TF32_PERIODS = ([KC['CHUNK']], [2 * KC['TC_OWN']])
+# storage of X in HBM: bytes per count.  uint16 (ORI_F_X_U16) runs the kernels' uint16 instances: their own TMA boxes and
+# swizzles, their own widening and an 8-count row pitch
+ESZ = {'f32': 4, 'u16': 2}
+
+
+def with_storage(plans, ids):
+    """pytest params of (plan, storage): the float32 runs keep the plan's id, the uint16 runs add '-u16'."""
+    return [pytest.param(pl, st, id=ids(pl) + ('' if st == 'f32' else '-' + st)) for st in ESZ for pl in plans]
+
+
+plan_id = lambda t: '%s-%s-k%d' % t
 
 
 # --------------------------------------------------------------------------- CPU checks of the harness itself
@@ -387,12 +425,20 @@ def test_kernel_edges_are_read_from_the_sources():
     for line in TC_SPLIT_RULE:
         assert line in src, line
     assert devi_chunk(257, 2049, sms=148) == 192
+    with open(os.path.join(CSRC, 'kernels_simt.cu')) as f:
+        src = f.read()
+    for line in COUNT_SPLIT_RULE:
+        assert line in src, line
+    assert count_chunk_rows(3000, 127) == count_chunk_rows(3000, 257) == 24 and count_chunk_rows(20, 129) == 20
     assert tc_chunk(NOMINAL[1], NOMINAL[0], True, sweep_width(32, True), True, sms=148) == KC['CHUNK_PRECISE']
+    for KP in (32, 64):
+        assert tc_chunk(NOMINAL_TF32[1], NOMINAL_TF32[0], True, sweep_width(KP, False), False, sms=148) == KC['CHUNK']
+    assert periods(129, 63, 12, 'tf32', esz=2)[1][-1] == 8 and periods(129, 63, 12, 'simt', esz=2)[1][-1] == 8
 
 
-def _power(n, p, K, model, plan, kind, start, pers=None):
+def _power(n, p, K, model, plan, kind, start, pers=None, esz=4):
     """Probes of one problem whose mistake moves their check by less than 20x the plan's tolerance."""
-    s, probes = edge_case(n, p, K, model, 'tf32' if model == 'sparse' else plan, start, kind, sms=148, pers=pers)
+    s, probes = edge_case(n, p, K, model, 'tf32' if model == 'sparse' else plan, start, kind, sms=148, pers=pers, esz=esz)
     assert probes, (n, p, kind)
     base = oracle_step(s, model)
     weak = []
@@ -409,47 +455,65 @@ def _power(n, p, K, model, plan, kind, start, pers=None):
 
 @pytest.mark.parametrize('start', ['mid', 'init'])
 @pytest.mark.parametrize('kind', ['edges', 'rare'])
-@pytest.mark.parametrize('plan', PLANS, ids=lambda t: '%s-%s-k%d' % t)
-def test_probes_move_their_checks_far_beyond_every_tolerance(plan, kind, start):
+@pytest.mark.parametrize('plan,storage', with_storage(PLANS, plan_id))
+def test_probes_move_their_checks_far_beyond_every_tolerance(plan, storage, kind, start):
     """Over the problems of test_one_step_of_every_plan_matches_the_oracle_on_the_probes: every probe's mistake, applied to
     the oracle's input, moves what the probe is checked by at least 20x the plan's tolerance, so a kernel that drops or
-    misplaces the probe cannot pass."""
+    misplaces the probe cannot pass.  The uint16 problems differ by their row pitch of 8 counts."""
     model, pl, K = plan
     if model == 'gap' and start == 'init' and kind == 'edges':
         pytest.skip('the same problems as the mid-run start')
+    if kind == 'rare' and storage == 'u16':
+        pytest.skip('the rare-path probes do not depend on the row pitch')
     weak = []
     for (n, p) in SHAPES:
-        weak += _power(n, p, K, model, pl, kind, start)
+        weak += _power(n, p, K, model, pl, kind, start, esz=ESZ[storage])
     assert not weak, weak
 
 
-@pytest.mark.parametrize('case', ['sparse', 'nominal_chunk'])
+@pytest.mark.parametrize('case', ['sparse', 'sparse-u16', 'nominal_chunk', 'tf32_nominal_chunk-k40', 'tf32_nominal_chunk-k20'])
 def test_probes_of_the_other_gpu_problems_move_their_checks(case):
-    """The same for the SparseZIGaP problems (both tensor modes use them; the looser TF32 tolerance counts) and for the
-    fp32-grade problem at its nominal 2048-cell chunk."""
+    """The same for the SparseZIGaP problems (both tensor modes use them; the looser TF32 tolerance counts), for the
+    fp32-grade problem at its nominal 2048-cell chunk and for the TF32 problem at its nominal 16384-cell chunk (one float64
+    oracle step of it at K = 40 takes ~5 s, its ELBO ~7 s: only probes checked by the ELBO compute it)."""
     weak = []
-    if case == 'sparse':
+    if case.startswith('sparse'):
         for (n, p, K) in SPARSE_SHAPES:
-            for kind in ('edges', 'rare'):
+            for kind in (('edges', 'rare') if case == 'sparse' else ('edges',)):
                 for start in ('mid', 'init'):
-                    weak += _power(n, p, K, 'sparse', 'sparse_tf32', kind, start)
-    else:
+                    weak += _power(n, p, K, 'sparse', 'sparse_tf32', kind, start, esz=2 if case == 'sparse-u16' else 4)
+    elif case == 'nominal_chunk':
         n, p, K = NOMINAL
         weak += _power(n, p, K, 'zigap', 'precise', 'edges', 'mid', pers=NOMINAL_PERIODS)
+    else:
+        (n, p), K = NOMINAL_TF32, int(case[-2:])
+        weak += _power(n, p, K, 'zigap', 'tf32', 'edges', 'mid', pers=NOMINAL_TF32_PERIODS)
     assert not weak, weak
 
 
 # --------------------------------------------------------------------------- GPU: one step of every plan
-def _model(s, model, plan, **kw):
+def _model(s, model, plan, storage='f32', **kw):
+    """The device model of state `s`.  storage='u16': X handed in as uint16 and kept as uint16 in HBM at any size (the
+    models choose uint16 storage only where float32 would not fit the device, `oriana_b200.problem.counts_storage`)."""
+    import torch
     from oriana.models import GaP, SparseZIGaP, ZIGaP
     from oriana.singlecell import CountMatrix
+    from oriana_b200 import problem
     cls = dict(zigap=ZIGaP, gap=GaP, sparse=SparseZIGaP)[model]
     K = s['a1'].shape[1]
     kw = dict(kw)
     kw.setdefault('tensor', plan != 'simt')
     if plan == 'precise' or (model == 'sparse' and plan != 'simt' and 'precise' not in kw):
         kw.setdefault('precise', True)
-    return cls(CountMatrix(s['X']), k=K, use_factors=False, state=s, **kw)
+    if storage == 'f32':
+        return cls(CountMatrix(s['X']), k=K, use_factors=False, state=s, **kw)
+    assert storage == 'u16' and 0 <= s['X'].min() and s['X'].max() <= 65535
+    with pytest.MonkeyPatch.context() as mp:
+        mp.setattr(problem, 'counts_storage', lambda u16, *args: torch.uint16 if u16 else torch.float32)
+        m = cls(CountMatrix(s['X'].astype(np.uint16)), k=K, use_factors=False, state=s, **kw)
+    # no silent float32 run
+    assert m.counts_dtype == torch.uint16 and m._X.element_size() == 2 and m._ldx % 8 == 0
+    return m
 
 
 def _check_step(m, s, probes, model, plan, ref=None, elbo=True):
@@ -492,14 +556,14 @@ def _check_step(m, s, probes, model, plan, ref=None, elbo=True):
 @pytest.mark.gpu
 @pytest.mark.parametrize('start', ['mid', 'init'])
 @pytest.mark.parametrize('kind', ['edges', 'rare'])
-@pytest.mark.parametrize('plan', PLANS, ids=lambda t: '%s-%s-k%d' % t)
-def test_one_step_of_every_plan_matches_the_oracle_on_the_probes(cuda_lib, plan, kind, start):
+@pytest.mark.parametrize('plan,storage', with_storage(PLANS, plan_id))
+def test_one_step_of_every_plan_matches_the_oracle_on_the_probes(cuda_lib, plan, storage, kind, start):
     model, pl, K = plan
     if model == 'gap' and start == 'init' and kind == 'edges':
         pytest.skip('GaP has no dropout state: the initial and the mid-run start differ only in the factors')
     for (n, p) in SHAPES:
-        s, probes = edge_case(n, p, K, model, pl, start, kind)
-        m = _model(s, model, pl)
+        s, probes = edge_case(n, p, K, model, pl, start, kind, esz=ESZ[storage])
+        m = _model(s, model, pl, storage)
         assert m.uses_tensor_path == (pl != 'simt')
         if pl != 'simt':
             assert m._KP == (32 if K <= 32 else 64) and m.precise == (pl == 'precise')
@@ -508,14 +572,14 @@ def test_one_step_of_every_plan_matches_the_oracle_on_the_probes(cuda_lib, plan,
 
 @pytest.mark.gpu
 @pytest.mark.parametrize('start', ['mid', 'init'])
-@pytest.mark.parametrize('plan', ['sparse_precise', 'sparse_tf32'])
-def test_sparse_model_on_the_probes(cuda_lib, plan, start):
+@pytest.mark.parametrize('plan,storage', with_storage(['sparse_precise', 'sparse_tf32'], str))
+def test_sparse_model_on_the_probes(cuda_lib, plan, storage, start):
     """SparseZIGaP, tcgen05 kernels: fp32-grade (its default) and TF32 operands.  The S update amplifies operand rounding
     (a sigmoid of a difference of large sums), so p_s is checked at 20x the factor tolerance."""
     for (n, p, K) in SPARSE_SHAPES:
         for kind in ('edges', 'rare'):
-            s, probes = edge_case(n, p, K, 'sparse', 'tf32', start, kind)
-            m = _model(s, 'sparse', plan, precise=(plan == 'sparse_precise'), tensor=True)
+            s, probes = edge_case(n, p, K, 'sparse', 'tf32', start, kind, esz=ESZ[storage])
+            m = _model(s, 'sparse', plan, storage, precise=(plan == 'sparse_precise'), tensor=True)
             assert m.uses_tensor_path and m.precise == (plan == 'sparse_precise')
             ref = _check_step(m, s, probes, 'sparse', plan)
             if plan == 'sparse_precise':      # TF32 operands: p_s is not comparable step by step (test_sparse_gpu.py)
@@ -526,18 +590,38 @@ def test_sparse_model_on_the_probes(cuda_lib, plan, start):
 @pytest.mark.gpu
 def test_fp32_grade_gene_pass_at_its_nominal_chunk(cuda_lib):
     """A problem large enough that the fp32-grade gene pass keeps its nominal 2048-cell chunk (no halving), probed at the
-    chunk seams 2047 / 2048 / 4095 / 4096 and at the gene pairs."""
+    chunk seams 2047 / 2048 / 4095 / 4096 and at the gene pairs; float32 and uint16 storage against one oracle step."""
     n, p, K = NOMINAL
     assert tc_chunk(p, n, True, sweep_width(32, True), True) == KC['CHUNK_PRECISE'] < n
     s, probes = edge_case(n, p, K, 'zigap', 'precise', 'mid', 'edges', pers=NOMINAL_PERIODS)
-    m = _model(s, 'zigap', 'precise')
-    assert m.uses_tensor_path and m.precise
-    _check_step(m, s, probes, 'zigap', 'precise')
+    ref = None
+    for storage in ESZ:
+        m = _model(s, 'zigap', 'precise', storage)
+        assert m.uses_tensor_path and m.precise
+        ref = _check_step(m, s, probes, 'zigap', 'precise', ref=ref)
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('model', ['zigap', 'gap'])
-def test_underflow_emulation_on_the_probes(cuda_lib, monkeypatch, model):
+@pytest.mark.parametrize('K', [40, 20])
+def test_tf32_gene_pass_at_its_nominal_chunk(cuda_lib, K):
+    """The TF32 gene pass at its nominal 16384-cell chunk, two chunks (configs 4 and 5 run it so; every other TF32 problem
+    here is small enough that `tc_partition` halves the chunk): probed at the chunk seams 16383 / 16384 and at the gene
+    pairs.  K = 40 (KP = 64, config 5's plan) with float32 and uint16 storage against one oracle step, K = 20 (KP = 32)
+    with uint16 storage."""
+    n, p = NOMINAL_TF32
+    assert tc_chunk(p, n, True, sweep_width(32 if K <= 32 else 64, False), False) == KC['CHUNK'] < n
+    s, probes = edge_case(n, p, K, 'zigap', 'tf32', 'mid', 'edges', pers=NOMINAL_TF32_PERIODS)
+    ref = None
+    for storage in (('f32', 'u16') if K == 40 else ('u16',)):
+        m = _model(s, 'zigap', 'tf32', storage)
+        assert m.uses_tensor_path and not m.precise and m._KP == (32 if K <= 32 else 64)
+        ref = _check_step(m, s, probes, 'zigap', 'tf32', ref=ref)
+        del m
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize('model,storage', with_storage(['zigap', 'gap'], str))
+def test_underflow_emulation_on_the_probes(cuda_lib, monkeypatch, model, storage):
     """`emulate_underflow=True`, fp32-grade: the probed state with 40 % of the cells and genes 70 below the rest (their
     float32 exp underflows where two meet, see test_underflow_gpu.py) against the oracle with the sequential float32 loop."""
     from oracle import cavi_numpy as cn, zloop
@@ -548,7 +632,7 @@ def test_underflow_emulation_on_the_probes(cuda_lib, monkeypatch, model):
         return zloop.zigap_z(lU, lV, D_hat, X.astype(np.float32), quirk=quirk)
 
     for (n, p) in [(2049, 129), (257, 1025)]:
-        s, probes = edge_case(n, p, 12, model, 'precise', 'init', 'edges')
+        s, probes = edge_case(n, p, 12, model, 'precise', 'init', 'edges', esz=ESZ[storage])
         rows = {idx[0] for pr in probes for k, idx in pr['checks'] if k == 'a1'}
         genes = {idx[0] for pr in probes for k, idx in pr['checks'] if k == 'b1'}
         rng = np.random.default_rng(n)
@@ -556,7 +640,7 @@ def test_underflow_emulation_on_the_probes(cuda_lib, monkeypatch, model):
         low_i[list(rows)] = False; low_j[list(genes)] = False        # the probed cells and genes keep their scale
         s['a1'][low_i] = 0.0143; s['b1'][low_j] = 0.0143
         s = _refresh(s, 'init', model)
-        m = _model(s, model, 'precise', emulate_underflow=True)
+        m = _model(s, model, 'precise', storage, emulate_underflow=True)
         assert m.uses_tensor_path and m.precise
         with monkeypatch.context() as mp:
             mp.setattr(cn, 'z_expectations', literal_z)
@@ -570,23 +654,29 @@ def test_underflow_emulation_on_the_probes(cuda_lib, monkeypatch, model):
 @pytest.mark.gpu
 @pytest.mark.parametrize('model', ['zigap', 'gap'])
 def test_deterministic_mode_on_the_probes(cuda_lib, model):
-    """Deterministic mode at the edge shapes: two runs agree bit for bit and with the plain kernels within tolerance."""
+    """Deterministic mode at the edge shapes: two runs agree bit for bit and with the plain kernels within tolerance.  A
+    deterministic run on uint16 storage agrees bit for bit with the float32 one: widening a count is exact, the rest is the
+    same code."""
     names = FACTORS + HYPER + (('pi_d',) if model == 'zigap' else ())
     for (n, p, K, pl) in [(257, 2049, 20, 'tf32'), (16385, 63, 40, 'tf32'), (2049, 129, 12, 'precise')]:
         s, _ = edge_case(n, p, K, model, pl, 'mid', 'edges')
 
-        def run(**kw):
-            m = _model(s, model, pl, **kw)
+        def run(storage='f32', **kw):
+            m = _model(s, model, pl, storage, **kw)
             for _ in range(2):
                 m.step()
             return {k: getattr(m, k).asarray().copy() for k in names}, m.elbo()
 
         (a, ea), (b, eb) = run(deterministic=True), run(deterministic=True)
-        plain, ep = run()
+        (c, ec), (plain, ep), (plain16, ep16) = run('u16', deterministic=True), run(), run('u16')
         for k in names:
             assert np.array_equal(a[k], b[k]), (n, p, k)
+            assert np.array_equal(a[k], c[k]), (n, p, k, 'u16')
             assert relerr(plain[k], a[k]) < 2 * TOL[pl][0], (n, p, k)
-        assert ea == eb and abs(ep - ea) < TOL[pl][3] * abs(ea)
+            assert relerr(plain16[k], a[k]) < 2 * TOL[pl][0], (n, p, k, 'u16')
+        # sum lgamma(X + 1) is formed with float64 atomics in either order (test_u16_counts_gpu.py)
+        assert ea == eb and abs(ec - ea) <= 1e-13 * abs(ea), (ea, ec)
+        assert abs(ep - ea) < TOL[pl][3] * abs(ea) and abs(ep16 - ea) < TOL[pl][3] * abs(ea)
 
 
 @pytest.mark.gpu
@@ -633,17 +723,22 @@ def _ll_int(X, lam, pi):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('precise', [True, False])
+@pytest.mark.parametrize('precise,storage', with_storage([True, False], str))
 @pytest.mark.parametrize('masked', [False, True])
-def test_deviance_pass_at_tensor_shapes_matches_the_oracle(cuda_lib, masked, precise):
+def test_deviance_pass_at_tensor_shapes_matches_the_oracle(cuda_lib, masked, precise, storage):
     """The tensor deviance pass (DEVI) against the float64 oracle on edge-probed SparseZIGaP states: counts of 5000 on the
     edges (one truncated term is a visible share of the sum), observed counts under a rate that underflows float32 in the
     last ragged group (the float64 redo) and, `masked`, genes with p_s = 0 at group edges (an exactly zero rate: INT64_MIN
-    terms, compared by their parity bit)."""
+    terms, compared by their parity bit).  uint16 storage: one edge count is 65535, a count with the top bit set through
+    the widening and the log x of large counts."""
     from oracle import sparse_numpy as sn
     for (n, p, K) in [(2049, 33, 20), (257, 2049, 8), (129, 65, 12), (16385, 17, 4)]:
-        rp, gp = periods(n, p, K, 'tf32')
-        s, _ = edge_case(n, p, K, 'sparse', 'tf32', 'mid', 'edges', pers=(rp, gp + [devi_chunk(n, p)]))   # + its own chunks
+        rp, gp = periods(n, p, K, 'tf32', esz=ESZ[storage])
+        s, _ = edge_case(n, p, K, 'sparse', 'tf32', 'mid', 'edges', pers=(rp, gp + [devi_chunk(n, p)]),   # + its own chunks
+                         esz=ESZ[storage])
+        if storage == 'u16':
+            i, j = np.argwhere(s['X'] == BIG)[-1]
+            s['X'][i, j] = 65535
         g = KC['GROUP']
         last = [j for j in (p - 1, p - 2) if j >= (p - 1) // g * g]
         tiny = [i for i in (n // 2, n // 2 + 1) if i < n]
@@ -655,7 +750,8 @@ def test_deviance_pass_at_tensor_shapes_matches_the_oracle(cuda_lib, masked, pre
             s['X'][:, mg] = np.maximum(s['X'][:, mg], 1)[:, :]
             s['X'][1::2, mg] = 0
         s = _refresh(s, 'mid', 'sparse')
-        m = _model(s, 'sparse', 'sparse_precise' if precise else 'sparse_tf32', tensor=True, precise=precise)
+        assert storage == 'f32' or s['X'].max() == 65535
+        m = _model(s, 'sparse', 'sparse_precise' if precise else 'sparse_tf32', storage, tensor=True, precise=precise)
         assert m.uses_tensor_path and m.precise == precise
         li = [int(v) for v in m._loglikelihood_sums(want_f64=False)[0]]
         lam = sn.model_rate(s)

@@ -1,6 +1,6 @@
 """GPU, needs >= 2 devices (skipped on a single-GPU box): the device models row-sharded over two ranks on NCCL against
-the same models unsharded -- ZIGaP on the tensor path and SparseZIGaP with its deviance metrics (integer sums
-all-reduced as int64)."""
+the same models unsharded -- ZIGaP on the tensor path, ZIGaP at K = 40 on uint16 storage, and SparseZIGaP with its
+deviance metrics (integer sums all-reduced as int64)."""
 import os
 import socket
 import sys
@@ -81,6 +81,34 @@ def _worker(rank, world, port, out):
                 a, b = getattr(mz, k).asarray(), getattr(fz, k).asarray()
                 res['zigap_' + k] = float(np.max(np.abs(a - b) / (np.abs(b) + 1e-6 * np.abs(b).max())))
             res['zigap_elbo'] = float(np.max(np.abs(tr - fz.elbo_trace) / np.abs(fz.elbo_trace)))
+        # ---- ZIGaP, tensor path, K = 40 (KP = 64), each rank's row block kept as uint16 in HBM, against the unsharded
+        # float32 model.  uint16 storage is forced here, in the spawned process: the models choose it only where float32
+        # would not fit the device
+        import torch
+        from oriana_b200 import problem
+        problem.counts_storage = lambda u16, *args: torch.uint16 if u16 else torch.float32
+        n, p, K = 5000, 1200, 40
+        X = cn.synth_counts(n, p, K, seed=23)
+        X[7, 11] = 65535
+        s = cn.init_state(X, K, np.random.default_rng(4), 'zigap')
+        r0, r1 = RowSharding.row_block(n, rank, world)
+        mine = {k: (v[r0:r1].copy() if k in ('X', 'a1', 'a2', 'p_d') else v.copy()) for k, v in s.items()}
+        mu = ZIGaP(CountMatrix(mine['X'].astype(np.uint16)), k=K, use_factors=False, state=mine, sharded=True, tensor=True)
+        assert mu.counts_dtype == torch.uint16 and mu._X.element_size() == 2 and mu._ldx % 8 == 0
+        fu = ZIGaP(CountMatrix(X.astype(np.float32)), k=K, use_factors=False, state=s, tensor=True) if rank == 0 else None
+        assert fu is None or fu.counts_dtype == torch.float32
+        for _ in range(3):
+            mu.step()
+            if fu is not None:
+                fu.step()
+        tr = mu.elbo_trace
+        if rank == 0:
+            for k in ('b1', 'b2', 'pi_d', 'alpha1', 'beta2'):
+                a, b = getattr(mu, k).asarray(), getattr(fu, k).asarray()
+                res['zigap_u16_' + k] = float(np.max(np.abs(a - b) / (np.abs(b) + 1e-6 * np.abs(b).max())))
+            a, b = mu.a1.asarray(), fu.a1.asarray()[r0:r1]
+            res['zigap_u16_a1'] = float(np.max(np.abs(a - b) / (np.abs(b) + 1e-6 * np.abs(b).max())))
+            res['zigap_u16_elbo'] = float(np.max(np.abs(tr - fu.elbo_trace) / np.abs(fu.elbo_trace)))
             out.update(res)
     finally:
         dist.destroy_process_group()
@@ -98,7 +126,7 @@ def test_two_gpu_sharded_models_match_unsharded(cuda_lib):
     assert res, 'rank 0 reported nothing'
     print(res)
     for k, e in res.items():
-        if k == 'zigap_elbo':
+        if k in ('zigap_elbo', 'zigap_u16_elbo'):
             tol = 1e-5
         elif k in ('sparse_deviance', 'sparse_explained'):     # integer-truncated sums masked by round(D_hat): they inherit
             tol = 2e-4                                         # the p_s differences below (measured 4e-7 ... 6e-5 between runs)

@@ -257,3 +257,92 @@ def test_uint16_inputs_that_fit_as_float32_keep_float32_storage(cuda_lib, monkey
     for m in models[1:]:
         for k in PARAMS:
             assert np.array_equal(getattr(m, k).asarray(), getattr(models[0], k).asarray()), k
+
+
+# --------------------------------------------------------------------------- every uint16 value
+def _all_values(n, p, seed):
+    """[n, p] int64 counts that hold each of the 65536 uint16 values at least once, at random places."""
+    rng = np.random.default_rng(seed)
+    X = rng.poisson(2.0, (n, p)) * (rng.random((n, p)) < 0.5)
+    X.flat[rng.permutation(n * p)[:65536]] = np.arange(65536)
+    return X
+
+
+@pytest.mark.parametrize('p', [127, 128, 129, 257])
+def test_uint16_count_statistics_are_exact(cuda_lib, p):
+    """The constant statistics of uint16 X against exact sums, over the 128-gene blocks (p = 127 ... 257) and the row
+    chunks of `launch_count_stats` / `launch_col_sums` (every row on either side of a chunk seam holds no zero, so a chunk
+    that loses its first or last row changes every column's sum):
+    - ori_column_sums_u16_f64 is exact: every partial sum is an integer below 2^53, whatever the order of the atomics;
+    - ori_row_sums_u16_f32 is exact where the row sums to less than 2^24; above, off by the float32 roundings of its
+      five warp-shuffle additions at most (each lane's partial sum is below 2^24);
+    - a ZIGaP model on uint16 storage, initial start: pi_d = (X > 0).sum(0) / n and the non-zero count exactly, and
+      sum lgamma(X + 1) (lgammaf per entry, CUDA: 6 ulp for positive arguments) within 4e-7 of the float64 sum.
+      Measured: 2.9e-9 relative at every p (one B200, 1000 W power limit)."""
+    import math
+    import torch
+    from oriana.models import ZIGaP
+    from oriana.singlecell import CountMatrix
+    from oriana_b200 import _lib
+    from oriana_b200.problem import row_pitch
+    from test_kernel_edges_gpu import count_chunk_rows
+    n = 3000
+    X = _all_values(n - 1, p, seed=p)
+    X = np.vstack([np.full((1, p), 65535 if p > 256 else 1), X])        # p = 257: a row sum of 1.68e7 > 2^24
+    rpc = count_chunk_rows(n, p)
+    assert 16 <= rpc < n // 64
+    seams = [r for b in range(rpc, n, rpc) for r in (b - 1, b)]
+    X[seams] = np.maximum(X[seams], 1)
+    assert np.unique(X).size == 65536
+    Xd = _u16_block(X, row_pitch(p, 2))
+    cols = torch.zeros((p,), dtype=torch.float64, device='cuda')
+    rows = torch.full((n,), float('nan'), dtype=torch.float32, device='cuda')
+    _lib.check(cuda_lib.ori_column_sums_u16_f64(Xd.data_ptr(), Xd.stride(0), n, p, cols.data_ptr(), _lib.stream_ptr()))
+    _lib.check(cuda_lib.ori_row_sums_u16_f32(Xd.data_ptr(), Xd.stride(0), n, p, rows.data_ptr(), _lib.stream_ptr()))
+    torch.cuda.synchronize()
+    assert np.array_equal(cols.cpu().numpy(), X.sum(0).astype(np.float64))
+    got, want = rows.cpu().numpy().astype(np.float64), X.sum(1)
+    small = want < 1 << 24
+    assert np.array_equal(got[small], want[small].astype(np.float64))
+    assert (p > 256) == (not small.all())
+    assert np.all(np.abs(got[~small] - want[~small]) <= 5 * 2.0 ** -24 * want[~small])
+
+    np.random.seed(1)
+    m = ZIGaP(CountMatrix(X.astype(np.uint16)), k=4, use_factors=False)
+    assert m.counts_dtype == torch.uint16 and m._X.element_size() == 2 and m._ldx % 8 == 0
+    assert np.array_equal(m.pi_d.asarray(), (X > 0).sum(0) / n)
+    scal = m._scal.cpu().numpy()
+    assert scal[_lib.ORI_SC_NNZ] == np.count_nonzero(X)
+    lg = np.array([math.lgamma(v + 1.) for v in range(65536)])
+    want_lg = float(np.bincount(X.ravel(), minlength=65536) @ lg)
+    err = abs(scal[_lib.ORI_SC_LGAMX] - want_lg) / want_lg
+    print('p = %d: sum lgamma(X + 1) relative error %.2e' % (p, err))
+    assert err < 4e-7, err
+
+
+ALL_VALUE_PLANS = {      # model, K, model arguments, plan of test_kernel_edges_gpu.py (its tolerances)
+    'zigap_tf32_kp32': ('zigap', 12, dict(tensor=True), 'tf32'),
+    'zigap_tf32_kp64': ('zigap', 40, dict(tensor=True), 'tf32'),
+    'zigap_precise': ('zigap', 12, dict(tensor=True, precise=True), 'precise'),
+    'zigap_cuda_core': ('zigap', 12, dict(force_simt=True), 'simt'),
+    'gap_tf32_kp32': ('gap', 12, dict(tensor=True), 'tf32'),
+}
+
+
+@pytest.mark.parametrize('case', sorted(ALL_VALUE_PLANS))
+def test_every_uint16_value_through_the_passes(cuda_lib, case):
+    """A ragged 300 x 257 problem whose counts take each of the 65536 uint16 values: in deterministic mode the uint16
+    model is bit-identical to the float32 model (the widening is exact for every bit pattern, not only the few `_counts`
+    places), and one plain step from the initial state matches the float64 oracle at the plan's tolerances."""
+    from oracle import cavi_numpy as cn
+    from test_kernel_edges_gpu import _check_step, _model, _refresh
+    model, K, kw, plan = ALL_VALUE_PLANS[case]
+    X = _all_values(300, 257, seed=K)
+    m32, m16 = _pair(model, X, K, deterministic=True, **kw)
+    assert m16.uses_tensor_path == (plan != 'simt')
+    _assert_identical(m32, m16)
+    s = _refresh(cn.init_state(X, K, np.random.default_rng(2), model), 'init', model)
+    kw = {k: v for k, v in kw.items() if k != 'force_simt'}
+    m = _model(s, model, plan, 'u16', **kw)
+    assert m.uses_tensor_path == (plan != 'simt')
+    _check_step(m, s, [], model, plan)
